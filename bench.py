@@ -27,6 +27,10 @@ weak scaling); time = max over ranks.
 
 `--impl reference` times that CPU implementation alone (the reference's own libx264/libswscale path
 cannot be built in this image: no headers, no libraries -- see DESIGN.md), all host threads.
+
+`--dump-outputs DIR` writes what the last step of the timed `e2e` leg handed its caller, plus the reconstruction that step left
+on the GPU (read back after timing), to DIR/*.npy (see dump_outputs).
+The inputs depend on the arguments alone, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -222,6 +226,35 @@ def verify_final_state(eng, b2enc, b2oracle, rank, groups, ftype, last_step, arg
                     "regions == CPU oracle replay from the group's last I step (bit-exact)"}
 
 
+DUMP_MBS = 16384                                                # --dump-outputs sample: ~57 MB of .npy files, under 64 MB
+
+
+def dump_outputs(eng, out_dir):
+    """--dump-outputs: the results of the engine's last step for a fixed sample of DUMP_MBS macroblocks drawn over all slots
+    (numpy seed 0, sorted by slot and macroblock; every macroblock when there are fewer):
+      mb_info.npy  float64 (n, 33): the per-MB decisions the caller receives, MBINFO fields in order, subarrays flattened
+      levels.npy   float32 (n, 26, 16): the quantised levels the caller receives (unpacked when they leave the GPU packed)
+      recon.npy    float32 (n, 384): the reconstructed macroblock, 16x16 luma then 8x8 Cb and 8x8 Cr, row by row.  The caller
+                   does not receive it: it is the reference state of the next step, read back from the GPU after timing
+    Every value is exact in its type."""
+    import numpy as np
+    from numpy.lib import recfunctions
+    n = min(DUMP_MBS, eng.slots * eng.nmb)
+    pick = np.sort(np.random.default_rng(0).choice(eng.slots * eng.nmb, n, replace=False))
+    info, levels, recon = [], [], []
+    for s in np.unique(pick // eng.nmb):
+        mbs = pick[pick // eng.nmb == s] % eng.nmb
+        i, coef = eng.results(int(s))
+        info.append(recfunctions.structured_to_unstructured(i[mbs], np.float64))
+        levels.append(coef["blk"][mbs].astype(np.float32))
+        blocks = [p.reshape(eng.mbh, b, eng.mbw, b).transpose(0, 2, 1, 3).reshape(eng.nmb, b * b)[mbs]
+                  for p, b in zip(eng.recon(int(s)), (16, 8, 8))]
+        recon.append(np.concatenate(blocks, axis=1).astype(np.float32))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, parts in (("mb_info", info), ("levels", levels), ("recon", recon)):
+        np.save(os.path.join(out_dir, name + ".npy"), np.concatenate(parts))
+
+
 def cpu_encode_gop(b2oracle, np, stream, n_p, times):
     """one closed GOP on one host thread: 1 I + n_p P frames through the oracle encode stage"""
     prm = b2oracle.Params(QP, MERANGE, 1, 1)
@@ -327,9 +360,13 @@ def main():
                     "pruned figures are reported beside them under `pruned`)")
     ap.add_argument("--no-pruned-leg", action="store_true", help="skip the `pruned` leg")
     ap.add_argument("--transform8x8", type=int, default=0, help="1: adaptive 8x8 transform for inter MBs (row N1, outside the named path)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last `e2e` step, and the reconstruction "
+                    "read back from the GPU after timing, for a fixed sample of macroblocks (rank 0) to DIR/*.npy")
     args = ap.parse_args()
     select_workload(args.workload)
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to --impl b200")
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
 
@@ -428,6 +465,8 @@ def main():
     barrier()
     clk = clocks.stop(mark)
     e2e = world * SLOTS * n_e2e / e2e_s
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(eng, args.dump_outputs)                     # the e2e leg's last step: its results are in the host buffers
 
     # ---- after the timed legs: verification of the state they left (rank 0), then the same legs with the search pruning on ------
     iso = None

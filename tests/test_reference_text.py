@@ -1,12 +1,12 @@
 """Compile-level proof of the drop-in (SURVEY.md 8b): the reference's OWN TEXT -- x264_context_t (av_encode.c:369-376),
 enc_x264_open (:378-438), enc_x264_close (:440-444), enc_avfilter_pull_to_x264_context (:525-560), the encode loop (:968-975)
-and the drain loop (:1076-1083) -- is read from /root/reference at test time (never copied into the repository), compiled
-unchanged through include/b2enc_compat.h with stub libavcodec / libavfilter types, and
+and the drain loop (:1076-1083) -- is read at test time from the av_encode.c that B2ENC_AV_ENCODE_C names (never copied into
+the repository), compiled unchanged through include/b2enc_compat.h with stub libavcodec / libavfilter types, and
   * linked against the real libb2enc.so (every symbol the text needs resolves), and
   * linked against the host sources + the oracle-backed mock engine (tests/mock) and RUN on the CPU: the stream it muxes is
     byte-identical to the oracle encoder's at the reference's defaults (preset medium, tune film, CRF 20, profile NULL;
     av_encode.c:102-105).
-Skipped where /root/reference does not exist (the GPU box)."""
+Skipped when B2ENC_AV_ENCODE_C is not set."""
 import ctypes as C
 import glob
 import os
@@ -16,7 +16,7 @@ import pytest
 from test_oracle_decode import smooth_seq
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/av_encode.c"
+REF = os.environ.get("B2ENC_AV_ENCODE_C", "")                 # the reference program's av_encode.c
 
 HARNESS_HEAD = r"""
 #include <stdbool.h>
@@ -127,7 +127,7 @@ def build_harness(tmp_path):
 @pytest.fixture(scope="module")
 def mock_so():
     if not os.path.exists(REF):
-        pytest.skip("/root/reference is not on this machine")
+        pytest.skip("B2ENC_AV_ENCODE_C does not name the reference's av_encode.c")
     out = os.path.join(ROOT, "tests", "mock", "_build")
     os.makedirs(out, exist_ok=True)
     so = os.path.join(out, "libb2enc_mock.so")
@@ -140,7 +140,7 @@ def mock_so():
 
 def test_reference_text_links_against_libb2enc(b2, tmp_path):
     if not os.path.exists(REF):
-        pytest.skip("/root/reference is not on this machine")
+        pytest.skip("B2ENC_AV_ENCODE_C does not name the reference's av_encode.c")
     c = build_harness(tmp_path)
     libdir = os.path.dirname(b2.so_path())
     r = subprocess.run(["gcc", "-std=gnu99", "-O1", "-I" + os.path.join(ROOT, "include"), "-o", str(tmp_path / "harness_real"), str(c),
