@@ -43,9 +43,9 @@ int b2k_me_fullpel_pruned(const uint8_t *cur_y, const uint8_t *ref_y, int w, int
                           float *sums_ms, unsigned long long *swept_candidates, unsigned long long *all_candidates);
 /* K1a alone on the padded (B2_PAD, replicated border) planes; out [nframes][rows][pitch] u32 (may be NULL to query the geometry):
  * position (Y,X) = min | max << 16 over rows Y..Y+ks-1 of S[.][X], S[Y][X] = sum of padded[Y..Y+15][X..X+15]; 0 | 0xffff where a
- * block leaves the allocation.  ks in {1, 3, 5, 11, 13} */
+ * block leaves the allocation.  ks in {1, 3, 5} */
 int b2k_block_sums(const uint8_t *y, int w, int h, int nframes, int ks, uint32_t *out, int *pitch_out, int *rows_out);
-/* rows per lane-task of the pruned search for +-merange (environment B2_K1_PRUNE_ROWS=coarse|fine) */
+/* rows per lane-task of the pruned search for +-merange: 5 (+-32) or 3 (+-16) */
 int b2_k1_prune_rows(int merange);
 
 /* K1, partition variant (row N1, partitions = 2): best full-pel vector and cost of each of the nine shape parts per MB

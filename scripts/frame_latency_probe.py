@@ -22,6 +22,6 @@ for slots in (1, 4):
         eng.sync()
         ms = eng.kernel_ms()
         tot = sum(v[0] / max(v[1], 1) for v in ms.values())
-        print("%dx%d +-%d deblock %d, %d slot(s), %s frame, wavefrontK8 %s: chain %.3f ms | " % (W, H, R, deblock, slots, kind, os.environ.get("B2_K8_WAVEFRONT", "0"), tot)
+        print("%dx%d +-%d deblock %d, %d slot(s), %s frame: chain %.3f ms | " % (W, H, R, deblock, slots, kind, tot)
               + "  ".join("%s %.3f" % (k.split()[0], v[0] / max(v[1], 1)) for k, v in ms.items() if v[1]), flush=True)
     eng.close()

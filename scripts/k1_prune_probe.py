@@ -1,16 +1,9 @@
 """K1 exhaustive vs pruned (K1a block sums + successive elimination), kernel alone: the bench's synthetic sequence (uniform pan,
 predictor = the previous frame's vector = exact) and a smooth 'natural-like' field with a differently moving object and a
 predictor that is right only for the background; +-32 at 1080p, +-16 at 720p; 16 frames per launch.  Results are compared."""
-import os, sys, json, subprocess
+import os, sys, json
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "video-encoder_b200")); sys.path.insert(0, os.path.join(ROOT, "oracle"))
-if len(sys.argv) < 2 or sys.argv[1] != "child":
-    # the lane-task depth and the CTA size are read once per process: one child per variant
-    for rows_, nt in (("coarse", "256"), ("fine", "256")):
-        env = dict(os.environ, B2_K1_PRUNE_ROWS=rows_, B2_K1_THREADS=nt)
-        print("== B2_K1_PRUNE_ROWS=%s B2_K1_THREADS=%s" % (rows_, nt), flush=True)
-        subprocess.run([sys.executable, os.path.abspath(__file__), "child"], env=env)
-    sys.exit(0)
 import numpy as np, b2enc, b2oracle
 import scipy.ndimage as ndi
 

@@ -54,6 +54,6 @@ run(6)
 for g in range(G):
     issued[g] = fetched[g] = 0
 dt = run(steps)
-print("slots %2d groups %2d deblock %d wavefrontK8 %s me_prune %d: %d frames in %.3f s = %.0f frames/s" %
-      (slots, G, deblock, os.environ.get("B2_K8_WAVEFRONT", "0"), prune, slots * steps, dt, slots * steps / dt), flush=True)
+print("slots %2d groups %2d deblock %d me_prune %d: %d frames in %.3f s = %.0f frames/s" %
+      (slots, G, deblock, prune, slots * steps, dt, slots * steps / dt), flush=True)
 eng.close()

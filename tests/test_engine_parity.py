@@ -12,12 +12,12 @@ INFO_FIELDS = ["mb_type", "mvx", "mvy", "i16_mode", "chroma_mode", "cbp", "i4_mo
 
 
 def run_and_compare(oracle, b2, seqs, w, h, qp, R, subpel=1, intra_in_p=1, fmt="yuv420p", deblock=0, transform8x8=0, pack_levels=0,
-                    partitions=0, deblock_offsets=(0, 0), me_prune=0):
-    """seqs: list (one per slot) of lists of (y,u,v) frames"""
+                    partitions=0, deblock_offsets=(0, 0), me_prune=0, streams=0):
+    """seqs: list (one per slot) of lists of (y,u,v) frames; streams: stream groups (0: the engine's default)"""
     S, T = len(seqs), len(seqs[0])
     eng = b2.Engine(w, h, slots=S, fmt=fmt, ring=2, merange=R, qp=qp, subpel=subpel, intra_in_p=intra_in_p, deblock=deblock,
                     transform8x8=transform8x8, pack_levels=pack_levels, partitions=partitions, deblock_offsets=deblock_offsets,
-                    me_prune=me_prune)
+                    me_prune=me_prune, streams=streams)
     prm = oracle.Params(qp, R, subpel, intra_in_p, deblock, transform8x8, partitions, deblock_offsets[0], deblock_offsets[1])
     stats = {"t8": 0, "coded4": 0, "i8": 0, "parts": np.zeros(4, int), "mvx_mod4": np.zeros(4, int)}
     prev = [None] * S; prev_mv = [None] * S
@@ -174,6 +174,17 @@ def test_engine_with_deblocking(oracle, b2, w, h, qp, R, cut):
     """K8 in-loop deblocking (SURVEY.md 8f N2): reconstruction and everything downstream stay bit-exact"""
     seqs = [smooth_seq(w, h, 5, seed=qp + 1, cut=cut), smooth_seq(w, h, 5, seed=qp + 2)]
     run_and_compare(oracle, b2, seqs, w, h, qp, R, deblock=1)
+
+
+def test_engine_deblocking_wavefront(oracle, b2):
+    """K8 takes its anti-diagonal wavefront when a launch covers 4 frames or more (bench.py's shape: 8 slots per stream group); the
+    other deblocking tests put at most 3 slots in a group and so reach only the row pipeline.  Here 4 slots share one stream group.
+    At 576x320 a diagonal holds up to 18 macroblocks, so each frame is a cluster of two CTAs with a cluster barrier per diagonal.
+    The second run adds the 8x8 transform and 8x8 partitions, whose edge rules the wavefront derives on its own."""
+    w, h = 576, 320
+    seqs = [smooth_seq(w, h, 4, seed=41 + s, cut=(2 if s == 1 else None)) for s in range(3)] + [[oracle.synth_frame(w, h, t, 3) for t in range(4)]]
+    run_and_compare(oracle, b2, seqs, w, h, 30, 16, deblock=1, streams=1)
+    run_and_compare(oracle, b2, seqs, w, h, 26, 16, deblock=1, transform8x8=1, partitions=1, streams=1)
 
 
 @pytest.mark.parametrize("offs", [(-1, -1), (3, -2), (-6, 6)])

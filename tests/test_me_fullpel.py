@@ -124,17 +124,6 @@ def test_parts_ties_lambda_and_predictors(oracle, b2, R):
         _check_parts(oracle, b2, cur, ref, R, pmv, lam)
 
 
-def test_persistent_pipelined_kernel_is_bit_exact():
-    """B2_K1_PERSISTENT=1: the persistent, TMA-pipelined form of K1 (producer warps + three buffers + mbarriers) gives the same
-    vectors and costs; the switch is read once per process, so the full-pel tests are re-run in a child process"""
-    import os, subprocess, sys
-    env = dict(os.environ, B2_K1_PERSISTENT="1")
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-m", "gpu", "-x", "-q", "-k", "not persistent"],
-                       capture_output=True, text=True, env=env, timeout=600, cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    assert " passed" in r.stdout
-
-
 # ---- K1 with lossless pruning (engine option me_prune): K1a block sums + successive elimination ---------------------------
 def _check_pruned(oracle, b2, cur, ref, R, pmv=None, lam=0):
     """vectors and costs equal the oracle's exhaustive scan (and hence the un-pruned kernel's); returns evaluated / all candidates"""
@@ -147,7 +136,7 @@ def _check_pruned(oracle, b2, cur, ref, R, pmv=None, lam=0):
     return st["swept"] / st["all"]
 
 
-@pytest.mark.parametrize("ks", [1, 3, 5, 11, 13])
+@pytest.mark.parametrize("ks", [1, 3, 5])
 def test_block_sums_kernel(b2, ks):
     """K1a against numpy: minimum and maximum over ks rows of the 16x16 block sums of the padded plane"""
     rng = np.random.default_rng(5 + ks)
@@ -245,13 +234,3 @@ def test_pruned_synth_1080p(oracle, b2):
     assert np.array_equal(mv_a, mv_b) and np.array_equal(cost_a, cost_b)
     assert st["swept"] < 0.6 * st["all"], st
 
-
-def test_pruned_coarse_lane_tasks_are_bit_exact():
-    """B2_K1_PRUNE_ROWS=coarse: lane-tasks of 13 / 11 rows like the exhaustive kernel's (the default is 5 / 3); the switch is read once
-    per process, so the pruned tests are re-run in a child process"""
-    import os, subprocess, sys
-    env = dict(os.environ, B2_K1_PRUNE_ROWS="coarse")
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-m", "gpu", "-x", "-q", "-k", "pruned and not coarse"],
-                       capture_output=True, text=True, env=env, timeout=600, cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    assert " passed" in r.stdout

@@ -18,7 +18,7 @@ MBCOEF = np.dtype([("blk", "<i2", (26, 16))])
 
 
 def so_path():
-    return os.environ.get("B2ENC_LIB") or os.path.join(_HERE, "libb2enc.so")      # B2ENC_LIB: tuning variants (scripts/k1_variants.sh)
+    return os.environ.get("B2ENC_LIB") or os.path.join(_HERE, "libb2enc.so")      # B2ENC_LIB: a libb2enc.so built elsewhere
 
 
 def build(force=False):

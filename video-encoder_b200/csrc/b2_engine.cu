@@ -50,7 +50,7 @@ struct Group {
     int slot0 = 0, n = 0;
     cudaStream_t st = nullptr;
     CUtensorMap tm_cur, tm_ref[2];
-    CUtensorMap tm_sum, tm_cur_p, tm_ref_p[2];         // cfg.me_prune: (min | max) block-sum words; cur / window boxes of the pruned search's strips
+    CUtensorMap tm_sum;                    // cfg.me_prune: (min | max) block-sum words
     int ref_idx = 0;                       // d_rec[ref_idx] holds this group's latest reconstruction
     int res_set = 0, host_set = 0;
     int last_n = 0;                        // slots covered by the most recent encode
@@ -258,13 +258,8 @@ static int engine_alloc(b2_engine *e)
         if (b2_make_plane_tmap(&gr.tm_cur, e->d_cur[0] + gr.slot0 * e->stride_y, e->pitch, e->rows, gr.n, 16 * b2_k1_strip_mbs(c.merange), 16)) return -1;
         if (b2_make_plane_tmap(&gr.tm_ref[0], e->d_rec[0][0] + gr.slot0 * e->stride_y, e->pitch, e->rows, gr.n, bw, bh)) return -1;
         if (b2_make_plane_tmap(&gr.tm_ref[1], e->d_rec[1][0] + gr.slot0 * e->stride_y, e->pitch, e->rows, gr.n, bw, bh)) return -1;
-        if (e->d_sum) {
-            if (b2_make_plane_tmap32(&gr.tm_sum, e->d_sum + gr.slot0 * e->stride_y, e->pitch, e->rows, gr.n, b2_k1_mm_box(c.merange))) return -1;
-            const int pw = 16 * b2_k1_prune_strip_mbs(c.merange);
-            if (b2_make_plane_tmap(&gr.tm_cur_p, e->d_cur[0] + gr.slot0 * e->stride_y, e->pitch, e->rows, gr.n, pw, 16)) return -1;
-            for (int r = 0; r < 2; r++)
-                if (b2_make_plane_tmap(&gr.tm_ref_p[r], e->d_rec[r][0] + gr.slot0 * e->stride_y, e->pitch, e->rows, gr.n, pw + 2 * c.merange, bh)) return -1;
-        }
+        if (e->d_sum && b2_make_plane_tmap32(&gr.tm_sum, e->d_sum + gr.slot0 * e->stride_y, e->pitch, e->rows, gr.n, b2_k1_mm_box(c.merange)))
+            return -1;
     }
     return 0;
 }
@@ -619,7 +614,7 @@ static int encode_group(b2_engine *e, Group &gr, int frame_type, int ns, int rin
             if (e->d_sum) {
                 // lossless pruning: block sums of this step's reference planes, then the search over the surviving candidates
                 if (b2_launch_block_sums(b2_k1_prune_rows(c.merange), ref[0], e->pitch, e->rows, ns, e->d_sum + gr.slot0 * e->stride_y, st)) return -1;
-                if (b2_launch_me_fullpel_pruned(c.merange, &gr.tm_cur_p, &gr.tm_ref_p[gr.ref_idx], &gr.tm_sum, e->mbw, e->mbh, ns, e->d_prev_mv + om,
+                if (b2_launch_me_fullpel_pruned(c.merange, &gr.tm_cur, &gr.tm_ref[gr.ref_idx], &gr.tm_sum, e->mbw, e->mbh, ns, e->d_prev_mv + om,
                                                 e->lambda, e->d_mvf + om, e->d_cost_full + om, e->d_k1_swept, st))
                     return -1;
                 e->k1_all += b2_k1_candidates(c.merange, e->mbw, e->mbh, ns);

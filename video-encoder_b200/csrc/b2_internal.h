@@ -22,7 +22,6 @@ int b2_launch_me_fullpel(int R, const CUtensorMap *tm_cur, const CUtensorMap *tm
 int b2_make_plane_tmap32(CUtensorMap *tm, const void *base, int pitch, int rows, int nplanes, int bw);   // u32 planes, box {bw, 1, 1}
 extern "C" int b2_k1_prune_rows(int R);
 extern "C" int b2_k1_mm_box(int R);
-extern "C" int b2_k1_prune_strip_mbs(int R);              // strip width of the pruned search (its own cur / window boxes)
 extern "C" long long b2_k1_candidates(int R, int mbw, int mbh, int nframes);
 int b2_launch_block_sums(int ks, const uint8_t *d_planes, int pitch, int rows, int nplanes, uint32_t *d_mm /* [nplanes][rows][pitch] */,
                          cudaStream_t st);

@@ -119,9 +119,8 @@ static int me_fullpel_impl(const uint8_t *cur_y, const uint8_t *ref_y, int w, in
         B2_CUDA_OK(cudaMemcpy(d_pmv.p, pmv, nmb * sizeof(b2_mv_t), cudaMemcpyHostToDevice));
     }
     CUtensorMap tm_cur, tm_ref, tm_sum;
-    const int strip = prune ? b2_k1_prune_strip_mbs(merange) : b2_k1_strip_mbs(merange);     // the pruned search has its own strip width
-    if (b2_make_plane_tmap(&tm_cur, d_cur.p, pitch, rows, nframes, 16 * strip, 16)) return -1;
-    if (b2_make_plane_tmap(&tm_ref, d_ref.p, pitch, rows, nframes, 16 * strip + 2 * merange, bh)) return -1;
+    if (b2_make_plane_tmap(&tm_cur, d_cur.p, pitch, rows, nframes, 16 * b2_k1_strip_mbs(merange), 16)) return -1;
+    if (b2_make_plane_tmap(&tm_ref, d_ref.p, pitch, rows, nframes, bw, bh)) return -1;
     DevBuf d_sum, d_swept;
     if (prune) {
         if (mv9_out) return -1;

@@ -26,41 +26,32 @@
 //    The shared-memory pipe still runs at only 0.46 wavefronts/clk/SM while the ALU pipe is 92 % busy, so this is not the limiter --
 //    and the fix was measured to cost more than it saves: a pitch with K * pitch = 1 (mod 32) lines the two segments' banks up, but
 //    such a pitch is odd, so the expansion can no longer store 16 bytes per lane; bit-identical, 0.889 -> 0.868 of the VABSDIFF4 peak
-//    with word-wise expansion alone and 0.853 with the padded pitch (+-16: 0.836 -> 0.787; scripts/k1_exppad_probe.py,
-//    profiles/r2_k1_exppad_ab.txt).  The conflicts stay.
+//    with word-wise expansion alone and 0.853 with the padded pitch (+-16: 0.836 -> 0.787; profiles/r2_k1_exppad_ab.txt).
+//    The conflicts stay.
 //  * Winner: key = (cost << 13) | scan_index, CREDUX.MIN over the warp, atomicMin in smem.
 //    Lowest scan index wins ties by construction, exactly like the oracle's strict '<'.
-#include <stdlib.h>
-#include <string.h>
 #include <atomic>
 #include "b2_common.cuh"
 
 namespace {
 
-// Strip width and residency, tuned on the B200 (scripts/k1_variants.sh + k1_variant_probe.py, 1080p +-32, 32 frames):
+// Strip width and residency, tuned on the B200 (1080p +-32, 32 frames):
 //   NMB x CTAs/SM :  8x2 0.859   10x2 0.874   12x2 0.879   5x3 0.885   6x3 0.888   7x3 0.881   4x3 0.871   of the VABSDIFF4 peak.
 // Three resident CTAs (80 registers, 67 KB of shared memory each) keep the ALU pipe fed while one of them waits for its
 // TMA window / expands it; a wider strip only amortises the halo.
-#ifndef B2_K1_NMB
-#define B2_K1_NMB 6
-#endif
-#ifndef B2_K1_MINCTAS
-#define B2_K1_MINCTAS 3
-#endif
-#ifndef B2_K1_SMEM_PAD
-#define B2_K1_SMEM_PAD 0    // extra dynamic shared memory per CTA (bytes): lowers K1's residency without touching its register budget,
-#endif                      // so that other stream groups' kernels can co-reside (experiment knob, scripts/k1_variants.sh)
-#ifndef B2_K1_NMB16
-#define B2_K1_NMB16 10      // +-16: strips of 10 MBs.  Swept on the B200 with 192/256/320/384 threads (scripts/k1_r16_variant_probe.py,
-#endif                      // profiles/r2_k1_r16_strip_sweep.txt): 8 -> 0.821, 10 -> 0.838, 12 -> 0.817, 14 -> 0.829 of the VABSDIFF4 peak at 720p
-
+// +-16: strips of 10 MBs.  Swept on the B200 with 192/256/320/384 threads (profiles/r2_k1_r16_strip_sweep.txt):
+//   8 -> 0.821, 10 -> 0.838, 12 -> 0.817, 14 -> 0.829 of the VABSDIFF4 peak at 720p.
+// 256 threads per CTA: a sweep of 192/256/320/384 threads found the ALU pipe itself to be the plateau (256 and 384 both 0.85 of the
+// peak), not the rounding of 82 (+-32) / 41 (+-16) warp-tasks per full strip over the warps.
+constexpr int K1_THREADS = 256;
+constexpr int K1_MINCTAS = 3;
 template <int R> struct K1Cfg;
-// NMB = macroblocks per CTA strip (tuning: scripts/k1_variants.sh)
-template <> struct K1Cfg<32> { static constexpr int K = 13, NG = 5, NMB = B2_K1_NMB; };     // 65 = 5 x 13
-template <> struct K1Cfg<16> { static constexpr int K = 11, NG = 3, NMB = B2_K1_NMB16; };   // 33 = 3 x 11
+// NMB = macroblocks per CTA strip
+template <> struct K1Cfg<32> { static constexpr int K = 13, NG = 5, NMB = 6; };      // 65 = 5 x 13
+template <> struct K1Cfg<16> { static constexpr int K = 11, NG = 3, NMB = 10; };     // 33 = 3 x 11
 
-template <int R, int NMB_ = K1Cfg<R>::NMB> struct K1Smem {
-    static constexpr int NMB = NMB_;
+template <int R> struct K1Smem {
+    static constexpr int NMB = K1Cfg<R>::NMB;
     static constexpr int ND = 2 * R + 1;
     static constexpr int WIN_W = NMB * 16 + 2 * R;      // bytes per raw window row
     static constexpr int WIN_H = 16 + 2 * R;
@@ -83,8 +74,8 @@ template <int R, int NMB_ = K1Cfg<R>::NMB> struct K1Smem {
 // the nine shape parts (16x16 | 16x8 top,bottom | 8x16 left,right | four 8x8).  The number of VABSDIFF4 is unchanged; a lane
 // sweeps the top half of the current MB, packs the two 8x8 SADs of its K candidates into K registers, sweeps the bottom
 // half, and then forms 9 sums / keys per candidate (9 running minima, 9 CREDUX.MIN + 9 shared atomicMin per warp task).
-template <int R, int NTHREADS, bool PART>
-__global__ void __launch_bounds__(NTHREADS, PART ? 2 : B2_K1_MINCTAS)      // the partition variant needs ~90 registers: two CTAs
+template <int R, bool PART>
+__global__ void __launch_bounds__(K1_THREADS, PART ? 2 : K1_MINCTAS)      // the partition variant needs ~90 registers: two CTAs
 k1_me_fullpel_kernel(const __grid_constant__ CUtensorMap tm_cur,
                      const __grid_constant__ CUtensorMap tm_ref,
                      int mbw, int mbh, const b2_mv_t *__restrict__ pmv, int lambda,
@@ -92,7 +83,7 @@ k1_me_fullpel_kernel(const __grid_constant__ CUtensorMap tm_cur,
                      b2_mv_t *__restrict__ mv9_out, uint32_t *__restrict__ cost9_out)
 {
     using S = K1Smem<R>;
-    constexpr int NWARPS = NTHREADS / 32;
+    constexpr int NWARPS = K1_THREADS / 32;
     constexpr int K = K1Cfg<R>::K, NG = K1Cfg<R>::NG, ND = S::ND, NMB = K1Cfg<R>::NMB;
     static_assert(K * NG == ND, "dy groups must tile the search range");
 
@@ -123,7 +114,7 @@ k1_me_fullpel_kernel(const __grid_constant__ CUtensorMap tm_cur,
 
     // while the TMA is in flight: motion-vector cost tables and best-key init
     const size_t mb_base = ((size_t)frame * mbh + mby) * mbw + mb0;
-    for (int i = tid; i < NMB * ND; i += NTHREADS) {
+    for (int i = tid; i < NMB * ND; i += K1_THREADS) {
         int m = i / ND, d = i - m * ND;
         int px = 0, py = 0;
         if (pmv != nullptr && m < nmb) { b2_mv_t p = pmv[mb_base + m]; px = p.x; py = p.y; }
@@ -139,7 +130,7 @@ k1_me_fullpel_kernel(const __grid_constant__ CUtensorMap tm_cur,
     {
         constexpr int WPR = S::WIN_W / 4;             // aligned words per raw row
         const uint32_t *raw32 = (const uint32_t *)s_raw;
-        for (int i = tid; i < WPR * S::WIN_H; i += NTHREADS) {
+        for (int i = tid; i < WPR * S::WIN_H; i += K1_THREADS) {
             int r = i / WPR, j = i - r * WPR;
             uint32_t lo = raw32[i], hi = raw32[i + 1];    // last word of the buffer: 16 B slack
             uint4 o;
@@ -306,218 +297,6 @@ k1_me_fullpel_kernel(const __grid_constant__ CUtensorMap tm_cur,
     }
 }
 
-// ---- persistent, software-pipelined form of the single-vector search ------------------------------------------------------
-// One CTA per SM walks a list of strips.  A PRODUCER warp fetches strip k+1 (TMA raw window + current tile), expands the
-// window, fills the cost tables and publishes the buffer through an mbarrier while NCW CONSUMER warps still sweep strip k out
-// of the other buffer; consumers take warp-tasks from one global sequence (task T -> strip T / TPS), so they drift across the
-// strip boundary without a CTA-wide barrier and the ALU pipe never sees a strip prologue.  Each finished task arrives on the
-// buffer's "empty" barrier; when all TPS tasks of a strip are in, the producer writes that strip's vectors and refills the
-// buffer.  Arithmetic, scan order and tie-break are those of k1_me_fullpel_kernel.
-__device__ __forceinline__ void mbar_arrive(uint64_t *bar)
-{
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-
-template <int R> struct K1PSmem {
-    using S1 = K1Smem<R>;
-    static constexpr int NMB = S1::NMB, ND = S1::ND;
-    static constexpr int TAB = NMB * ND * 4;
-    static constexpr int OFF_RAW = 0;
-    static constexpr int BUF0 = (S1::RAW_BYTES + 16 + 127) & ~127;
-    // per buffer: cur | exp | costx | costy | best
-    static constexpr int B_CUR = 0;
-    static constexpr int B_EXP = S1::CUR_BYTES;
-    static constexpr int B_COSTX = B_EXP + S1::EXP_BYTES;
-    static constexpr int B_COSTY = B_COSTX + TAB;
-    static constexpr int B_BEST = B_COSTY + TAB;
-    static constexpr int BUF_BYTES = (B_BEST + NMB * 4 + 127) & ~127;
-    static constexpr int NBUF = 3;                           // strips in flight: one being swept, two prepared ahead
-    static constexpr int OFF_BAR = BUF0 + NBUF * BUF_BYTES;  // full[NBUF], empty[NBUF], tma
-    static constexpr int TOTAL = OFF_BAR + (2 * NBUF + 1) * 8 + 128;      // +128: manual alignment slack
-};
-
-constexpr int K1P_PW = 4;                                   // producer warps
-__device__ __forceinline__ void producer_sync() { asm volatile("bar.sync 1, %0;" ::"n"(K1P_PW * 32) : "memory"); }
-
-template <int R, int NCW>
-__global__ void __launch_bounds__((NCW + K1P_PW) * 32, 1)
-k1_me_fullpel_persistent_kernel(const __grid_constant__ CUtensorMap tm_cur, const __grid_constant__ CUtensorMap tm_ref,
-                                int mbw, int mbh, int nframes, const b2_mv_t *__restrict__ pmv, int lambda,
-                                b2_mv_t *__restrict__ mv_out, uint32_t *__restrict__ cost_out)
-{
-    using S = K1Smem<R>;
-    using P = K1PSmem<R>;
-    constexpr int K = K1Cfg<R>::K, NG = K1Cfg<R>::NG, ND = S::ND, NMB = K1Cfg<R>::NMB;
-    constexpr int TPS = (NMB * NG * ND + 31) / 32;              // warp-tasks of a full strip (ragged strips pad with no-ops)
-
-    extern __shared__ uint8_t smem_raw_[];
-    uint8_t *smem = smem_raw_ + ((128u - (smem_u32(smem_raw_) & 127u)) & 127u);
-    uint8_t *s_raw = smem + P::OFF_RAW;
-    constexpr int NBUF = P::NBUF;
-    uint64_t *s_full = (uint64_t *)(smem + P::OFF_BAR), *s_empty = s_full + NBUF, *s_tma = s_full + 2 * NBUF;
-
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int spr = (mbw + NMB - 1) / NMB;                       // strips per macroblock row
-    const int nstrips = spr * mbh * nframes;
-    const int mine = nstrips > (int)blockIdx.x ? (nstrips - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;   // strips of this CTA
-
-    if (tid == 0) {
-        for (int b = 0; b < NBUF; b++) { mbar_init(&s_full[b], 1); mbar_init(&s_empty[b], TPS); }
-        mbar_init(s_tma, 1);
-        fence_mbar_init();
-    }
-    __syncthreads();
-
-    if (warp >= NCW) {
-        // ================= producer warps =================
-        const int ptid = tid - NCW * 32;                         // 0 .. K1P_PW*32-1
-        __shared__ int s_pmv[2][16];                             // predictors of the strip being prepared (NMB <= 16)
-        static_assert(NMB <= 16, "strip wider than the predictor staging");
-        for (int k = 0; k < mine + NBUF; k++) {
-            const int buf = k % NBUF, use = k / NBUF;
-            uint8_t *bb = smem + P::BUF0 + buf * P::BUF_BYTES;
-            uint32_t *s_best = (uint32_t *)(bb + P::B_BEST);
-            if (k >= NBUF) {
-                // all tasks of strip k-NBUF have arrived: write its vectors, then the buffer is free
-                mbar_wait(&s_empty[buf], (uint32_t)((use - 1) & 1));
-                const int sidx = (int)blockIdx.x + (k - NBUF) * (int)gridDim.x;
-                const int frame = sidx / (spr * mbh), rem = sidx - frame * (spr * mbh);
-                const int mby = rem / spr, mb0 = (rem - mby * spr) * NMB;
-                const int nmb = min(NMB, mbw - mb0);
-                if (ptid < nmb) {
-                    const uint32_t key = s_best[ptid];
-                    const int idx = (int)(key & 8191u);
-                    const int dyi = idx / ND, dxi = idx - dyi * ND;
-                    b2_mv_t mv;
-                    mv.x = (int16_t)(dxi - R); mv.y = (int16_t)(dyi - R);
-                    const size_t o = ((size_t)frame * mbh + mby) * mbw + mb0 + ptid;
-                    mv_out[o] = mv; cost_out[o] = key >> 13;
-                }
-                producer_sync();                                 // the keys are read before the buffer is refilled
-            }
-            if (k >= mine) continue;
-            const int sidx = (int)blockIdx.x + k * (int)gridDim.x;
-            const int frame = sidx / (spr * mbh), rem = sidx - frame * (spr * mbh);
-            const int mby = rem / spr, mb0 = (rem - mby * spr) * NMB;
-            const int nmb = min(NMB, mbw - mb0);
-            uint8_t *s_cur = bb + P::B_CUR;
-            uint32_t *s_exp = (uint32_t *)(bb + P::B_EXP);
-            uint32_t *s_costx = (uint32_t *)(bb + P::B_COSTX), *s_costy = (uint32_t *)(bb + P::B_COSTY);
-            if (ptid == 0) {
-                fence_proxy_async();                             // earlier generic reads of raw / cur before the async writes
-                mbar_expect_tx(s_tma, S::RAW_BYTES + S::CUR_BYTES);
-                tma_load_3d(s_raw, &tm_ref, B2_PAD + mb0 * 16 - R, B2_PAD + mby * 16 - R, frame, s_tma);
-                tma_load_3d(s_cur, &tm_cur, B2_PAD + mb0 * 16, B2_PAD + mby * 16, frame, s_tma);
-            }
-            // while the TMA is in flight: predictors (one global load per macroblock), cost tables and best keys
-            const size_t mb_base = ((size_t)frame * mbh + mby) * mbw + mb0;
-            if (ptid < NMB) {
-                int px = 0, py = 0;
-                if (pmv != nullptr && ptid < nmb) { const b2_mv_t pp = pmv[mb_base + ptid]; px = pp.x; py = pp.y; }
-                s_pmv[0][ptid] = px; s_pmv[1][ptid] = py;
-                s_best[ptid] = 0xffffffffu;
-            }
-            producer_sync();
-            for (int i = ptid; i < NMB * ND; i += K1P_PW * 32) {
-                const int m = i / ND, d = i - m * ND;
-                s_costx[i] = ((uint32_t)(lambda * b2_mvbits(4 * (d - R) - s_pmv[0][m])) << 13) + (uint32_t)d;
-                s_costy[i] = ((uint32_t)(lambda * b2_mvbits(4 * (d - R) - s_pmv[1][m])) << 13) + (uint32_t)(d * ND);
-            }
-            mbar_wait(s_tma, (uint32_t)(k & 1));
-            {   // expand: word x of a row = pixels x..x+3 (little endian), all 4 byte alignments
-                constexpr int WPR = S::WIN_W / 4;
-                const uint32_t *raw32 = (const uint32_t *)s_raw;
-                for (int i = ptid; i < WPR * S::WIN_H; i += K1P_PW * 32) {
-                    const int r = i / WPR, j = i - r * WPR;
-                    const uint32_t lo = raw32[i], hi = raw32[i + 1];
-                    uint4 o;
-                    o.x = lo; o.y = __funnelshift_r(lo, hi, 8); o.z = __funnelshift_r(lo, hi, 16); o.w = __funnelshift_r(lo, hi, 24);
-                    *(uint4 *)(s_exp + r * S::EXP_PITCH + 4 * j) = o;
-                }
-            }
-            producer_sync();                                     // every producer thread's stores precede the release below
-            if (ptid == 0) mbar_arrive(&s_full[buf]);            // release: the buffer is complete
-        }
-        return;
-    }
-
-    // ================= consumer warps =================
-    // per-warp state is kept small (one buffer offset instead of six pointers): the sweep itself needs ~75 registers
-    int cur_k = -1, nmb = 0, bo = 0;
-    const int ntasks = mine * TPS;
-    for (int T = warp; T < ntasks; T += NCW) {
-        const int k = T / TPS, t0 = (T - k * TPS) * 32;
-        if (k != cur_k) {
-            cur_k = k;
-            mbar_wait(&s_full[k % NBUF], (uint32_t)((k / NBUF) & 1));
-            bo = P::BUF0 + (k % NBUF) * P::BUF_BYTES;
-            const int sidx = (int)blockIdx.x + k * (int)gridDim.x;
-            nmb = min(NMB, mbw - (sidx % spr) * NMB);
-        }
-        const uint8_t *s_cur = smem + bo + P::B_CUR;
-        const uint32_t *s_exp = (const uint32_t *)(smem + bo + P::B_EXP);
-        const uint32_t *s_costx = (const uint32_t *)(smem + bo + P::B_COSTX), *s_costy = (const uint32_t *)(smem + bo + P::B_COSTY);
-        uint32_t *s_best = (uint32_t *)(smem + bo + P::B_BEST);
-        const int total = nmb * NG * ND;
-        if (t0 < total) {
-            const int t = t0 + lane;
-            const bool active = t < total;
-            const int tt = active ? t : t0;               // idle lanes shadow lane 0's task
-            const int m = tt / (NG * ND);
-            const int rem = tt - m * (NG * ND);
-            const int g = rem / ND;
-            const int dxi = rem - g * ND;
-            uint32_t cur[64];
-            {
-                const uint4 *c4 = (const uint4 *)(s_cur + m * 16);
-#pragma unroll
-                for (int y = 0; y < 16; y++) {
-                    uint4 v = c4[y * (NMB * 16 / 16)];
-                    cur[y * 4 + 0] = v.x; cur[y * 4 + 1] = v.y; cur[y * 4 + 2] = v.z; cur[y * 4 + 3] = v.w;
-                }
-            }
-            uint32_t acc[K];
-#pragma unroll
-            for (int kk = 0; kk < K; kk++) acc[kk] = 0;
-            const uint32_t *wp = s_exp + (g * K) * S::EXP_PITCH + m * 16 + dxi;
-#pragma unroll
-            for (int r = 0; r < K + 15; r++) {
-                const uint32_t w0 = wp[r * S::EXP_PITCH + 0];
-                const uint32_t w1 = wp[r * S::EXP_PITCH + 4];
-                const uint32_t w2 = wp[r * S::EXP_PITCH + 8];
-                const uint32_t w3 = wp[r * S::EXP_PITCH + 12];
-#pragma unroll
-                for (int kk = 0; kk < K; kk++) {
-                    const int y = r - kk;
-                    if (y >= 0 && y < 16) {
-                        acc[kk] = vsad4_acc(w0, cur[y * 4 + 0], acc[kk]);
-                        acc[kk] = vsad4_acc(w1, cur[y * 4 + 1], acc[kk]);
-                        acc[kk] = vsad4_acc(w2, cur[y * 4 + 2], acc[kk]);
-                        acc[kk] = vsad4_acc(w3, cur[y * 4 + 3], acc[kk]);
-                    }
-                }
-            }
-            uint32_t key = 0xffffffffu;
-            if (active) {
-                const uint32_t kx = s_costx[m * ND + dxi];
-                const uint32_t *ky = s_costy + m * ND + g * K;
-#pragma unroll
-                for (int kk = 0; kk + 1 < K; kk += 2) key = __vimin3_u32(key, acc[kk] * 8192u + (kx + ky[kk]), acc[kk + 1] * 8192u + (kx + ky[kk + 1]));
-                if (K & 1) key = min(key, acc[K - 1] * 8192u + (kx + ky[K - 1]));
-            }
-            const int m0 = __shfl_sync(0xffffffffu, m, 0);
-            if (__all_sync(0xffffffffu, m == m0)) {
-                const uint32_t wmin = __reduce_min_sync(0xffffffffu, key);
-                if (lane == 0) atomicMin(&s_best[m0], wmin);
-            } else if (active) {
-                atomicMin(&s_best[m], key);
-            }
-        }
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&s_empty[k % NBUF]);          // release: this task's reads and atomics are done
-    }
-}
-
 // ---- lossless pruning: successive elimination in front of the same sweep (engine option me_prune) ---------------------------
 // |sum(cur MB) - sum(ref block)| <= SAD(cur MB, ref block) (triangle inequality), so a candidate whose
 //     |C - S(dx,dy)| + mvcost(dx,dy)  >  U,     U = exact cost of any candidate already evaluated,
@@ -540,32 +319,20 @@ k1_me_fullpel_persistent_kernel(const __grid_constant__ CUtensorMap tm_cur, cons
 //      macroblocks they work on (a plain survivor list gave 1.9 wavefronts per load: the band of survivors of neighbouring dy groups
 //      overlaps in x; ncu: profiles/r2_k1_pruned_ncu.txt).  Queues that overflow (more than QCAP survivors: predictors that point
 //      nowhere) make the strip fall back to sweeping every lane-task in natural order.
-// KS (rows per lane-task) is a template parameter: fewer rows = finer pruning but fewer VABSDIFF4 per shared-memory load
-// (13 -> 5 rows: 7.4 -> 4.0 per LDS.32, still ALU-bound when the loads are conflict-free).  What is skipped is reported, never
-// folded into the roofline figure: `swept` counts the candidates that ran (b2_engine_k1_stats).
-#ifndef B2_K1_PRUNE_MINCTAS
-#define B2_K1_PRUNE_MINCTAS 3
-#endif
-// reference rows after which the exit is tested: K + FIRST, K + FIRST + STEP, ... <= K + LAST (every candidate has then seen at least
-// FIRST + 1 rows); swept on the B200: profiles/r2_k1_pde_schedule.txt
-#ifndef B2_K1_PDE_FIRST
-#define B2_K1_PDE_FIRST 5
-#endif
-#ifndef B2_K1_PDE_LAST
-#define B2_K1_PDE_LAST 9
-#endif
-#ifndef B2_K1_PDE_STEP
-#define B2_K1_PDE_STEP 4
-#endif
-#ifndef B2_K1_PRUNE_PDE
-#define B2_K1_PRUNE_PDE 1     // partial-distortion exit inside the sweep (0: every surviving lane-task is swept to the end)
-#endif
-template <int R> struct K1PruneCfg { static constexpr int NMB = K1Cfg<R>::NMB; };        // the exhaustive kernel's strips (and tensor maps)
+// What is skipped is reported, never folded into the roofline figure: `swept` counts the candidates that ran (b2_engine_k1_stats).
+// KS (rows per lane-task): 5 (+-32) / 3 (+-16) instead of the exhaustive kernel's 13 / 11.  Fewer rows = finer pruning but fewer
+// VABSDIFF4 per shared-memory load (13 -> 5 rows: 7.4 -> 4.0 per LDS.32, still ALU-bound when the loads are conflict-free); measured
+// faster at 1080p +-32: 0.871 -> 0.803 ms on the synthetic pan, 0.908 -> 0.886 ms on natural-like content (profiles/r2_k1_pruned_forms.txt).
+template <int R> constexpr int K1_PRUNE_KS = R == 32 ? 5 : 3;
+constexpr int K1_PRUNE_MINCTAS = 3;
+// partial-distortion exit inside the sweep: reference rows after which it is tested, K + FIRST, K + FIRST + STEP, ... <= K + LAST
+// (every candidate has then seen at least FIRST + 1 rows); swept on the B200: profiles/r2_k1_pde_schedule.txt
+constexpr int K1_PDE_FIRST = 5, K1_PDE_LAST = 9, K1_PDE_STEP = 4;
 
 constexpr int k1_cmax(int a, int b) { return a > b ? a : b; }
 template <int R, int KS> struct K1SeaSmem {
-    static constexpr int NMB = K1PruneCfg<R>::NMB;
-    using S = K1Smem<R, NMB>;
+    using S = K1Smem<R>;                                          // the exhaustive kernel's strips (and tensor maps)
+    static constexpr int NMB = S::NMB;
     static constexpr int ND = S::ND, NG = ND / KS;
     static_assert(NG * KS == ND, "dy groups must tile the search range");
     static_assert(S::EXP_PITCH % 32 == 0, "bank queues need expanded rows of a multiple of 32 words");
@@ -594,17 +361,17 @@ template <int R, int KS> struct K1SeaSmem {
     static constexpr int OFF_BAR = (OFF_CNT + 33 * 4 + 7) & ~7;
     static constexpr int TOTAL = OFF_BAR + 16 + 128;             // +128: manual alignment slack
 };
-static_assert(B2_K1_PRUNE_MINCTAS * (K1SeaSmem<32, 5>::TOTAL + 1024) <= 228 * 1024, "pruned K1 (+-32, 5 rows): the CTAs per SM asked for do not fit");
+static_assert(K1_PRUNE_MINCTAS * (K1SeaSmem<32, K1_PRUNE_KS<32>>::TOTAL + 1024) <= 228 * 1024, "pruned K1 (+-32, 5 rows): the CTAs per SM asked for do not fit");
 
-template <int R, int KS, int NTHREADS>
-__global__ void __launch_bounds__(NTHREADS, B2_K1_PRUNE_MINCTAS)
+template <int R, int KS>
+__global__ void __launch_bounds__(K1_THREADS, K1_PRUNE_MINCTAS)
 k1_me_fullpel_sea_kernel(const __grid_constant__ CUtensorMap tm_cur, const __grid_constant__ CUtensorMap tm_ref,
                          const __grid_constant__ CUtensorMap tm_mm, int mbw, int mbh, const b2_mv_t *__restrict__ pmv, int lambda,
                          b2_mv_t *__restrict__ mv_out, uint32_t *__restrict__ cost_out, unsigned long long *__restrict__ swept)
 {
     using Q = K1SeaSmem<R, KS>;
     using S = typename Q::S;
-    constexpr int NWARPS = NTHREADS / 32;
+    constexpr int NWARPS = K1_THREADS / 32;
     constexpr int K = KS, NG = Q::NG, ND = S::ND, NMB = Q::NMB, QCAP = Q::QCAP;
 
     extern __shared__ uint8_t smem_raw_[];
@@ -647,7 +414,7 @@ k1_me_fullpel_sea_kernel(const __grid_constant__ CUtensorMap tm_cur, const __gri
         tma_load_3d(s_cur, &tm_cur, B2_PAD + mb0 * 16, B2_PAD + mby * 16, frame, &s_bar[0]);
     }
 
-    for (int i = tid; i < NMB * ND; i += NTHREADS) {
+    for (int i = tid; i < NMB * ND; i += K1_THREADS) {
         const int m = i / ND, d = i - m * ND;
         s_costx[i] = ((uint32_t)(lambda * b2_mvbits(4 * (d - R) - s_pmv[2 * m])) << 13) + (uint32_t)d;
         s_costy[i] = ((uint32_t)(lambda * b2_mvbits(4 * (d - R) - s_pmv[2 * m + 1])) << 13) + (uint32_t)(d * ND);
@@ -657,7 +424,7 @@ k1_me_fullpel_sea_kernel(const __grid_constant__ CUtensorMap tm_cur, const __gri
     {
         constexpr int WPR = S::WIN_W / 4;
         const uint32_t *raw32 = (const uint32_t *)s_raw;
-        for (int i = tid; i < WPR * S::WIN_H; i += NTHREADS) {
+        for (int i = tid; i < WPR * S::WIN_H; i += K1_THREADS) {
             int r = i / WPR, j = i - r * WPR;
             uint32_t lo = raw32[i], hi = raw32[i + 1];
             uint4 o;
@@ -795,7 +562,7 @@ k1_me_fullpel_sea_kernel(const __grid_constant__ CUtensorMap tm_cur, const __gri
                     acc[k] = vsad4_acc(w3, cur[y * 4 + 3], acc[k]);
                 }
             }
-            if (B2_K1_PRUNE_PDE && r >= K + B2_K1_PDE_FIRST && r <= K + B2_K1_PDE_LAST && ((r - (K + B2_K1_PDE_FIRST)) % B2_K1_PDE_STEP) == 0) {
+            if (r >= K + K1_PDE_FIRST && r <= K + K1_PDE_LAST && ((r - (K + K1_PDE_FIRST)) % K1_PDE_STEP) == 0) {
                 bool hopeless = true;
                 if (active) {
                     const uint32_t bk = ((volatile uint32_t *)s_best)[m];
@@ -947,43 +714,7 @@ __global__ void __launch_bounds__(256) k1a_block_sums_kernel(const uint8_t *__re
     }
 }
 
-#ifndef B2_K1P_WARPS
-#define B2_K1P_WARPS 16      // 16 consumer warps (92 registers, no spills) + 4 producer warps; 20 consumers fit only at 80 registers
-#endif
-template <int R>
-int launch_k1_persistent(const CUtensorMap &tm_cur, const CUtensorMap &tm_ref, int mbw, int mbh, int nframes, const b2_mv_t *pmv,
-                         int lambda, b2_mv_t *mv_out, uint32_t *cost_out, cudaStream_t st)
-{
-    static std::atomic<int> nsm[64];                          // SM count per device, 0 = not looked up yet
-    int dev = 0;
-    B2_CUDA_OK(cudaGetDevice(&dev));
-    int sms = (dev >= 0 && dev < 64) ? nsm[dev].load(std::memory_order_acquire) : 0;
-    if (!sms) {
-        B2_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-        B2_CUDA_OK(cudaFuncSetAttribute(k1_me_fullpel_persistent_kernel<R, B2_K1P_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                        K1PSmem<R>::TOTAL));
-        if (dev >= 0 && dev < 64) nsm[dev].store(sms, std::memory_order_release);
-    }
-    constexpr int NMB = K1Cfg<R>::NMB;
-    const int nstrips = ((mbw + NMB - 1) / NMB) * mbh * nframes;
-    const int grid = nstrips < sms ? nstrips : sms;
-    k1_me_fullpel_persistent_kernel<R, B2_K1P_WARPS><<<grid, (B2_K1P_WARPS + K1P_PW) * 32, K1PSmem<R>::TOTAL, st>>>(
-        tm_cur, tm_ref, mbw, mbh, nframes, pmv, lambda, mv_out, cost_out);
-    B2_CUDA_OK(cudaGetLastError());
-    return 0;
-}
-
-// B2_K1_PERSISTENT=1 selects the persistent, pipelined kernel for the single-vector search.  Measured on the B200 (1080p, +-32,
-// 64 frames per launch): 0.889 of the VABSDIFF4 peak with 16 consumer + 4 producer warps and three buffers (0.866 with two
-// buffers and two producer warps, 0.861 with 20 consumer warps at 80 registers) against 0.888 for one strip per CTA x 3 resident
-// CTAs, and 5,333 vs 5,361 frames/s for the whole step: both forms sit at the same ceiling, so the simpler one stays the default.
-int k1_persistent()
-{
-    static const int v = [] { const char *e = getenv("B2_K1_PERSISTENT"); return e ? atoi(e) : 0; }();
-    return v;
-}
-
-template <int R, int NT, bool PART>
+template <int R, bool PART>
 int launch_k1p(const CUtensorMap &tm_cur, const CUtensorMap &tm_ref, int mbw, int mbh, int nframes, const b2_mv_t *pmv, int lambda,
                b2_mv_t *mv_out, uint32_t *cost_out, b2_mv_t *mv9_out, uint32_t *cost9_out, cudaStream_t st)
 {
@@ -992,60 +723,42 @@ int launch_k1p(const CUtensorMap &tm_cur, const CUtensorMap &tm_ref, int mbw, in
     int dev = 0;
     B2_CUDA_OK(cudaGetDevice(&dev));
     if (dev < 0 || dev >= 64 || !attr_set[dev].load(std::memory_order_acquire)) {
-        B2_CUDA_OK(cudaFuncSetAttribute(k1_me_fullpel_kernel<R, NT, PART>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                        K1Smem<R>::TOTAL + B2_K1_SMEM_PAD));
+        B2_CUDA_OK(cudaFuncSetAttribute(k1_me_fullpel_kernel<R, PART>, cudaFuncAttributeMaxDynamicSharedMemorySize, K1Smem<R>::TOTAL));
         if (dev >= 0 && dev < 64) attr_set[dev].store(true, std::memory_order_release);
     }
     constexpr int NMB = K1Cfg<R>::NMB;
     dim3 grid((mbw + NMB - 1) / NMB, mbh, nframes);
-    k1_me_fullpel_kernel<R, NT, PART><<<grid, NT, K1Smem<R>::TOTAL + B2_K1_SMEM_PAD, st>>>(tm_cur, tm_ref, mbw, mbh, pmv, lambda, mv_out, cost_out,
-                                                                            mv9_out, cost9_out);
+    k1_me_fullpel_kernel<R, PART><<<grid, K1_THREADS, K1Smem<R>::TOTAL, st>>>(tm_cur, tm_ref, mbw, mbh, pmv, lambda, mv_out, cost_out,
+                                                                              mv9_out, cost9_out);
     B2_CUDA_OK(cudaGetLastError());
     return 0;
 }
-template <int R, int NT>
+template <int R>
 int launch_k1(const CUtensorMap &tm_cur, const CUtensorMap &tm_ref, int mbw, int mbh, int nframes, const b2_mv_t *pmv, int lambda,
               b2_mv_t *mv_out, uint32_t *cost_out, b2_mv_t *mv9_out, uint32_t *cost9_out, cudaStream_t st)
 {
-    if (mv9_out) return launch_k1p<R, NT, true>(tm_cur, tm_ref, mbw, mbh, nframes, pmv, lambda, mv_out, cost_out, mv9_out, cost9_out, st);
-    return launch_k1p<R, NT, false>(tm_cur, tm_ref, mbw, mbh, nframes, pmv, lambda, mv_out, cost_out, nullptr, nullptr, st);
+    if (mv9_out) return launch_k1p<R, true>(tm_cur, tm_ref, mbw, mbh, nframes, pmv, lambda, mv_out, cost_out, mv9_out, cost9_out, st);
+    return launch_k1p<R, false>(tm_cur, tm_ref, mbw, mbh, nframes, pmv, lambda, mv_out, cost_out, nullptr, nullptr, st);
 }
 
-template <int R, int KS, int NT>
+template <int R>
 int launch_k1_sea(const CUtensorMap &tm_cur, const CUtensorMap &tm_ref, const CUtensorMap &tm_mm, int mbw, int mbh, int nframes,
                   const b2_mv_t *pmv, int lambda, b2_mv_t *mv_out, uint32_t *cost_out, unsigned long long *swept, cudaStream_t st)
 {
+    constexpr int KS = K1_PRUNE_KS<R>;
     static std::atomic<bool> attr_set[64];
     int dev = 0;
     B2_CUDA_OK(cudaGetDevice(&dev));
     if (dev < 0 || dev >= 64 || !attr_set[dev].load(std::memory_order_acquire)) {
-        B2_CUDA_OK(cudaFuncSetAttribute(k1_me_fullpel_sea_kernel<R, KS, NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, K1SeaSmem<R, KS>::TOTAL));
+        B2_CUDA_OK(cudaFuncSetAttribute(k1_me_fullpel_sea_kernel<R, KS>, cudaFuncAttributeMaxDynamicSharedMemorySize, K1SeaSmem<R, KS>::TOTAL));
         if (dev >= 0 && dev < 64) attr_set[dev].store(true, std::memory_order_release);
     }
-    constexpr int NMB = K1PruneCfg<R>::NMB;
+    constexpr int NMB = K1Cfg<R>::NMB;
     dim3 grid((mbw + NMB - 1) / NMB, mbh, nframes);
-    k1_me_fullpel_sea_kernel<R, KS, NT><<<grid, NT, K1SeaSmem<R, KS>::TOTAL, st>>>(tm_cur, tm_ref, tm_mm, mbw, mbh, pmv, lambda, mv_out, cost_out, swept);
+    k1_me_fullpel_sea_kernel<R, KS><<<grid, K1_THREADS, K1SeaSmem<R, KS>::TOTAL, st>>>(tm_cur, tm_ref, tm_mm, mbw, mbh, pmv, lambda, mv_out,
+                                                                                       cost_out, swept);
     B2_CUDA_OK(cudaGetLastError());
     return 0;
-}
-
-// rows per lane-task of the pruned search: B2_K1_PRUNE_ROWS = "coarse" keeps the exhaustive kernel's 13 (+-32) / 11 (+-16), the
-// default "fine" uses 5 / 3 (A/B: scripts/k1_prune_probe.py, profiles/r2_k1_prune_probe.txt)
-int k1_prune_fine()
-{
-    static const int v = [] { const char *e = getenv("B2_K1_PRUNE_ROWS"); return !(e && !strcmp(e, "coarse")); }();
-    return v;
-}
-
-// threads per CTA: 82 (R=32) / 41 (R=16) warp-tasks per full strip should divide evenly over the warps
-int k1_threads()
-{
-    static const int nt = [] {                          // thread-safe one-time initialisation
-        const char *e = getenv("B2_K1_THREADS");
-        const int v = e ? atoi(e) : 256;
-        return (v == 192 || v == 256 || v == 320 || v == 384) ? v : 256;
-    }();
-    return nt;
 }
 
 }  // namespace
@@ -1067,17 +780,9 @@ int b2_launch_me_fullpel(int R, const CUtensorMap *tm_cur, const CUtensorMap *tm
                          int nframes, const b2_mv_t *d_pmv, int lambda, b2_mv_t *d_mv, uint32_t *d_cost,
                          b2_mv_t *d_mv9, uint32_t *d_cost9, cudaStream_t st)
 {
-#define K1_DISPATCH(RR)                                                                                              \
-    if (!d_mv9 && k1_persistent()) return launch_k1_persistent<RR>(*tm_cur, *tm_ref, mbw, mbh, nframes, d_pmv, lambda, d_mv, d_cost, st); \
-    switch (k1_threads()) {                                                                                          \
-    case 192: return launch_k1<RR, 192>(*tm_cur, *tm_ref, mbw, mbh, nframes, d_pmv, lambda, d_mv, d_cost, d_mv9, d_cost9, st);       \
-    case 320: return launch_k1<RR, 320>(*tm_cur, *tm_ref, mbw, mbh, nframes, d_pmv, lambda, d_mv, d_cost, d_mv9, d_cost9, st);       \
-    case 384: return launch_k1<RR, 384>(*tm_cur, *tm_ref, mbw, mbh, nframes, d_pmv, lambda, d_mv, d_cost, d_mv9, d_cost9, st);       \
-    default: return launch_k1<RR, 256>(*tm_cur, *tm_ref, mbw, mbh, nframes, d_pmv, lambda, d_mv, d_cost, d_mv9, d_cost9, st);        \
-    }
     switch (R) {
-    case 32: K1_DISPATCH(32)
-    case 16: K1_DISPATCH(16)
+    case 32: return launch_k1<32>(*tm_cur, *tm_ref, mbw, mbh, nframes, d_pmv, lambda, d_mv, d_cost, d_mv9, d_cost9, st);
+    case 16: return launch_k1<16>(*tm_cur, *tm_ref, mbw, mbh, nframes, d_pmv, lambda, d_mv, d_cost, d_mv9, d_cost9, st);
     default:
         fprintf(stderr, "b2enc: merange %d not supported (16 or 32)\n", R);
         return -1;
@@ -1088,27 +793,23 @@ int b2_launch_me_fullpel(int R, const CUtensorMap *tm_cur, const CUtensorMap *tm
 // rows per lane-task the pruned search uses for +-R (K1a has to be run with the same number)
 extern "C" int b2_k1_prune_rows(int R)
 {
-    if (R == 32) return k1_prune_fine() ? 5 : K1Cfg<32>::K;
-    if (R == 16) return k1_prune_fine() ? 3 : K1Cfg<16>::K;
+    if (R == 32) return K1_PRUNE_KS<32>;
+    if (R == 16) return K1_PRUNE_KS<16>;
     return -1;
 }
 // words per row of the (min | max) box a strip fetches (the box is {this, 1, 1}; a strip issues one per dy group)
 extern "C" int b2_k1_mm_box(int R)
 {
-    if (R == 32) return K1SeaSmem<32, 13>::MP;
-    if (R == 16) return K1SeaSmem<16, 11>::MP;
+    if (R == 32) return K1SeaSmem<32, K1_PRUNE_KS<32>>::MP;
+    if (R == 16) return K1SeaSmem<16, K1_PRUNE_KS<16>>::MP;
     return -1;
 }
-// macroblocks per strip of the pruned search: its current-tile box is {16 * this, 16, 1}, its window box {16 * this + 2R, 16 + 2R, 1}
-extern "C" int b2_k1_prune_strip_mbs(int R) { return R == 16 ? K1PruneCfg<16>::NMB : K1PruneCfg<32>::NMB; }
 
 int b2_launch_block_sums(int ks, const uint8_t *d_planes, int pitch, int rows, int nplanes, uint32_t *d_mm, cudaStream_t st)
 {
     dim3 grid((pitch + K1A_TW - 1) / K1A_TW, (rows + K1A_TH - 1) / K1A_TH, nplanes);
     const size_t stride = (size_t)pitch * rows;
     switch (ks) {
-    case 13: k1a_block_sums_kernel<13><<<grid, 256, 0, st>>>(d_planes, pitch, rows, stride, d_mm); break;
-    case 11: k1a_block_sums_kernel<11><<<grid, 256, 0, st>>>(d_planes, pitch, rows, stride, d_mm); break;
     case 5: k1a_block_sums_kernel<5><<<grid, 256, 0, st>>>(d_planes, pitch, rows, stride, d_mm); break;
     case 3: k1a_block_sums_kernel<3><<<grid, 256, 0, st>>>(d_planes, pitch, rows, stride, d_mm); break;
     case 1: k1a_block_sums_kernel<1><<<grid, 256, 0, st>>>(d_planes, pitch, rows, stride, d_mm); break;      // the plain block sums (tests)
@@ -1128,20 +829,9 @@ int b2_launch_me_fullpel_pruned(int R, const CUtensorMap *tm_cur, const CUtensor
                                 int nframes, const b2_mv_t *d_pmv, int lambda, b2_mv_t *d_mv, uint32_t *d_cost,
                                 unsigned long long *d_swept, cudaStream_t st)
 {
-#define K1S_ARGS *tm_cur, *tm_ref, *tm_mm, mbw, mbh, nframes, d_pmv, lambda, d_mv, d_cost, d_swept, st
-#define K1S_DISPATCH(RR, KC, KF)                                                                              \
-    if (k1_prune_fine()) {                                                                                    \
-        switch (k1_threads()) {                                                                               \
-        case 192: return launch_k1_sea<RR, KF, 192>(K1S_ARGS);                                                \
-        case 320: return launch_k1_sea<RR, KF, 320>(K1S_ARGS);                                                \
-        case 384: return launch_k1_sea<RR, KF, 384>(K1S_ARGS);                                                \
-        default: return launch_k1_sea<RR, KF, 256>(K1S_ARGS);                                                 \
-        }                                                                                                     \
-    }                                                                                                         \
-    return launch_k1_sea<RR, KC, 256>(K1S_ARGS);
     switch (R) {
-    case 32: K1S_DISPATCH(32, 13, 5)
-    case 16: K1S_DISPATCH(16, 11, 3)
+    case 32: return launch_k1_sea<32>(*tm_cur, *tm_ref, *tm_mm, mbw, mbh, nframes, d_pmv, lambda, d_mv, d_cost, d_swept, st);
+    case 16: return launch_k1_sea<16>(*tm_cur, *tm_ref, *tm_mm, mbw, mbh, nframes, d_pmv, lambda, d_mv, d_cost, d_swept, st);
     default:
         fprintf(stderr, "b2enc: merange %d not supported (16 or 32)\n", R);
         return -1;

@@ -6,22 +6,26 @@
 // The filter is defined in macroblock raster order and every macroblock reads samples its left, top and
 // top-right neighbours have already modified: MB (x, y) may run once (x-1, y) and (x+1, y-1) are done.
 //
-// Schedule: ROW PIPELINE.  One warp owns one macroblock row and walks it left to right; row r trails row r-1 by two
-// macroblocks.  The only cross-warp communication is one progress counter per row: "x+1 macroblocks done", in shared
-// memory when producer and consumer row sit in the same CTA (15 of 16 rows), in global memory across CTAs.  The pixels
-// travel through L2 (fence.gpu before the flag store, fence + ld.global.cg after the flag load).  The dependency depth is
-// the same mbw + 2*mbh steps as the anti-diagonal wavefront, but a step is one warp's macroblock (no cluster-wide barrier:
-// 7 us per diagonal before) and the loads are off the chain: a warp prefetches the next macroblock's own samples and
-// decision records while it filters the current one, carries the four left columns in shared memory, and only fetches
-// the four rows above after the flag.  Plain launch (no cluster to place): a 1080p frame is five half-SM CTAs that slot
-// in beside the other stream groups' kernels; waiting warps sleep instead of spinning on the issue slots.
-// Per macroblock: the 20x20 luma and two 12x12 chroma neighbourhoods live in a per-warp shared-memory tile, lanes
+// Two schedules; b2_launch_deblock picks one by the number of frames a launch covers.
+//
+// ROW PIPELINE (fewer than 4 frames).  One warp owns one macroblock row and walks it left to right; row r trails row r-1 by two
+// macroblocks.  The CTAs of a frame (8 warps each; up to 16 CTAs for 4K's 135 rows) form a thread-block cluster.  A row hands
+// the bottom samples of every macroblock and a progress counter ("x+1 macroblocks done") to the row below through shared
+// memory -- distributed shared memory (st.shared::cluster + fence.acq_rel.cluster) when the row below sits in the next CTA --
+// and the row below reports back what it has read.  The dependency depth is the same mbw + 2*mbh steps as the wavefront, but
+// a step is one warp's macroblock (no cluster-wide barrier: 7 us per diagonal in the wavefront) and the loads are off the
+// chain: a warp prefetches the next macroblock's own samples and decision records while it filters the current one, carries
+// the four left columns in shared memory, and only fetches the four rows above after the counter.
+//
+// ANTI-DIAGONAL WAVEFRONT (4 frames and more).  Macroblocks of one diagonal mbx + 2*mby are independent; a cluster of up to
+// 8 CTAs x 16 warps per frame takes them, with a cluster barrier between diagonals.  Its chain is longer, its footprint
+// smaller: when many frames' chains overlap the other stream groups' kernels, it is the faster one.
+//
+// Per macroblock (both forms): the 20x20 luma and two 12x12 chroma neighbourhoods live in a per-warp shared-memory tile, lanes
 // 0-15 filter the luma lines (rows for vertical edges, columns for horizontal edges), lanes 16-31 the U and V lines;
 // the four edges of a line are filtered by the same lane in order.
-// (The anti-diagonal cluster-barrier form is kept behind B2_K8_WAVEFRONT=1 for A/B measurements.)
 // Bound: latency of the dependency chain; algorithmic bytes 1.5*W*H read + written.
 #include <stddef.h>
-#include <stdlib.h>
 #include "b2_mbcode.cuh"
 
 namespace {
@@ -326,26 +330,28 @@ __device__ __forceinline__ void fence_cluster() { asm volatile("fence.acq_rel.cl
 // row's g-th macroblock (counted over all rows the warp has walked): y[r * 4 + w] = luma row 12 + r, word w;
 // c[p * 4 + r * 2 + w] = chroma plane p, row 6 + r, word w
 constexpr int K8_RING = 8;
+// warps (macroblock rows) per CTA of the row pipeline: the register-resident lines need ~120 registers; 16 warps per CTA squeeze them
+// into 64 and spill
+constexpr int K8_ROW_WARPS = 8;
 struct K8Ring { uint32_t y[K8_RING][16]; uint32_t c[K8_RING][8]; };      // c directly behind y: word index K8_RING * 16 + ...
 static_assert(offsetof(K8Ring, c) == K8_RING * 16 * 4, "K8Ring layout");
 
-template <int WARPS>
-__global__ void __launch_bounds__(WARPS * 32, 2)
+__global__ void __launch_bounds__(K8_ROW_WARPS * 32, 2)
 k8_deblock_rows_kernel(uint8_t *ry, uint8_t *ru, uint8_t *rv, int pitch, int pitchc, size_t stride_y, size_t stride_c, int mbw, int mbh,
                        int qp, int alpha_off, int beta_off, const b2_mbinfo_t *__restrict__ info)
 {
-    __shared__ K8Warp s_warp[WARPS];
+    __shared__ K8Warp s_warp[K8_ROW_WARPS];
     // s_ring[w] / s_done[w]: bottom rows and progress of the producer OF warp w, i.e. of the row above warp w's row.  Warp w - 1
     // of this CTA writes them for w > 0; the last warp of the previous CTA of the cluster writes s_ring[0] / s_done[0] through
     // distributed shared memory.  s_back[w]: progress of the consumer of warp w (next warp, or warp 0 of the next CTA), for the
     // ring's back-pressure.  Every warp only ever POLLS its own CTA's shared memory.
-    __shared__ K8Ring s_ring[WARPS];
-    __shared__ int s_done[WARPS];
-    __shared__ int s_back[WARPS];
+    __shared__ K8Ring s_ring[K8_ROW_WARPS];
+    __shared__ int s_done[K8_ROW_WARPS];
+    __shared__ int s_back[K8_ROW_WARPS];
     const int frame = blockIdx.y;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int ncta = (int)cluster_nctarank(), crank = (int)cluster_ctarank();
-    const int gwarp = crank * WARPS + warp, nwarps = ncta * WARPS;
+    const int gwarp = crank * K8_ROW_WARPS + warp, nwarps = ncta * K8_ROW_WARPS;
     const b2_mbinfo_t *finfo = info + (size_t)frame * mbw * mbh;
     uint8_t *const py = ry + frame * stride_y, *const pu = ru + frame * stride_c, *const pv = rv + frame * stride_c;
     // per-lane filter constants: lanes 0-15 carry luma lines, 16-31 chroma lines.  8.7.2.2: indexA = qPav + 2 * slice_alpha_c0_offset_div2,
@@ -356,7 +362,7 @@ k8_deblock_rows_kernel(uint8_t *ry, uint8_t *ru, uint8_t *rv, int pitch, int pit
     const int l_alpha = c_alpha[l_ia], l_beta = c_beta[l_ib];
     const int l_tc = c_tc0[l_ia][0] | c_tc0[l_ia][1] << 8 | c_tc0[l_ia][2] << 16;
     const int cl = lane - 16, c_pl = (cl >> 3) & 1, c_i = cl & 7;             // chroma lanes: plane, row (vertical pass) / column (horizontal)
-    if (threadIdx.x < WARPS) { s_done[threadIdx.x] = 0; s_back[threadIdx.x] = 0; }
+    if (threadIdx.x < K8_ROW_WARPS) { s_done[threadIdx.x] = 0; s_back[threadIdx.x] = 0; }
     if (ncta > 1) cluster_barrier();      // nobody stores into a neighbour's counters before they are cleared
     else __syncthreads();
 
@@ -365,10 +371,10 @@ k8_deblock_rows_kernel(uint8_t *ry, uint8_t *ru, uint8_t *rv, int pitch, int pit
     // bottom rows go into THAT warp's ring (s_ring[consumer warp] of the consumer's CTA) with st.shared::cluster, then the
     // progress counter; the consumer reports back into s_back[] of this CTA the same way.  No global round trip and no
     // GPU-scope fence anywhere on the chain.
-    const bool cons_remote = warp == WARPS - 1, prod_remote = warp == 0;
+    const bool cons_remote = warp == K8_ROW_WARPS - 1, prod_remote = warp == 0;
     const unsigned cons_cta = cons_remote ? (unsigned)((crank + 1) % ncta) : (unsigned)crank;
     const unsigned prod_cta = prod_remote ? (unsigned)((crank + ncta - 1) % ncta) : (unsigned)crank;
-    const int cons_w = cons_remote ? 0 : warp + 1, prod_w = prod_remote ? WARPS - 1 : warp - 1;
+    const int cons_w = cons_remote ? 0 : warp + 1, prod_w = prod_remote ? K8_ROW_WARPS - 1 : warp - 1;
     const uint32_t out_ring = dsmem_addr(&s_ring[cons_w], cons_cta);             // where this warp's bottom rows go
     const uint32_t out_done = dsmem_addr(&s_done[cons_w], cons_cta);
     const uint32_t out_back = dsmem_addr(&s_back[prod_w], prod_cta);             // where this warp reports what it has consumed
@@ -564,47 +570,34 @@ int b2_launch_deblock(uint8_t *const rec[3], int pitch, int pitchc, size_t strid
     // frames wants -- the drop-in's one-GOP-per-stream shape, live streams.  A launch that covers many frames (bench.py: 8 per
     // stream group, 8 groups) is throughput-bound, its chains hide behind the other groups' K1, and there the anti-diagonal
     // wavefront's smaller footprint (40 registers, nothing spinning) is worth ~3 % of the step: 4 frames and up take it.
-    // B2_K8_WAVEFRONT=0/1 forces one form (A/B measurements).
-    static const int forced = getenv("B2_K8_WAVEFRONT") ? (atoi(getenv("B2_K8_WAVEFRONT")) != 0) : -1;
-    const bool wavefront = forced >= 0 ? forced != 0 : nframes >= 4;
-    int ncta = 1;
-    if (wavefront) {
-        const int maxdiag = mbh < (mbw + 1) / 2 ? mbh : (mbw + 1) / 2;
-        while (ncta < 8 && ncta * K8_WARPS < maxdiag) ncta *= 2;
-    }
-    if (!wavefront) {
+    (void)d_flags;
+    if (nframes < 4) {
         // One warp per macroblock row (beyond 8 CTAs of rows, warps take several); the CTAs of a frame form a cluster so that
         // the hand-off between the last row of one CTA and the first row of the next stays in (distributed) shared memory.
-        // 8 warps per CTA: the register-resident lines need ~120 registers (16 warps per CTA squeeze them into 64 with spills:
-        // B2_K8_ROW_WARPS=16, kept for measurements).
-        static const int rw = getenv("B2_K8_ROW_WARPS") && atoi(getenv("B2_K8_ROW_WARPS")) == 16 ? 16 : 8;
-        ncta = (mbh + rw - 1) / rw;
+        int ncta = (mbh + K8_ROW_WARPS - 1) / K8_ROW_WARPS;
         if (ncta > 8) {
             // tall pictures (4K: 135 rows): a cluster of up to 16 CTAs (non-portable size, supported on B200) keeps one warp per row;
             // with 8 CTAs the rows beyond the 64th would have to wait for a warp of the first rows to finish its whole row
             // (the attribute is per device; engines may live on several devices of one process, so it is set on every such launch)
-            const bool np_ok = (rw == 16 ? cudaFuncSetAttribute(k8_deblock_rows_kernel<16>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1)
-                                         : cudaFuncSetAttribute(k8_deblock_rows_kernel<8>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1)) == cudaSuccess;
+            const bool np_ok = cudaFuncSetAttribute(k8_deblock_rows_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess;
             ncta = np_ok ? (ncta > 16 ? 16 : ncta) : 8;
             cudaGetLastError();
         }
-        (void)d_flags;
         cudaLaunchConfig_t rcfg = {};
         rcfg.gridDim = dim3(ncta, nframes, 1);
-        rcfg.blockDim = dim3(rw * 32, 1, 1);
+        rcfg.blockDim = dim3(K8_ROW_WARPS * 32, 1, 1);
         rcfg.stream = st;
         cudaLaunchAttribute rattr[1];
         rattr[0].id = cudaLaunchAttributeClusterDimension;
         rattr[0].val.clusterDim.x = ncta; rattr[0].val.clusterDim.y = 1; rattr[0].val.clusterDim.z = 1;
         rcfg.attrs = rattr; rcfg.numAttrs = 1;
-        if (rw == 16)
-            B2_CUDA_OK(cudaLaunchKernelEx(&rcfg, k8_deblock_rows_kernel<16>, rec[0], rec[1], rec[2], pitch, pitchc, stride_y, stride_c, mbw, mbh, qp,
-                                          alpha_off, beta_off, d_info));
-        else
-            B2_CUDA_OK(cudaLaunchKernelEx(&rcfg, k8_deblock_rows_kernel<8>, rec[0], rec[1], rec[2], pitch, pitchc, stride_y, stride_c, mbw, mbh, qp,
-                                          alpha_off, beta_off, d_info));
+        B2_CUDA_OK(cudaLaunchKernelEx(&rcfg, k8_deblock_rows_kernel, rec[0], rec[1], rec[2], pitch, pitchc, stride_y, stride_c, mbw, mbh, qp,
+                                      alpha_off, beta_off, d_info));
         return 0;
     }
+    int ncta = 1;
+    const int maxdiag = mbh < (mbw + 1) / 2 ? mbh : (mbw + 1) / 2;
+    while (ncta < 8 && ncta * K8_WARPS < maxdiag) ncta *= 2;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(ncta, nframes, 1);
     cfg.blockDim = dim3(K8_WARPS * 32, 1, 1);
