@@ -45,6 +45,14 @@ int b2k_me_fullpel_pruned(const uint8_t *cur_y, const uint8_t *ref_y, int w, int
  * position (Y,X) = min | max << 16 over rows Y..Y+ks-1 of S[.][X], S[Y][X] = sum of padded[Y..Y+15][X..X+15]; 0 | 0xffff where a
  * block leaves the allocation.  ks in {1, 3, 5} */
 int b2k_block_sums(const uint8_t *y, int w, int h, int nframes, int ks, uint32_t *out, int *pitch_out, int *rows_out);
+/* K8 (in-loop deblocking, H.264 8.7) alone on planes in the engine's padded layout: pitch = w + 2*B2_PAD,
+ * pitchc = (w/2 + 2*B2_PADC + 15) & ~15, rows h + 2*B2_PAD / h/2 + 2*B2_PADC, nframes frames one after the other per plane;
+ * w and h multiples of 16; info [nframes][mbh*mbw]; qp 0..51, offsets (slice_alpha_c0_offset_div2 / slice_beta_offset_div2)
+ * -6..6.  All frames go through one launch and the planes are filtered in place; y == NULL only reports the shape.
+ * Out (each may be NULL): wavefront 0 (row pipeline) / 1 (anti-diagonal wavefront), ncta = CTAs per frame actually launched,
+ * rounds = rows / macroblocks of a diagonal per warp. */
+int b2k_deblock(uint8_t *y, uint8_t *u, uint8_t *v, int w, int h, int nframes, int qp, int alpha_off, int beta_off,
+                const b2_mbinfo_t *info, int *wavefront, int *ncta, int *rounds);
 /* rows per lane-task of the pruned search for +-merange: 5 (+-32) or 3 (+-16) */
 int b2_k1_prune_rows(int merange);
 

@@ -131,6 +131,25 @@ def me_fullpel_parts(cur: OFrame, ref: OFrame, R, pmv=None, lam=0):
 
 
 # ---- frame-level oracle encoder + host entropy coder (linked into libb2oracle.so) ---------------
+def deblock_frame(y, u, v, info, qp, alpha_off=0, beta_off=0):
+    """b2o_deblock_frame in place on one frame's padded planes: y [h16 + 2*PAD, w16 + 2*PAD], u/v [h16/2 + 2*PADC, pitchc]
+    C-contiguous uint8 arrays (any chroma pitch); info MBINFO [mbs] in raster order"""
+    for p in (y, u, v):
+        assert p.dtype == np.uint8 and p.flags.c_contiguous and p.flags.writeable
+    assert u.shape == v.shape
+    f = Frame()
+    f.w16 = f.w = y.shape[1] - 2 * PAD
+    f.h16 = f.h = y.shape[0] - 2 * PAD
+    f.mbw, f.mbh = f.w16 // 16, f.h16 // 16
+    f.pitch, f.pitchc = y.strides[0], u.strides[0]
+    f.y = y.ctypes.data + PAD * f.pitch + PAD
+    f.u = u.ctypes.data + PADC * f.pitchc + PADC
+    f.v = v.ctypes.data + PADC * f.pitchc + PADC
+    info = np.ascontiguousarray(info, MBINFO)
+    assert info.size == f.mbw * f.mbh
+    lib().b2o_deblock_frame(C.byref(f), _p(info), qp, alpha_off, beta_off)
+
+
 class Seq(C.Structure):
     _fields_ = [("width", C.c_int), ("height", C.c_int), ("fps_num", C.c_int), ("fps_den", C.c_int),
                 ("sar_w", C.c_int), ("sar_h", C.c_int), ("qp", C.c_int), ("deblock", C.c_int),

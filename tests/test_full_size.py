@@ -9,11 +9,14 @@ pytestmark = pytest.mark.gpu
 
 
 def _encode_and_check(oracle, b2, w, h, R, qp, nslots, nframes, oracle_slots, subpel=1, intra_in_p=1, deblock=0, cabac=0, t8=0,
-                      partitions=0, pack=0, frame_fn=None):
+                      partitions=0, pack=0, frame_fn=None, deblock_offsets=(0, 0), streams=0, expect_groups=None):
+    """expect_groups: the engine's stream groups as (first slot, slots) -- the frames of a group share every launch"""
     eng = b2.Engine(w, h, slots=nslots, ring=1, merange=R, qp=qp, subpel=subpel, intra_in_p=intra_in_p, deblock=deblock,
-                    transform8x8=t8, partitions=partitions, pack_levels=pack)
-    prm = oracle.Params(qp, R, subpel, intra_in_p, deblock, t8, partitions)
-    ents = [oracle.Entropy(w, h, qp, deblock=deblock, cabac=cabac, transform8x8=t8) for _ in range(nslots)]
+                    transform8x8=t8, partitions=partitions, pack_levels=pack, deblock_offsets=deblock_offsets, streams=streams)
+    if expect_groups is not None:
+        assert eng.groups() == expect_groups
+    prm = oracle.Params(qp, R, subpel, intra_in_p, deblock, t8, partitions, *deblock_offsets)
+    ents = [oracle.Entropy(w, h, qp, deblock=deblock, cabac=cabac, transform8x8=t8, deblock_offsets=deblock_offsets) for _ in range(nslots)]
     frame_fn = frame_fn or (lambda t, s: oracle.synth_frame(w, h, t, s))
     streams = [bytearray() for _ in range(nslots)]
     recons = [[] for _ in range(nslots)]

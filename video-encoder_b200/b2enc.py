@@ -110,6 +110,45 @@ def block_sums(y, ks=1):
     return (out & 0xffff).astype(np.uint16), (out >> 16).astype(np.uint16)
 
 
+PAD, PADC = 64, 32                     # B2_PAD / B2_PADC (include/b2enc_types.h)
+
+
+def padded_layout(w, h):
+    """(pitch, rows, pitchc, rowsc) of the device planes of a coded size w x h (b2_padded_layout, csrc/b2_internal.h)"""
+    return w + 2 * PAD, h + 2 * PAD, (w // 2 + 2 * PADC + 15) & ~15, h // 2 + 2 * PADC
+
+
+def _deblock_lib():
+    L = lib()
+    L.b2k_deblock.argtypes = [C.c_void_p] * 3 + [C.c_int] * 6 + [C.c_void_p] * 4
+    return L
+
+
+def deblock_shape(w, h, nframes):
+    """K8's launch shape for nframes frames of coded size w x h: (wavefront 0/1, CTAs per frame, rounds per warp)"""
+    out = [C.c_int(0) for _ in range(3)]
+    if _deblock_lib().b2k_deblock(None, None, None, w, h, nframes, 26, 0, 0, None, *[C.addressof(o) for o in out]) != 0:
+        raise RuntimeError("b2k_deblock failed")
+    return tuple(o.value for o in out)
+
+
+def deblock(y, u, v, info, qp, alpha_off=0, beta_off=0):
+    """K8 alone (b2k_deblock): y [n, h + 2*PAD, w + 2*PAD], u/v [n, h/2 + 2*PADC, pitchc] uint8 planes in the engine's padded
+    layout (see padded_layout), info MBINFO [n, mbs].  Returns (filtered copies of y, u, v, (wavefront, ncta, rounds))."""
+    require_gpu()
+    y, u, v = (np.array(p, np.uint8, order="C", copy=True) for p in (y, u, v))
+    n = y.shape[0]
+    w, h = y.shape[2] - 2 * PAD, y.shape[1] - 2 * PAD
+    pitch, rows, pitchc, rowsc = padded_layout(w, h)
+    if y.shape != (n, rows, pitch) or u.shape != (n, rowsc, pitchc) or v.shape != u.shape:
+        raise ValueError("planes are not in the padded layout of %dx%d" % (w, h))
+    info = np.ascontiguousarray(info, MBINFO).reshape(n, (w // 16) * (h // 16))
+    out = [C.c_int(0) for _ in range(3)]
+    if _deblock_lib().b2k_deblock(_p(y), _p(u), _p(v), w, h, n, qp, alpha_off, beta_off, _p(info), *[C.addressof(o) for o in out]) != 0:
+        raise RuntimeError("b2k_deblock failed")
+    return y, u, v, tuple(o.value for o in out)
+
+
 def k1_prune_rows(merange):
     return lib().b2_k1_prune_rows(merange)
 

@@ -286,8 +286,7 @@ extern "C" b2_engine_t *b2_engine_create(const b2_engine_cfg_t *cfg)
     e->cfg = *cfg;
     e->w16 = (cfg->width + 15) & ~15; e->h16 = (cfg->height + 15) & ~15;
     e->mbw = e->w16 / 16; e->mbh = e->h16 / 16; e->nmb = e->mbw * e->mbh;
-    e->pitch = e->w16 + 2 * B2_PAD; e->rows = e->h16 + 2 * B2_PAD;
-    e->pitchc = (e->w16 / 2 + 2 * B2_PADC + 15) & ~15; e->rowsc = e->h16 / 2 + 2 * B2_PADC;
+    b2_padded_layout(e->w16, e->h16, &e->pitch, &e->rows, &e->pitchc, &e->rowsc);
     e->stride_y = (size_t)e->pitch * e->rows; e->stride_c = (size_t)e->pitchc * e->rowsc;
     e->in_bytes = input_bytes(cfg->in_fmt, cfg->width, cfg->height);
     if (!e->in_bytes) { fprintf(stderr, "b2enc: unsupported input format %d\n", cfg->in_fmt); delete e; return nullptr; }

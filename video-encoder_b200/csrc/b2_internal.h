@@ -5,6 +5,13 @@
 #include <stdint.h>
 #include "../../include/b2enc_types.h"
 
+// padded layout of the device planes of a coded size w16 x h16: luma pitch / rows, chroma pitch (a multiple of 16) / rows
+inline void b2_padded_layout(int w16, int h16, int *pitch, int *rows, int *pitchc, int *rowsc)
+{
+    *pitch = w16 + 2 * B2_PAD; *rows = h16 + 2 * B2_PAD;
+    *pitchc = (w16 / 2 + 2 * B2_PADC + 15) & ~15; *rowsc = h16 / 2 + 2 * B2_PADC;
+}
+
 int b2_make_plane_tmap(CUtensorMap *tm, const void *base, int pitch, int rows, int nplanes, int bw, int bh);
 int b2_launch_extend_border(uint8_t *d_planes, int pitch, int rows, int nplanes, int pad, int iw, int ih,
                             cudaStream_t st);
@@ -49,6 +56,10 @@ int b2_launch_intra_recon(const uint8_t *const cur[3], uint8_t *const rec[3], in
                           size_t stride_c, int mbw, int mbh, int nframes, int qp, int all_intra, b2_mbinfo_t *d_info,
                           b2_mbcoef_t *d_coef, cudaStream_t st);
 int b2_lambda_for_qp(int qp);
+// K8's launch shape for `nframes` frames of mbw x mbh macroblocks: wavefront 0 = row pipeline, 1 = anti-diagonal wavefront;
+// ncta = CTAs per frame (one cluster); rounds = rows (row pipeline) / macroblocks of one diagonal (wavefront) per warp.  Above
+// 8 CTAs of rows it allows the non-portable cluster size on the current device; where that is refused it reports 8 CTAs.
+void b2_deblock_shape(int mbw, int mbh, int nframes, int *wavefront, int *ncta, int *rounds);
 int b2_launch_deblock(uint8_t *const rec[3], int pitch, int pitchc, size_t stride_y, size_t stride_c, int mbw, int mbh,
                       int nframes, int qp, int alpha_off, int beta_off, const b2_mbinfo_t *d_info,
                       int *d_flags /* [nframes][8] cross-CTA progress flags (scratch) */, cudaStream_t st);

@@ -82,6 +82,45 @@ extern "C" int b2k_block_sums(const uint8_t *y, int w, int h, int nframes, int k
     return 0;
 }
 
+// K8 alone: the planes go to the device as they are (padding included), are filtered in one launch and come back whole, so
+// that a caller can see any store outside the picture
+extern "C" int b2k_deblock(uint8_t *y, uint8_t *u, uint8_t *v, int w, int h, int nframes, int qp, int alpha_off, int beta_off,
+                           const b2_mbinfo_t *info, int *wavefront, int *ncta, int *rounds)
+{
+    if ((w & 15) || (h & 15) || w <= 0 || h <= 0 || nframes <= 0 || qp < 0 || qp > 51 || alpha_off < -6 || alpha_off > 6 ||
+        beta_off < -6 || beta_off > 6) {
+        fprintf(stderr, "b2enc: b2k_deblock needs w,h multiples of 16, qp 0..51, offsets -6..6\n");
+        return -1;
+    }
+    const int mbw = w / 16, mbh = h / 16;
+    int wf, nc, rd;
+    b2_deblock_shape(mbw, mbh, nframes, &wf, &nc, &rd);
+    if (wavefront) *wavefront = wf;
+    if (ncta) *ncta = nc;
+    if (rounds) *rounds = rd;
+    if (!y) return 0;
+    if (!u || !v || !info) return -1;
+    int pitch, rows, pitchc, rowsc;
+    b2_padded_layout(w, h, &pitch, &rows, &pitchc, &rowsc);
+    const size_t ny = (size_t)pitch * rows * nframes, nc_bytes = (size_t)pitchc * rowsc * nframes;
+    const size_t ni = (size_t)mbw * mbh * nframes * sizeof(b2_mbinfo_t);
+    DevBuf d_y, d_u, d_v, d_info;
+    if (d_y.alloc(ny) || d_u.alloc(nc_bytes) || d_v.alloc(nc_bytes) || d_info.alloc(ni)) { fprintf(stderr, "b2enc: cudaMalloc failed\n"); return -1; }
+    B2_CUDA_OK(cudaMemcpy(d_y.p, y, ny, cudaMemcpyHostToDevice));
+    B2_CUDA_OK(cudaMemcpy(d_u.p, u, nc_bytes, cudaMemcpyHostToDevice));
+    B2_CUDA_OK(cudaMemcpy(d_v.p, v, nc_bytes, cudaMemcpyHostToDevice));
+    B2_CUDA_OK(cudaMemcpy(d_info.p, info, ni, cudaMemcpyHostToDevice));
+    uint8_t *const rec[3] = {(uint8_t *)d_y.p, (uint8_t *)d_u.p, (uint8_t *)d_v.p};
+    if (b2_launch_deblock(rec, pitch, pitchc, (size_t)pitch * rows, (size_t)pitchc * rowsc, mbw, mbh, nframes, qp, alpha_off, beta_off,
+                          (const b2_mbinfo_t *)d_info.p, nullptr, 0))
+        return -1;
+    B2_CUDA_OK(cudaDeviceSynchronize());
+    B2_CUDA_OK(cudaMemcpy(y, d_y.p, ny, cudaMemcpyDeviceToHost));
+    B2_CUDA_OK(cudaMemcpy(u, d_u.p, nc_bytes, cudaMemcpyDeviceToHost));
+    B2_CUDA_OK(cudaMemcpy(v, d_v.p, nc_bytes, cudaMemcpyDeviceToHost));
+    return 0;
+}
+
 extern "C" int b2k_me_fullpel(const uint8_t *cur_y, const uint8_t *ref_y, int w, int h, int nframes, int merange,
                               const b2_mv_t *pmv, int lambda, b2_mv_t *mv_out, uint32_t *cost_out,
                               int iters, float *kernel_ms)

@@ -40,8 +40,7 @@ extern "C" void *b2_sws_rt_create(int w, int h, int fmt)
     c->device = 0;
     cudaGetDevice(&c->device);                          // the device current at creation owns the buffers and runs K0
     c->w16 = (w + 15) & ~15; c->h16 = (h + 15) & ~15;
-    c->pitch = c->w16 + 2 * B2_PAD; c->rows = c->h16 + 2 * B2_PAD;
-    c->pitchc = (c->w16 / 2 + 2 * B2_PADC + 15) & ~15; c->rowsc = c->h16 / 2 + 2 * B2_PADC;
+    b2_padded_layout(c->w16, c->h16, &c->pitch, &c->rows, &c->pitchc, &c->rowsc);
     c->in_bytes = 0;
     for (int p = 0; p < 3; p++) c->in_bytes += (size_t)rb[p] * rws[p];
     return c;                                           // buffers are allocated on first use

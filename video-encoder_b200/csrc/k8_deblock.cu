@@ -563,51 +563,55 @@ k8_deblock_rows_kernel(uint8_t *ry, uint8_t *ru, uint8_t *rv, int pitch, int pit
 
 }  // namespace
 
-int b2_launch_deblock(uint8_t *const rec[3], int pitch, int pitchc, size_t stride_y, size_t stride_c, int mbw, int mbh,
-                      int nframes, int qp, int alpha_off, int beta_off, const b2_mbinfo_t *d_info, int *d_flags, cudaStream_t st)
+void b2_deblock_shape(int mbw, int mbh, int nframes, int *wavefront, int *ncta, int *rounds)
 {
     // Two schedules.  The row pipeline has the shorter chain (0.87 vs 1.59 ms for one 1080p frame) and is what a launch of few
     // frames wants -- the drop-in's one-GOP-per-stream shape, live streams.  A launch that covers many frames (bench.py: 8 per
     // stream group, 8 groups) is throughput-bound, its chains hide behind the other groups' K1, and there the anti-diagonal
     // wavefront's smaller footprint (40 registers, nothing spinning) is worth ~3 % of the step: 4 frames and up take it.
-    (void)d_flags;
     if (nframes < 4) {
         // One warp per macroblock row (beyond 8 CTAs of rows, warps take several); the CTAs of a frame form a cluster so that
         // the hand-off between the last row of one CTA and the first row of the next stays in (distributed) shared memory.
-        int ncta = (mbh + K8_ROW_WARPS - 1) / K8_ROW_WARPS;
-        if (ncta > 8) {
+        int n = (mbh + K8_ROW_WARPS - 1) / K8_ROW_WARPS;
+        if (n > 8) {
             // tall pictures (4K: 135 rows): a cluster of up to 16 CTAs (non-portable size, supported on B200) keeps one warp per row;
             // with 8 CTAs the rows beyond the 64th would have to wait for a warp of the first rows to finish its whole row
             // (the attribute is per device; engines may live on several devices of one process, so it is set on every such launch)
             const bool np_ok = cudaFuncSetAttribute(k8_deblock_rows_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess;
-            ncta = np_ok ? (ncta > 16 ? 16 : ncta) : 8;
+            n = np_ok ? (n > 16 ? 16 : n) : 8;
             cudaGetLastError();
         }
-        cudaLaunchConfig_t rcfg = {};
-        rcfg.gridDim = dim3(ncta, nframes, 1);
-        rcfg.blockDim = dim3(K8_ROW_WARPS * 32, 1, 1);
-        rcfg.stream = st;
-        cudaLaunchAttribute rattr[1];
-        rattr[0].id = cudaLaunchAttributeClusterDimension;
-        rattr[0].val.clusterDim.x = ncta; rattr[0].val.clusterDim.y = 1; rattr[0].val.clusterDim.z = 1;
-        rcfg.attrs = rattr; rcfg.numAttrs = 1;
-        B2_CUDA_OK(cudaLaunchKernelEx(&rcfg, k8_deblock_rows_kernel, rec[0], rec[1], rec[2], pitch, pitchc, stride_y, stride_c, mbw, mbh, qp,
-                                      alpha_off, beta_off, d_info));
-        return 0;
+        *wavefront = 0; *ncta = n;
+        *rounds = (mbh + n * K8_ROW_WARPS - 1) / (n * K8_ROW_WARPS);
+        return;
     }
-    int ncta = 1;
+    int n = 1;
     const int maxdiag = mbh < (mbw + 1) / 2 ? mbh : (mbw + 1) / 2;
-    while (ncta < 8 && ncta * K8_WARPS < maxdiag) ncta *= 2;
+    while (n < 8 && n * K8_WARPS < maxdiag) n *= 2;
+    *wavefront = 1; *ncta = n;
+    *rounds = (maxdiag + n * K8_WARPS - 1) / (n * K8_WARPS);
+}
+
+int b2_launch_deblock(uint8_t *const rec[3], int pitch, int pitchc, size_t stride_y, size_t stride_c, int mbw, int mbh,
+                      int nframes, int qp, int alpha_off, int beta_off, const b2_mbinfo_t *d_info, int *d_flags, cudaStream_t st)
+{
+    (void)d_flags;
+    int wavefront, ncta, rounds;
+    b2_deblock_shape(mbw, mbh, nframes, &wavefront, &ncta, &rounds);
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(ncta, nframes, 1);
-    cfg.blockDim = dim3(K8_WARPS * 32, 1, 1);
+    cfg.blockDim = dim3((wavefront ? K8_WARPS : K8_ROW_WARPS) * 32, 1, 1);
     cfg.dynamicSmemBytes = 0;
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
     attr[0].val.clusterDim.x = ncta; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
-    B2_CUDA_OK(cudaLaunchKernelEx(&cfg, k8_deblock_kernel, rec[0], rec[1], rec[2], pitch, pitchc, stride_y, stride_c, mbw, mbh, qp,
-                                  alpha_off, beta_off, d_info));
+    if (wavefront)
+        B2_CUDA_OK(cudaLaunchKernelEx(&cfg, k8_deblock_kernel, rec[0], rec[1], rec[2], pitch, pitchc, stride_y, stride_c, mbw, mbh, qp,
+                                      alpha_off, beta_off, d_info));
+    else
+        B2_CUDA_OK(cudaLaunchKernelEx(&cfg, k8_deblock_rows_kernel, rec[0], rec[1], rec[2], pitch, pitchc, stride_y, stride_c, mbw, mbh, qp,
+                                      alpha_off, beta_off, d_info));
     return 0;
 }
