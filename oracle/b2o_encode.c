@@ -120,6 +120,18 @@ void b2o_recon_intra_mb(const b2o_params_t *prm, const b2o_frame_t *cur, b2o_fra
     finish_cbp(mi, mask);
 }
 
+void b2o_recon_intra_frame(int qp, const b2o_frame_t *cur, b2o_frame_t *recon, b2_mbinfo_t *info, b2_mbcoef_t *coef)
+{
+    b2o_params_t prm;
+    memset(&prm, 0, sizeof(prm));
+    prm.qp = qp;
+    for (int mby = 0; mby < cur->mbh; mby++)
+        for (int mbx = 0; mbx < cur->mbw; mbx++) {
+            int i = mby * cur->mbw + mbx;
+            if (info[i].mb_type != B2_MB_P16x16) b2o_recon_intra_mb(&prm, cur, recon, mbx, mby, &info[i], &coef[i]);
+        }
+}
+
 void b2o_encode_frame(const b2o_params_t *prm, int frame_type,
                       const b2o_frame_t *cur, const b2o_frame_t *ref, b2o_frame_t *recon,
                       const b2_mv_t *prev_mv, b2_mbinfo_t *info, b2_mbcoef_t *coef)

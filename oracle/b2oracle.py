@@ -134,8 +134,17 @@ def me_fullpel_parts(cur: OFrame, ref: OFrame, R, pmv=None, lam=0):
 def deblock_frame(y, u, v, info, qp, alpha_off=0, beta_off=0):
     """b2o_deblock_frame in place on one frame's padded planes: y [h16 + 2*PAD, w16 + 2*PAD], u/v [h16/2 + 2*PADC, pitchc]
     C-contiguous uint8 arrays (any chroma pitch); info MBINFO [mbs] in raster order"""
+    assert all(p.flags.writeable for p in (y, u, v))
+    f = _padded_frame(y, u, v)
+    info = np.ascontiguousarray(info, MBINFO)
+    assert info.size == f.mbw * f.mbh
+    lib().b2o_deblock_frame(C.byref(f), _p(info), qp, alpha_off, beta_off)
+
+
+def _padded_frame(y, u, v):
+    """b2o_frame_t over one frame's padded planes (y [h16 + 2*PAD, w16 + 2*PAD], u/v [h16/2 + 2*PADC, pitchc])"""
     for p in (y, u, v):
-        assert p.dtype == np.uint8 and p.flags.c_contiguous and p.flags.writeable
+        assert p.dtype == np.uint8 and p.flags.c_contiguous
     assert u.shape == v.shape
     f = Frame()
     f.w16 = f.w = y.shape[1] - 2 * PAD
@@ -145,9 +154,17 @@ def deblock_frame(y, u, v, info, qp, alpha_off=0, beta_off=0):
     f.y = y.ctypes.data + PAD * f.pitch + PAD
     f.u = u.ctypes.data + PADC * f.pitchc + PADC
     f.v = v.ctypes.data + PADC * f.pitchc + PADC
-    info = np.ascontiguousarray(info, MBINFO)
-    assert info.size == f.mbw * f.mbh
-    lib().b2o_deblock_frame(C.byref(f), _p(info), qp, alpha_off, beta_off)
+    return f
+
+
+def recon_intra_frame(cur, rec, info, coef, qp):
+    """b2o_recon_intra_frame on one frame: cur / rec = (y, u, v) padded planes as for deblock_frame; rec, info (MBINFO [mbs])
+    and coef (MBCOEF [mbs]) are updated in place -- intra macroblocks only, in raster order"""
+    fc, fr = _padded_frame(*cur), _padded_frame(*rec)
+    assert all(p.flags.writeable for p in rec) and (fc.w16, fc.h16, fc.pitchc) == (fr.w16, fr.h16, fr.pitchc)
+    for a, dt in ((info, MBINFO), (coef, MBCOEF)):
+        assert a.dtype == dt and a.flags.c_contiguous and a.flags.writeable and a.size == fc.mbw * fc.mbh
+    lib().b2o_recon_intra_frame(qp, C.byref(fc), C.byref(fr), _p(info), _p(coef))
 
 
 class Seq(C.Structure):

@@ -9,8 +9,9 @@ pytestmark = pytest.mark.gpu
 
 
 def _encode_and_check(oracle, b2, w, h, R, qp, nslots, nframes, oracle_slots, subpel=1, intra_in_p=1, deblock=0, cabac=0, t8=0,
-                      partitions=0, pack=0, frame_fn=None, deblock_offsets=(0, 0), streams=0, expect_groups=None):
-    """expect_groups: the engine's stream groups as (first slot, slots) -- the frames of a group share every launch"""
+                      partitions=0, pack=0, frame_fn=None, deblock_offsets=(0, 0), streams=0, expect_groups=None, infos=None):
+    """expect_groups: the engine's stream groups as (first slot, slots) -- the frames of a group share every launch;
+    infos: a list that receives (t, slot, the engine's info) of every frame"""
     eng = b2.Engine(w, h, slots=nslots, ring=1, merange=R, qp=qp, subpel=subpel, intra_in_p=intra_in_p, deblock=deblock,
                     transform8x8=t8, partitions=partitions, pack_levels=pack, deblock_offsets=deblock_offsets, streams=streams)
     if expect_groups is not None:
@@ -30,6 +31,8 @@ def _encode_and_check(oracle, b2, w, h, R, qp, nslots, nframes, oracle_slots, su
         eng.h2d(); eng.encode(ft); eng.d2h(); eng.sync()
         for s in range(nslots):
             info, coef = eng.results(s)
+            if infos is not None:
+                infos.append((t, s, info.copy()))
             if t == 0:
                 streams[s] += sc + ents[s].sps() + sc + ents[s].pps()
             streams[s] += sc + ents[s].slice(ft, t, 0, info, coef)

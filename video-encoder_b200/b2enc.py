@@ -149,6 +149,46 @@ def deblock(y, u, v, info, qp, alpha_off=0, beta_off=0):
     return y, u, v, tuple(o.value for o in out)
 
 
+def _intra_recon_lib():
+    L = lib()
+    L.b2k_intra_recon.argtypes = [C.c_void_p] * 6 + [C.c_int] * 5 + [C.c_void_p] * 5
+    return L
+
+
+def intra_recon_shape(w, h, all_intra):
+    """K7's launch shape for frames of coded size w x h: (CTAs per frame, tasks of the longest diagonal per warp, dynamic shared
+    memory bytes per CTA)"""
+    out = [C.c_int(0) for _ in range(3)]
+    if _intra_recon_lib().b2k_intra_recon(None, None, None, None, None, None, w, h, 1, 26, int(all_intra), None, None,
+                                          *[C.addressof(o) for o in out]) != 0:
+        raise RuntimeError("b2k_intra_recon failed")
+    return tuple(o.value for o in out)
+
+
+def intra_recon(cur, rec, info, coef, qp, all_intra):
+    """K7 alone (b2k_intra_recon): cur / rec = (y, u, v) uint8 planes [n, rows, pitch] in the engine's padded layout (see
+    padded_layout), info MBINFO [n, mbs], coef MBCOEF [n, mbs].  Returns (copies of rec y, u, v, info, coef after the launch,
+    (ncta, rounds, dyn_smem))."""
+    require_gpu()
+    cy, cu, cv = (np.ascontiguousarray(p, np.uint8) for p in cur)
+    ry, ru, rv = (np.array(p, np.uint8, order="C", copy=True) for p in rec)
+    n = cy.shape[0]
+    w, h = cy.shape[2] - 2 * PAD, cy.shape[1] - 2 * PAD
+    pitch, rows, pitchc, rowsc = padded_layout(w, h)
+    for p, shape in ((cy, (n, rows, pitch)), (ry, (n, rows, pitch)), (cu, (n, rowsc, pitchc)), (cv, (n, rowsc, pitchc)),
+                     (ru, (n, rowsc, pitchc)), (rv, (n, rowsc, pitchc))):
+        if p.shape != shape:
+            raise ValueError("planes are not in the padded layout of %dx%d" % (w, h))
+    nmb = (w // 16) * (h // 16)
+    info = np.array(info, MBINFO, order="C", copy=True).reshape(n, nmb)
+    coef = np.array(coef, MBCOEF, order="C", copy=True).reshape(n, nmb)
+    out = [C.c_int(0) for _ in range(3)]
+    if _intra_recon_lib().b2k_intra_recon(_p(cy), _p(cu), _p(cv), _p(ry), _p(ru), _p(rv), w, h, n, qp, int(all_intra), _p(info), _p(coef),
+                                          *[C.addressof(o) for o in out]) != 0:
+        raise RuntimeError("b2k_intra_recon failed")
+    return ry, ru, rv, info, coef, tuple(o.value for o in out)
+
+
 def k1_prune_rows(merange):
     return lib().b2_k1_prune_rows(merange)
 

@@ -52,6 +52,10 @@ int b2_launch_decide_inter(const uint8_t *const cur[3], const uint8_t *const ref
                            int do_intra, int qp, const b2_mv_t *d_mvq, const uint32_t *d_cost_inter, const uint32_t *d_c16,
                            const uint32_t *d_c4, const uint32_t *d_c8, b2_mbinfo_t *d_info, b2_mbcoef_t *d_coef, b2_mv_t *d_prev_mv,
                            const uint8_t *d_pred_y, int transform8x8, const uint8_t *d_part, const b2_mv_t *d_mv8, cudaStream_t st);
+// K7's launch shape for frames of mbw x mbh macroblocks: ncta = CTAs per frame (one cluster; 1 unless all_intra), rounds =
+// (macroblock, luma | chroma) tasks of the longest anti-diagonal per warp, dyn_smem = dynamic shared memory of one CTA
+void b2_intra_recon_shape(int mbw, int mbh, int all_intra, int *ncta, int *rounds, int *dyn_smem);
+// refuses (-1, before any launch) a picture whose diagonal tables exceed the kernel's dynamic shared memory (ndiag > 3134)
 int b2_launch_intra_recon(const uint8_t *const cur[3], uint8_t *const rec[3], int pitch, int pitchc, size_t stride_y,
                           size_t stride_c, int mbw, int mbh, int nframes, int qp, int all_intra, b2_mbinfo_t *d_info,
                           b2_mbcoef_t *d_coef, cudaStream_t st);

@@ -121,6 +121,56 @@ extern "C" int b2k_deblock(uint8_t *y, uint8_t *u, uint8_t *v, int w, int h, int
     return 0;
 }
 
+// K7 (+ its cbp pass) alone: as b2k_deblock, the planes, records and levels go to the device as they are and come back whole, so
+// that a caller can see any store outside an intra macroblock
+extern "C" int b2k_intra_recon(const uint8_t *cur_y, const uint8_t *cur_u, const uint8_t *cur_v, uint8_t *rec_y, uint8_t *rec_u,
+                               uint8_t *rec_v, int w, int h, int nframes, int qp, int all_intra, b2_mbinfo_t *info, b2_mbcoef_t *coef,
+                               int *ncta, int *rounds, int *dyn_smem)
+{
+    if ((w & 15) || (h & 15) || w <= 0 || h <= 0 || nframes <= 0 || qp < 10 || qp > 51) {
+        fprintf(stderr, "b2enc: b2k_intra_recon needs w,h multiples of 16, qp 10..51\n");
+        return -1;
+    }
+    const int mbw = w / 16, mbh = h / 16;
+    int nc, rd, ds;
+    b2_intra_recon_shape(mbw, mbh, all_intra, &nc, &rd, &ds);
+    if (ncta) *ncta = nc;
+    if (rounds) *rounds = rd;
+    if (dyn_smem) *dyn_smem = ds;
+    if (!rec_y) return 0;
+    if (!cur_y || !cur_u || !cur_v || !rec_u || !rec_v || !info || !coef) return -1;
+    int pitch, rows, pitchc, rowsc;
+    b2_padded_layout(w, h, &pitch, &rows, &pitchc, &rowsc);
+    const size_t sy = (size_t)pitch * rows, sc = (size_t)pitchc * rowsc, ny = sy * nframes, nc_bytes = sc * nframes;
+    const size_t nmb = (size_t)mbw * mbh * nframes, ni = nmb * sizeof(b2_mbinfo_t), ncf = nmb * sizeof(b2_mbcoef_t);
+    DevBuf d_cy, d_cu, d_cv, d_ry, d_ru, d_rv, d_info, d_coef;
+    if (d_cy.alloc(ny) || d_cu.alloc(nc_bytes) || d_cv.alloc(nc_bytes) || d_ry.alloc(ny) || d_ru.alloc(nc_bytes) || d_rv.alloc(nc_bytes) ||
+        d_info.alloc(ni) || d_coef.alloc(ncf)) {
+        fprintf(stderr, "b2enc: cudaMalloc failed\n");
+        return -1;
+    }
+    B2_CUDA_OK(cudaMemcpy(d_cy.p, cur_y, ny, cudaMemcpyHostToDevice));
+    B2_CUDA_OK(cudaMemcpy(d_cu.p, cur_u, nc_bytes, cudaMemcpyHostToDevice));
+    B2_CUDA_OK(cudaMemcpy(d_cv.p, cur_v, nc_bytes, cudaMemcpyHostToDevice));
+    B2_CUDA_OK(cudaMemcpy(d_ry.p, rec_y, ny, cudaMemcpyHostToDevice));
+    B2_CUDA_OK(cudaMemcpy(d_ru.p, rec_u, nc_bytes, cudaMemcpyHostToDevice));
+    B2_CUDA_OK(cudaMemcpy(d_rv.p, rec_v, nc_bytes, cudaMemcpyHostToDevice));
+    B2_CUDA_OK(cudaMemcpy(d_info.p, info, ni, cudaMemcpyHostToDevice));
+    B2_CUDA_OK(cudaMemcpy(d_coef.p, coef, ncf, cudaMemcpyHostToDevice));
+    const uint8_t *const cur[3] = {(const uint8_t *)d_cy.p, (const uint8_t *)d_cu.p, (const uint8_t *)d_cv.p};
+    uint8_t *const rec[3] = {(uint8_t *)d_ry.p, (uint8_t *)d_ru.p, (uint8_t *)d_rv.p};
+    if (b2_launch_intra_recon(cur, rec, pitch, pitchc, sy, sc, mbw, mbh, nframes, qp, all_intra, (b2_mbinfo_t *)d_info.p,
+                              (b2_mbcoef_t *)d_coef.p, 0))
+        return -1;
+    B2_CUDA_OK(cudaDeviceSynchronize());
+    B2_CUDA_OK(cudaMemcpy(rec_y, d_ry.p, ny, cudaMemcpyDeviceToHost));
+    B2_CUDA_OK(cudaMemcpy(rec_u, d_ru.p, nc_bytes, cudaMemcpyDeviceToHost));
+    B2_CUDA_OK(cudaMemcpy(rec_v, d_rv.p, nc_bytes, cudaMemcpyDeviceToHost));
+    B2_CUDA_OK(cudaMemcpy(info, d_info.p, ni, cudaMemcpyDeviceToHost));
+    B2_CUDA_OK(cudaMemcpy(coef, d_coef.p, ncf, cudaMemcpyDeviceToHost));
+    return 0;
+}
+
 extern "C" int b2k_me_fullpel(const uint8_t *cur_y, const uint8_t *ref_y, int w, int h, int nframes, int merange,
                               const b2_mv_t *pmv, int lambda, b2_mv_t *mv_out, uint32_t *cost_out,
                               int iters, float *kernel_ms)

@@ -558,6 +558,21 @@ k7_cbp_kernel(b2_mbinfo_t *__restrict__ info, int n)
 
 }  // namespace
 
+void b2_intra_recon_shape(int mbw, int mbh, int all_intra, int *ncta, int *rounds, int *dyn_smem)
+{
+    const int ndiag = mbw + 2 * (mbh - 1);
+    const int maxdiag = mbh < (mbw + 1) / 2 ? mbh : (mbw + 1) / 2;      // macroblocks on the longest anti-diagonal
+    // I frames: every MB of a diagonal gets its own luma + chroma warp (cluster of up to 8 CTAs).  P frames hold few,
+    // scattered intra MBs: one CTA per frame keeps the footprint at one SM so that other streams' kernels keep the rest.
+    const int warps = all_intra ? K7_WARPS_I : K7_WARPS_P;
+    int n = 1;
+    if (all_intra)
+        while (n < 8 && n * warps < 2 * maxdiag) n *= 2;
+    *ncta = n;
+    *rounds = (2 * maxdiag + n * warps - 1) / (n * warps);           // (MB, luma | chroma) tasks of the longest diagonal per warp
+    *dyn_smem = 2 * ndiag * (int)sizeof(int);                        // per diagonal: holds intra MBs | list entry
+}
+
 int b2_launch_intra_recon(const uint8_t *const cur[3], uint8_t *const rec[3], int pitch, int pitchc, size_t stride_y,
                           size_t stride_c, int mbw, int mbh, int nframes, int qp, int all_intra, b2_mbinfo_t *d_info,
                           b2_mbcoef_t *d_coef, cudaStream_t st)
@@ -565,17 +580,26 @@ int b2_launch_intra_recon(const uint8_t *const cur[3], uint8_t *const rec[3], in
     FramePlanes fp;
     for (int i = 0; i < 3; i++) { fp.cur[i] = cur[i]; fp.ref[i] = nullptr; fp.rec[i] = rec[i]; }
     fp.pitch = pitch; fp.pitchc = pitchc; fp.stride_y = stride_y; fp.stride_c = stride_c;
-    const int ndiag = mbw + 2 * (mbh - 1);
-    const int maxdiag = mbh < (mbw + 1) / 2 ? mbh : (mbw + 1) / 2;      // macroblocks on the longest anti-diagonal
-    // I frames: every MB of a diagonal gets its own luma + chroma warp (cluster of up to 8 CTAs).  P frames hold few,
-    // scattered intra MBs: one CTA per frame keeps the footprint at one SM so that other streams' kernels keep the rest.
-    int ncta = 1;
-    if (all_intra)
-        while (ncta < 8 && ncta * K7_WARPS_I < 2 * maxdiag) ncta *= 2;
+    int ncta, rounds, dyn_smem;
+    b2_intra_recon_shape(mbw, mbh, all_intra, &ncta, &rounds, &dyn_smem);
+    // The diagonal tables grow with mbw + 2*mbh and sit beside the per-warp tiles; the kernel does not opt in to more than the
+    // default dynamic shared memory (48 KB in all with the static part: ndiag <= 3134).  Every size within H.264 level 6.2
+    // stays below that (ndiag <= 2240, at 2112x16880); a taller picture is refused here rather than failing at launch.
+    // (a property of the kernel binary, the same for both instantiations' 16 warps: read once per process)
+    static_assert(K7_WARPS_I == K7_WARPS_P, "one shared-memory limit for both schedules");
+    static const int max_dyn = [] {
+        cudaFuncAttributes fa;
+        return cudaFuncGetAttributes(&fa, k7_intra_wavefront_kernel<K7_WARPS_I>) == cudaSuccess ? fa.maxDynamicSharedSizeBytes : -1;
+    }();
+    if (dyn_smem > max_dyn) {
+        fprintf(stderr, "b2enc: K7 needs %d bytes of dynamic shared memory for %d x %d macroblocks (%d diagonals), at most %d\n",
+                dyn_smem, mbw, mbh, mbw + 2 * (mbh - 1), max_dyn);
+        return -1;
+    }
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(ncta, nframes, 1);
     cfg.blockDim = dim3((all_intra ? K7_WARPS_I : K7_WARPS_P) * 32, 1, 1);
-    cfg.dynamicSmemBytes = 2 * ndiag * sizeof(int);
+    cfg.dynamicSmemBytes = dyn_smem;
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
