@@ -93,6 +93,10 @@ typedef struct {
                                            behind x264's me=esa): the stream is byte-identical with 0 and 1, only the time differs.
                                            Default 1; the environment variable B2ENC_ME_PRUNE=0/1 overrides it.  Takes effect for
                                            i_merange 32 (presets slow and up); at +-16 the exhaustive kernel is the faster one      */
+    int i_slice_count;                  /* slices per picture (x264 field of the same name): row-aligned, slice k covers macroblock
+                                           rows [(k mbh + n/2) / n, ((k+1) mbh + n/2) / n), n clamped to the picture's mbh rows.
+                                           0 (default) = environment variable B2ENC_SLICES, else 1.  With i_gop_slots = 1 the
+                                           slices of a picture are entropy-coded on several cores at once                          */
 } b2_param_t;
 
 typedef struct {

@@ -44,6 +44,9 @@ typedef struct {
                        /* block-sum lower bound exceeds an exactly evaluated cost are skipped).  Vectors, costs and tie-break  */
                        /* are those of the exhaustive scan; the time is content dependent.  Used for merange 32 without the    */
                        /* wide partition search (partitions == 2); elsewhere the exhaustive kernel is the faster one and runs. */
+    int slices;        /* row-aligned slices per picture (x264 i_slice_count; split: b2_slice_row, b2enc_types.h); 0 or 1: one. */
+                       /* Intra analysis (K3) and reconstruction (K7) see no neighbour in another slice; K7 runs every   */
+                       /* (frame, slice) as its own wavefront.  The loop filter (K8) crosses slice boundaries.             */
 } b2_engine_cfg_t;
 
 b2_engine_t *b2_engine_create(const b2_engine_cfg_t *cfg);      /* NULL on error */

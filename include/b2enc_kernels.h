@@ -56,17 +56,19 @@ int b2k_deblock(uint8_t *y, uint8_t *u, uint8_t *v, int w, int h, int nframes, i
 /* K7 (intra reconstruction on reconstructed neighbours, 8.3 / 8.5) and its cbp pass alone, in one launch, on planes in the
  * padded layout of b2k_deblock: cur_* the source, rec_* the reconstruction (inter macroblocks already reconstructed; read as
  * neighbours, never written); nframes frames one after the other; info / coef [nframes][mbh*mbw]; qp 10..51.
- * all_intra 1: the I-frame schedule (a cluster of up to 8 CTAs per frame), 0: the P-frame schedule (one CTA per frame).
+ * slices: row-aligned slices per frame (b2_slice_count, b2enc_types.h; 0 or 1 = one), each its own unit of work.
+ * all_intra 1: the I-frame schedule (a cluster of up to 8 CTAs per unit), 0: the P-frame schedule (one CTA per unit).
  * Preconditions, as the engine leaves them after K5: intra records are zero apart from mb_type, i16_mode, chroma_mode, i4_mode,
  * i8_modes and cost -- in particular nnz_mask == 0, because K7 ORs its masks in -- and every mode is legal for the
  * neighbours available to its block (K7 does not check).  coef need not be cleared: K7 writes all 26 x 16 levels of an intra
  * macroblock.  Writes cbp, nnz_mask, and for I8x8 i4_mode and transform8x8, of intra records; leaves inter macroblocks alone.
  * rec_*, info and coef are updated in place (padding included); rec_y == NULL only reports the shape.  Refuses a picture whose
- * diagonal tables exceed the kernel's dynamic shared memory (mbw + 2*(mbh-1) > 3134 on a B200).
- * Out (each may be NULL): ncta = CTAs per frame, rounds = tasks of the longest diagonal per warp, dyn_smem = bytes per CTA. */
+ * diagonal tables exceed the kernel's dynamic shared memory (mbw + 2*(rows of the tallest slice - 1) > 3134 on a B200).
+ * Out (each may be NULL), for the tallest slice: ncta = CTAs per unit, rounds = tasks of the longest diagonal per warp,
+ * dyn_smem = bytes per CTA. */
 int b2k_intra_recon(const uint8_t *cur_y, const uint8_t *cur_u, const uint8_t *cur_v, uint8_t *rec_y, uint8_t *rec_u, uint8_t *rec_v,
-                    int w, int h, int nframes, int qp, int all_intra, b2_mbinfo_t *info, b2_mbcoef_t *coef, int *ncta, int *rounds,
-                    int *dyn_smem);
+                    int w, int h, int nframes, int slices, int qp, int all_intra, b2_mbinfo_t *info, b2_mbcoef_t *coef, int *ncta,
+                    int *rounds, int *dyn_smem);
 /* rows per lane-task of the pruned search for +-merange: 5 (+-32) or 3 (+-16) */
 int b2_k1_prune_rows(int merange);
 

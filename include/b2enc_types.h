@@ -59,6 +59,24 @@ static inline int b2_fmt_size_ok(int fmt, int w, int h)
     }
 }
 
+/* Slices (x264 i_slice_count).  A picture of mbh macroblock rows is cut into n = b2_slice_count(i_slice_count, mbh) row-aligned
+ * slices; slice k covers rows [b2_slice_row(k, n, mbh), b2_slice_row(k + 1, n, mbh)).  Because slices are whole rows, the left
+ * neighbour is always in the macroblock's own slice, and the top, top-left and top-right neighbours are unavailable exactly when
+ * the row is the first of its slice (b2_slice_row0(mby, n, mbh) == mby).  0 or 1 means one slice. */
+#if defined(__CUDACC__)
+__host__ __device__
+#endif
+static inline int b2_slice_count(int slices, int mbh) { return slices < 1 ? 1 : (slices > mbh ? mbh : slices); }
+#if defined(__CUDACC__)
+__host__ __device__
+#endif
+static inline int b2_slice_row(int k, int n, int mbh) { return (k * mbh + n / 2) / n; }
+/* first row of the slice that holds row r: slice k = max{k : b2_slice_row(k) <= r} = ((r + 1) n - n/2 - 1) / mbh */
+#if defined(__CUDACC__)
+__host__ __device__
+#endif
+static inline int b2_slice_row0(int r, int n, int mbh) { return b2_slice_row(((r + 1) * n - n / 2 - 1) / mbh, n, mbh); }
+
 /* intra 16x16 modes (H.264 Table 8-4) */
 enum { B2_I16_V = 0, B2_I16_H = 1, B2_I16_DC = 2, B2_I16_PLANE = 3 };
 /* intra chroma modes (H.264 Table 8-5) */

@@ -13,7 +13,7 @@
  * (include/b2enc_filters.h); and when the output name ends in ".mp4" it writes an MP4 with one AVC track from the encoder's
  * b_annexb = 0 payloads (tools/b2_mp4.h + b2_avcc_write), the video half of enc_mp4_write_video_sample (:683-744).
  * Extensions (not in the reference): --size WxH --fps N[/D] for raw input, --merange, --gop, --slots, --device, --devices N (one
- * stream over N GPUs by closed GOP), --8x8dct, --partitions.
+ * stream over N GPUs by closed GOP), --8x8dct, --partitions, --slices N (row-aligned slices per picture, x264's --slices).
  * Regular input files are mmap'ed: the "decoded picture" the reference gets from libavcodec is then a pointer into the page
  * cache and b2_sws_scale's staging copy is the only time the host touches the pixels (pipes fall back to fread).
  */
@@ -33,7 +33,7 @@
 #include "b2_mp4.h"
 
 typedef struct {
-    int silent, width, height, fps_num, fps_den, merange, gop, slots, device, devices, dct8, partitions;
+    int silent, width, height, fps_num, fps_den, merange, gop, slots, device, devices, dct8, partitions, slices;
     long frame_limit;
     const char *input_file, *output_file, *preset, *tune, *profile, *video_filter;
     float quality;
@@ -42,7 +42,7 @@ typedef struct {
 static int parse_cli_options(cli_options_t *o, int argc, char **argv)
 {
     cli_options_t d = {.silent = 0, .width = 0, .height = 0, .fps_num = 25, .fps_den = 1, .merange = 0, .gop = 0, .slots = 0,
-                       .device = 0, .devices = 0, .dct8 = 0, .partitions = 0, .video_filter = NULL, .frame_limit = -1, .input_file = NULL, .output_file = NULL,
+                       .device = 0, .devices = 0, .dct8 = 0, .partitions = 0, .slices = 0, .video_filter = NULL, .frame_limit = -1, .input_file = NULL, .output_file = NULL,
                        .preset = "medium", .tune = "film", .profile = NULL, .quality = 20.0f};   /* av_encode.c:91-106 */
     *o = d;
     struct option long_opts[] = {
@@ -52,7 +52,7 @@ static int parse_cli_options(cli_options_t *o, int argc, char **argv)
         {"size", required_argument, NULL, 5}, {"fps", required_argument, NULL, 6}, {"merange", required_argument, NULL, 7},
         {"gop", required_argument, NULL, 8}, {"slots", required_argument, NULL, 9}, {"device", required_argument, NULL, 10},
         {"filters", required_argument, NULL, 'f'}, {"8x8dct", no_argument, NULL, 11}, {"partitions", required_argument, NULL, 12},
-        {"devices", required_argument, NULL, 13},
+        {"devices", required_argument, NULL, 13}, {"slices", required_argument, NULL, 14},
         {NULL, 0, NULL, 0}};
     int c, idx = 0;
     while ((c = getopt_long(argc, argv, "sl:f:", long_opts, &idx)) != -1) {
@@ -73,6 +73,7 @@ static int parse_cli_options(cli_options_t *o, int argc, char **argv)
         case 11: o->dct8 = 1; break;
         case 12: o->partitions = atoi(optarg); break;
         case 13: o->devices = atoi(optarg); break;
+        case 14: o->slices = atoi(optarg); break;
         default: return 0;
         }
     }
@@ -101,6 +102,7 @@ int main(int argc, char **argv)
     if (!parse_cli_options(&opts, argc, argv)) {
         fprintf(stderr, "usage: %s [--preset p] [--tune t] [--quality q] [--profile p] [--frame-limit n] [--silent]\n"
                         "          [--size WxH --fps N[/D]] [--merange 16|32] [--gop n] [--slots n] [--device n] [--devices n]\n"
+                        "          [--slices n]"
                         "          [--filters hqdn3d,yadif] [--8x8dct] [--partitions 0|1|2] input.{y4m,yuv} output.{h264,mp4}\n", argv[0]);
         return 1;
     }
@@ -131,6 +133,7 @@ int main(int argc, char **argv)
     if (opts.gop) params.i_keyint_max = opts.gop;
     if (opts.slots) params.i_gop_slots = opts.slots;
     params.i_device = opts.device; params.i_devices = opts.devices;
+    params.i_slice_count = opts.slices;
     if (b2_param_apply_profile(&params, opts.profile) != 0) { fprintf(stderr, "b2enc: failed to apply profile %s\n", opts.profile); return 8; }
     b2_t *enc = b2_encoder_open(&params);
     if (!enc) { fprintf(stderr, "b2enc: failed to initialize encoder\n"); return 8; }

@@ -151,24 +151,24 @@ def deblock(y, u, v, info, qp, alpha_off=0, beta_off=0):
 
 def _intra_recon_lib():
     L = lib()
-    L.b2k_intra_recon.argtypes = [C.c_void_p] * 6 + [C.c_int] * 5 + [C.c_void_p] * 5
+    L.b2k_intra_recon.argtypes = [C.c_void_p] * 6 + [C.c_int] * 6 + [C.c_void_p] * 5
     return L
 
 
-def intra_recon_shape(w, h, all_intra):
-    """K7's launch shape for frames of coded size w x h: (CTAs per frame, tasks of the longest diagonal per warp, dynamic shared
-    memory bytes per CTA)"""
+def intra_recon_shape(w, h, all_intra, slices=1):
+    """K7's launch shape for frames of coded size w x h cut into `slices` row-aligned slices: (CTAs per (frame, slice), tasks of
+    the longest diagonal per warp, dynamic shared memory bytes per CTA), for the tallest slice"""
     out = [C.c_int(0) for _ in range(3)]
-    if _intra_recon_lib().b2k_intra_recon(None, None, None, None, None, None, w, h, 1, 26, int(all_intra), None, None,
+    if _intra_recon_lib().b2k_intra_recon(None, None, None, None, None, None, w, h, 1, slices, 26, int(all_intra), None, None,
                                           *[C.addressof(o) for o in out]) != 0:
         raise RuntimeError("b2k_intra_recon failed")
     return tuple(o.value for o in out)
 
 
-def intra_recon(cur, rec, info, coef, qp, all_intra):
+def intra_recon(cur, rec, info, coef, qp, all_intra, slices=1):
     """K7 alone (b2k_intra_recon): cur / rec = (y, u, v) uint8 planes [n, rows, pitch] in the engine's padded layout (see
-    padded_layout), info MBINFO [n, mbs], coef MBCOEF [n, mbs].  Returns (copies of rec y, u, v, info, coef after the launch,
-    (ncta, rounds, dyn_smem))."""
+    padded_layout), info MBINFO [n, mbs], coef MBCOEF [n, mbs], frames of `slices` row-aligned slices.  Returns (copies of rec y,
+    u, v, info, coef after the launch, (ncta, rounds, dyn_smem))."""
     require_gpu()
     cy, cu, cv = (np.ascontiguousarray(p, np.uint8) for p in cur)
     ry, ru, rv = (np.array(p, np.uint8, order="C", copy=True) for p in rec)
@@ -183,7 +183,7 @@ def intra_recon(cur, rec, info, coef, qp, all_intra):
     info = np.array(info, MBINFO, order="C", copy=True).reshape(n, nmb)
     coef = np.array(coef, MBCOEF, order="C", copy=True).reshape(n, nmb)
     out = [C.c_int(0) for _ in range(3)]
-    if _intra_recon_lib().b2k_intra_recon(_p(cy), _p(cu), _p(cv), _p(ry), _p(ru), _p(rv), w, h, n, qp, int(all_intra), _p(info), _p(coef),
+    if _intra_recon_lib().b2k_intra_recon(_p(cy), _p(cu), _p(cv), _p(ry), _p(ru), _p(rv), w, h, n, slices, qp, int(all_intra), _p(info), _p(coef),
                                           *[C.addressof(o) for o in out]) != 0:
         raise RuntimeError("b2k_intra_recon failed")
     return ry, ru, rv, info, coef, tuple(o.value for o in out)
@@ -301,7 +301,7 @@ class EngineCfg(C.Structure):
     _fields_ = [("device", C.c_int), ("width", C.c_int), ("height", C.c_int), ("slots", C.c_int), ("in_fmt", C.c_int),
                 ("in_ring", C.c_int), ("merange", C.c_int), ("qp", C.c_int), ("subpel", C.c_int), ("intra_in_p", C.c_int),
                 ("profile", C.c_int), ("streams", C.c_int), ("deblock", C.c_int), ("transform8x8", C.c_int), ("partitions", C.c_int), ("pack_levels", C.c_int),
-                ("deblock_alpha", C.c_int), ("deblock_beta", C.c_int), ("me_prune", C.c_int)]
+                ("deblock_alpha", C.c_int), ("deblock_beta", C.c_int), ("me_prune", C.c_int), ("slices", C.c_int)]
 
 
 class Engine:
@@ -309,7 +309,7 @@ class Engine:
 
     def __init__(self, width, height, slots=1, fmt="yuv420p", ring=1, merange=16, qp=26, subpel=1, intra_in_p=1,
                  device=0, profile=0, streams=0, deblock=0, transform8x8=0, pack_levels=0, partitions=0, deblock_offsets=(0, 0),
-                 me_prune=0):
+                 me_prune=0, slices=1):
         require_gpu()
         L = lib()
         L.b2_engine_create.restype = C.c_void_p
@@ -349,7 +349,7 @@ class Engine:
         self.L = L
         self.cfg = EngineCfg(device, width, height, slots, FMT[fmt] if isinstance(fmt, str) else fmt, ring, merange, qp,
                              subpel, intra_in_p, profile, streams, deblock, transform8x8, partitions, pack_levels,
-                             deblock_offsets[0], deblock_offsets[1], me_prune)
+                             deblock_offsets[0], deblock_offsets[1], me_prune, slices)
         L.b2_engine_k1_stats.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         self.h = L.b2_engine_create(C.byref(self.cfg))
         if not self.h:
@@ -527,7 +527,7 @@ class Param(C.Structure):
                 ("b_subpel", C.c_int), ("b_intra_in_p", C.c_int), ("i_device", C.c_int), ("i_csp_in", C.c_int),
                 ("b_deblocking_filter", C.c_int), ("b_cabac", C.c_int), ("b_transform_8x8", C.c_int), ("b_partitions", C.c_int),
                 ("i_deblocking_filter_alphac0", C.c_int), ("i_deblocking_filter_beta", C.c_int), ("i_devices", C.c_int),
-                ("b_me_prune", C.c_int)]
+                ("b_me_prune", C.c_int), ("i_slice_count", C.c_int)]
 
 
 class Image(C.Structure):

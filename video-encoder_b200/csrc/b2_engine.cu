@@ -634,7 +634,7 @@ static int encode_group(b2_engine *e, Group &gr, int frame_type, int ns, int rin
     }
     if (do_intra) {
         KScope k(e, st, 4);
-        if (b2_launch_intra_analyse(cur[0], cur[1], cur[2], e->pitch, e->pitchc, e->stride_y, e->stride_c, e->mbw, e->mbh, ns,
+        if (b2_launch_intra_analyse(cur[0], cur[1], cur[2], e->pitch, e->pitchc, e->stride_y, e->stride_c, e->mbw, e->mbh, c.slices, ns,
                                     e->lambda, info, e->d_c16 + om, e->d_c4 + om, e->d_c8 ? e->d_c8 + om : nullptr, st))
             return -1;
     }
@@ -649,7 +649,7 @@ static int encode_group(b2_engine *e, Group &gr, int frame_type, int ns, int rin
     if (do_intra) {
         KScope k(e, st, 6);
         e->launches++;                                   // K7 + its cbp pass
-        if (b2_launch_intra_recon(cur, rec, e->pitch, e->pitchc, e->stride_y, e->stride_c, e->mbw, e->mbh, ns, c.qp, !is_p, info, coef, st))
+        if (b2_launch_intra_recon(cur, rec, e->pitch, e->pitchc, e->stride_y, e->stride_c, e->mbw, e->mbh, c.slices, ns, c.qp, !is_p, info, coef, st))
             return -1;
     }
     if (c.deblock) {

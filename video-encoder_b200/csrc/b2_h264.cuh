@@ -475,14 +475,15 @@ __device__ __forceinline__ int blk8_avail(int q, int mba)
     return a;
 }
 
-// MB-level neighbour availability (one slice per frame: geometric)
-__device__ __forceinline__ int mb_avail(int mbx, int mby, int mbw)
+// MB-level neighbour availability; row0 = first row of the macroblock's slice (b2_slice_row0, b2enc_types.h): the neighbours
+// above are in another slice, so unavailable, when mby == row0
+__device__ __forceinline__ int mb_avail(int mbx, int mby, int mbw, int row0)
 {
     int a = 0;
     if (mbx > 0) a |= 1;
-    if (mby > 0) a |= 2;
-    if (mbx > 0 && mby > 0) a |= 4;
-    if (mby > 0 && mbx < mbw - 1) a |= 8;
+    if (mby > row0) a |= 2;
+    if (mbx > 0 && mby > row0) a |= 4;
+    if (mby > row0 && mbx < mbw - 1) a |= 8;
     return a;
 }
 // availability of 4x4 block b (z order) given the MB's availability

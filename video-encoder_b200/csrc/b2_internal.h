@@ -44,7 +44,7 @@ int b2_launch_me_subpel(const uint8_t *d_cur, const uint8_t *d_ref, int pitch, s
                         b2_mv_t *d_mv8_out /* [nmb][3] */, const b2_mv_t *d_mv9 /* NULL, or K1<PART>'s vectors: wide partition search */,
                         const uint32_t *d_cost9, cudaStream_t st);
 int b2_launch_intra_analyse(const uint8_t *d_y, const uint8_t *d_u, const uint8_t *d_v, int pitch, int pitchc,
-                            size_t stride_y, size_t stride_c, int mbw, int mbh, int nframes, int lambda,
+                            size_t stride_y, size_t stride_c, int mbw, int mbh, int slices, int nframes, int lambda,
                             b2_mbinfo_t *d_info, uint32_t *d_c16, uint32_t *d_c4, uint32_t *d_c8 /* NULL: no I8x8 analysis */,
                             cudaStream_t st);
 int b2_launch_decide_inter(const uint8_t *const cur[3], const uint8_t *const ref[3], uint8_t *const rec[3], int pitch,
@@ -52,12 +52,13 @@ int b2_launch_decide_inter(const uint8_t *const cur[3], const uint8_t *const ref
                            int do_intra, int qp, const b2_mv_t *d_mvq, const uint32_t *d_cost_inter, const uint32_t *d_c16,
                            const uint32_t *d_c4, const uint32_t *d_c8, b2_mbinfo_t *d_info, b2_mbcoef_t *d_coef, b2_mv_t *d_prev_mv,
                            const uint8_t *d_pred_y, int transform8x8, const uint8_t *d_part, const b2_mv_t *d_mv8, cudaStream_t st);
-// K7's launch shape for frames of mbw x mbh macroblocks: ncta = CTAs per frame (one cluster; 1 unless all_intra), rounds =
-// (macroblock, luma | chroma) tasks of the longest anti-diagonal per warp, dyn_smem = dynamic shared memory of one CTA
-void b2_intra_recon_shape(int mbw, int mbh, int all_intra, int *ncta, int *rounds, int *dyn_smem);
+// K7's launch shape for frames of mbw x mbh macroblocks cut into `slices` row-aligned slices (b2_slice_count): one unit per
+// (frame, slice), sized for the tallest slice.  ncta = CTAs per unit (one cluster; 1 unless all_intra), rounds = (macroblock,
+// luma | chroma) tasks of the longest anti-diagonal per warp, dyn_smem = dynamic shared memory of one CTA
+void b2_intra_recon_shape(int mbw, int mbh, int slices, int all_intra, int *ncta, int *rounds, int *dyn_smem);
 // refuses (-1, before any launch) a picture whose diagonal tables exceed the kernel's dynamic shared memory (ndiag > 3134)
 int b2_launch_intra_recon(const uint8_t *const cur[3], uint8_t *const rec[3], int pitch, int pitchc, size_t stride_y,
-                          size_t stride_c, int mbw, int mbh, int nframes, int qp, int all_intra, b2_mbinfo_t *d_info,
+                          size_t stride_c, int mbw, int mbh, int slices, int nframes, int qp, int all_intra, b2_mbinfo_t *d_info,
                           b2_mbcoef_t *d_coef, cudaStream_t st);
 int b2_lambda_for_qp(int qp);
 // K8's launch shape for `nframes` frames of mbw x mbh macroblocks: wavefront 0 = row pipeline, 1 = anti-diagonal wavefront;

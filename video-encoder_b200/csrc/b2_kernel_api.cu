@@ -124,8 +124,8 @@ extern "C" int b2k_deblock(uint8_t *y, uint8_t *u, uint8_t *v, int w, int h, int
 // K7 (+ its cbp pass) alone: as b2k_deblock, the planes, records and levels go to the device as they are and come back whole, so
 // that a caller can see any store outside an intra macroblock
 extern "C" int b2k_intra_recon(const uint8_t *cur_y, const uint8_t *cur_u, const uint8_t *cur_v, uint8_t *rec_y, uint8_t *rec_u,
-                               uint8_t *rec_v, int w, int h, int nframes, int qp, int all_intra, b2_mbinfo_t *info, b2_mbcoef_t *coef,
-                               int *ncta, int *rounds, int *dyn_smem)
+                               uint8_t *rec_v, int w, int h, int nframes, int slices, int qp, int all_intra, b2_mbinfo_t *info,
+                               b2_mbcoef_t *coef, int *ncta, int *rounds, int *dyn_smem)
 {
     if ((w & 15) || (h & 15) || w <= 0 || h <= 0 || nframes <= 0 || qp < 10 || qp > 51) {
         fprintf(stderr, "b2enc: b2k_intra_recon needs w,h multiples of 16, qp 10..51\n");
@@ -133,7 +133,7 @@ extern "C" int b2k_intra_recon(const uint8_t *cur_y, const uint8_t *cur_u, const
     }
     const int mbw = w / 16, mbh = h / 16;
     int nc, rd, ds;
-    b2_intra_recon_shape(mbw, mbh, all_intra, &nc, &rd, &ds);
+    b2_intra_recon_shape(mbw, mbh, slices, all_intra, &nc, &rd, &ds);
     if (ncta) *ncta = nc;
     if (rounds) *rounds = rd;
     if (dyn_smem) *dyn_smem = ds;
@@ -159,7 +159,7 @@ extern "C" int b2k_intra_recon(const uint8_t *cur_y, const uint8_t *cur_u, const
     B2_CUDA_OK(cudaMemcpy(d_coef.p, coef, ncf, cudaMemcpyHostToDevice));
     const uint8_t *const cur[3] = {(const uint8_t *)d_cy.p, (const uint8_t *)d_cu.p, (const uint8_t *)d_cv.p};
     uint8_t *const rec[3] = {(uint8_t *)d_ry.p, (uint8_t *)d_ru.p, (uint8_t *)d_rv.p};
-    if (b2_launch_intra_recon(cur, rec, pitch, pitchc, sy, sc, mbw, mbh, nframes, qp, all_intra, (b2_mbinfo_t *)d_info.p,
+    if (b2_launch_intra_recon(cur, rec, pitch, pitchc, sy, sc, mbw, mbh, slices, nframes, qp, all_intra, (b2_mbinfo_t *)d_info.p,
                               (b2_mbcoef_t *)d_coef.p, 0))
         return -1;
     B2_CUDA_OK(cudaDeviceSynchronize());

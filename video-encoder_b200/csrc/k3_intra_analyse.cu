@@ -23,7 +23,7 @@ template <bool I8>
 __global__ void __launch_bounds__(K3_THREADS)
 k3_intra_analyse_kernel(const uint8_t *__restrict__ cur_y, const uint8_t *__restrict__ cur_u,
                         const uint8_t *__restrict__ cur_v, int pitch, int pitchc, size_t stride_y, size_t stride_c,
-                        int mbw, int mbh, int nmb_total, int lambda, b2_mbinfo_t *__restrict__ info,
+                        int mbw, int mbh, int nslices, int nmb_total, int lambda, b2_mbinfo_t *__restrict__ info,
                         uint32_t *__restrict__ cost_i16, uint32_t *__restrict__ cost_i4, uint32_t *__restrict__ cost_i8)
 {
     const int gt = blockIdx.x * K3_THREADS + threadIdx.x;
@@ -34,7 +34,7 @@ k3_intra_analyse_kernel(const uint8_t *__restrict__ cur_y, const uint8_t *__rest
     const int per_frame = mbw * mbh;
     const int frame = mbi / per_frame, r = mbi - frame * per_frame;
     const int mby = r / mbw, mbx = r - mby * mbw;
-    const int mba = b2::mb_avail(mbx, mby, mbw);
+    const int mba = b2::mb_avail(mbx, mby, mbw, nslices > 1 ? b2_slice_row0(mby, nslices, mbh) : 0);
     const int bx = b2::blk_x(b) * 4, by = b2::blk_y(b) * 4;
 
     const uint8_t *sy = cur_y + frame * stride_y + (size_t)(B2_PAD + mby * 16) * pitch + B2_PAD + mbx * 16;
@@ -280,16 +280,16 @@ k3_intra_analyse_kernel(const uint8_t *__restrict__ cur_y, const uint8_t *__rest
 }  // namespace
 
 int b2_launch_intra_analyse(const uint8_t *d_y, const uint8_t *d_u, const uint8_t *d_v, int pitch, int pitchc,
-                            size_t stride_y, size_t stride_c, int mbw, int mbh, int nframes, int lambda,
+                            size_t stride_y, size_t stride_c, int mbw, int mbh, int slices, int nframes, int lambda,
                             b2_mbinfo_t *d_info, uint32_t *d_c16, uint32_t *d_c4, uint32_t *d_c8, cudaStream_t st)
 {
-    const int nmb = mbw * mbh * nframes;
+    const int nmb = mbw * mbh * nframes, ns = b2_slice_count(slices, mbh);
     const int blocks = (nmb * 16 + K3_THREADS - 1) / K3_THREADS;
     if (d_c8)
-        k3_intra_analyse_kernel<true><<<blocks, K3_THREADS, 0, st>>>(d_y, d_u, d_v, pitch, pitchc, stride_y, stride_c, mbw, mbh, nmb,
+        k3_intra_analyse_kernel<true><<<blocks, K3_THREADS, 0, st>>>(d_y, d_u, d_v, pitch, pitchc, stride_y, stride_c, mbw, mbh, ns, nmb,
                                                                      lambda, d_info, d_c16, d_c4, d_c8);
     else
-        k3_intra_analyse_kernel<false><<<blocks, K3_THREADS, 0, st>>>(d_y, d_u, d_v, pitch, pitchc, stride_y, stride_c, mbw, mbh, nmb,
+        k3_intra_analyse_kernel<false><<<blocks, K3_THREADS, 0, st>>>(d_y, d_u, d_v, pitch, pitchc, stride_y, stride_c, mbw, mbh, ns, nmb,
                                                                       lambda, d_info, d_c16, d_c4, nullptr);
     B2_CUDA_OK(cudaGetLastError());
     return 0;

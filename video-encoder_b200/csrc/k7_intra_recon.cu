@@ -6,9 +6,11 @@
 //
 // Intra prediction reads reconstructed left / top / top-left / top-right neighbours, so macroblocks on
 // one anti-diagonal d = mbx + 2*mby are independent and diagonals are a serial chain (inter MBs of the
-// frame were already reconstructed by K5).  The chain is pure latency, so the kernel is built to make
-// one link short:
-//   * one THREAD-BLOCK CLUSTER per frame (up to 8 CTAs x 16 warps), hardware cluster barrier
+// frame were already reconstructed by K5).  Prediction never reads across a slice boundary, and slices are
+// whole macroblock rows (b2_slice_row, b2enc_types.h), so every slice is a chain of its own: the unit of work
+// is one (frame, slice), walking d = mbx + 2*(mby - row0) over its own rows.  The chain is pure latency, so
+// the kernel is built to make one link short:
+//   * one THREAD-BLOCK CLUSTER per unit (up to 8 CTAs x 16 warps), hardware cluster barrier
 //     (barrier.cluster release/acquire) between diagonals -> every MB of a diagonal has its own warps;
 //   * luma and chroma of a macroblock are separate warp tasks (they depend on different planes);
 //   * I4x4 luma: the MB's neighbourhood lives in a per-warp shared-memory tile; the sixteen blocks run as
@@ -148,10 +150,10 @@ __device__ __constant__ uint8_t c_izz[16] = {0, 1, 5, 6, 2, 4, 7, 12, 3, 8, 11, 
 __device__ __forceinline__ int zidx(int x, int y) { return (x & 1) | ((y & 1) << 1) | ((x >> 1) << 2) | ((y >> 1) << 3); }
 
 // ---- luma task ------------------------------------------------------------------------------------------
-__device__ void k7_luma_task(int lane, K7Warp &ws, const FramePlanes &fp, int frame, int mbx, int mby, int mbw, int qp,
+__device__ void k7_luma_task(int lane, K7Warp &ws, const FramePlanes &fp, int frame, int mbx, int mby, int mbw, int row0, int qp,
                              b2_mbinfo_t *mi, b2_mbcoef_t *cf)
 {
-    const int mba = mb_avail(mbx, mby, mbw);
+    const int mba = mb_avail(mbx, mby, mbw, row0);
     const bool hasT = mba & 2, hasL = mba & 1;
     const int mb_type = mi->mb_type;
     const size_t offy = (size_t)(B2_PAD + mby * 16) * fp.pitch + B2_PAD + mbx * 16;
@@ -420,10 +422,10 @@ __device__ void k7_luma_task(int lane, K7Warp &ws, const FramePlanes &fp, int fr
 }
 
 // ---- chroma task: lanes 0..7 own (plane, 4x4 block) ---------------------------------------------------------
-__device__ void k7_chroma_task(int lane, const FramePlanes &fp, int frame, int mbx, int mby, int mbw, int qp,
+__device__ void k7_chroma_task(int lane, const FramePlanes &fp, int frame, int mbx, int mby, int mbw, int row0, int qp,
                                b2_mbinfo_t *mi, b2_mbcoef_t *cf)
 {
-    const int mba = mb_avail(mbx, mby, mbw);
+    const int mba = mb_avail(mbx, mby, mbw, row0);
     const bool hasT = mba & 2, hasL = mba & 1;
     const bool act = lane < 8;
     const int pl = (lane >> 2) & 1, k = lane & 3, cbx = (k & 1) * 4, cby = (k >> 1) * 4;
@@ -485,17 +487,18 @@ __device__ void k7_chroma_task(int lane, const FramePlanes &fp, int frame, int m
 // stream group then waits on K7 -- so both variants use 16
 template <int WARPS>
 __global__ void __launch_bounds__(WARPS * 32)
-k7_intra_wavefront_kernel(FramePlanes fp, int mbw, int mbh, int qp, b2_mbinfo_t *__restrict__ info,
+k7_intra_wavefront_kernel(FramePlanes fp, int mbw, int mbh, int nslices, int qp, b2_mbinfo_t *__restrict__ info,
                           b2_mbcoef_t *__restrict__ coef)
 {
     constexpr int K7_WARPS = WARPS;
     extern __shared__ int s_diag_cnt[];                 // [ndiag] diagonal holds intra MBs | [ndiag] list of those diagonals
     __shared__ K7Warp s_warp[K7_WARPS];
-    const int frame = blockIdx.y;
+    const int frame = blockIdx.y / nslices, slice = blockIdx.y - frame * nslices;   // the unit: rows [row0, row0 + srows)
+    const int row0 = b2_slice_row(slice, nslices, mbh), srows = b2_slice_row(slice + 1, nslices, mbh) - row0;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int ncta = (int)cluster_nctarank(), crank = (int)cluster_ctarank();
     const int gwarp = crank * K7_WARPS + warp, nwarps = ncta * K7_WARPS;
-    const int ndiag = mbw + 2 * (mbh - 1);
+    const int ndiag = mbw + 2 * (srows - 1);
     b2_mbinfo_t *finfo = info + (size_t)frame * mbw * mbh;
     b2_mbcoef_t *fcoef = coef + (size_t)frame * mbw * mbh;
     // Anti-diagonals that hold intra macroblocks, as an ascending list (identical in every CTA of the cluster).  P frames hold
@@ -504,11 +507,11 @@ k7_intra_wavefront_kernel(FramePlanes fp, int mbw, int mbh, int qp, b2_mbinfo_t 
     __shared__ int s_nlist;
     for (int i = threadIdx.x; i < ndiag; i += blockDim.x) s_diag_cnt[i] = 0;
     __syncthreads();
-    const int nmb = mbw * mbh;
+    const int mb0 = row0 * mbw, nmb = srows * mbw;                           // the unit's macroblocks, from mb0
     for (int i0 = threadIdx.x; i0 < nmb; i0 += 4 * blockDim.x) {            // four independent loads in flight per thread
         uint8_t ty[4];
 #pragma unroll
-        for (int j = 0; j < 4; j++) { const int i = i0 + j * blockDim.x; ty[j] = i < nmb ? finfo[i].mb_type : (uint8_t)B2_MB_P16x16; }
+        for (int j = 0; j < 4; j++) { const int i = i0 + j * blockDim.x; ty[j] = i < nmb ? finfo[mb0 + i].mb_type : (uint8_t)B2_MB_P16x16; }
 #pragma unroll
         for (int j = 0; j < 4; j++) {
             const int i = i0 + j * blockDim.x;
@@ -531,14 +534,14 @@ k7_intra_wavefront_kernel(FramePlanes fp, int mbw, int mbh, int qp, b2_mbinfo_t 
     const int nlist = s_nlist;
     for (int k = 0; k < nlist; k++) {
         const int d = s_diag_list[k];
-        const int y_lo = max(0, (d - mbw + 2) >> 1), y_hi = min(mbh - 1, d >> 1);
+        const int y_lo = max(0, (d - mbw + 2) >> 1), y_hi = min(srows - 1, d >> 1);     // rows relative to row0
         const int ntask = 2 * (y_hi - y_lo + 1);        // (MB, luma|chroma)
         for (int t = gwarp; t < ntask; t += nwarps) {
-            const int mby = y_lo + (t >> 1), mbx = d - 2 * mby;
+            const int y = y_lo + (t >> 1), mbx = d - 2 * y, mby = row0 + y;
             const int i = mby * mbw + mbx;
             if (finfo[i].mb_type != B2_MB_P16x16) {
-                if (t & 1) k7_chroma_task(lane, fp, frame, mbx, mby, mbw, qp, &finfo[i], &fcoef[i]);
-                else k7_luma_task(lane, s_warp[warp], fp, frame, mbx, mby, mbw, qp, &finfo[i], &fcoef[i]);
+                if (t & 1) k7_chroma_task(lane, fp, frame, mbx, mby, mbw, row0, qp, &finfo[i], &fcoef[i]);
+                else k7_luma_task(lane, s_warp[warp], fp, frame, mbx, mby, mbw, row0, qp, &finfo[i], &fcoef[i]);
             }
         }
         if (ncta > 1) cluster_barrier();
@@ -558,12 +561,15 @@ k7_cbp_kernel(b2_mbinfo_t *__restrict__ info, int n)
 
 }  // namespace
 
-void b2_intra_recon_shape(int mbw, int mbh, int all_intra, int *ncta, int *rounds, int *dyn_smem)
+void b2_intra_recon_shape(int mbw, int mbh, int slices, int all_intra, int *ncta, int *rounds, int *dyn_smem)
 {
-    const int ndiag = mbw + 2 * (mbh - 1);
-    const int maxdiag = mbh < (mbw + 1) / 2 ? mbh : (mbw + 1) / 2;      // macroblocks on the longest anti-diagonal
-    // I frames: every MB of a diagonal gets its own luma + chroma warp (cluster of up to 8 CTAs).  P frames hold few,
-    // scattered intra MBs: one CTA per frame keeps the footprint at one SM so that other streams' kernels keep the rest.
+    const int ns = b2_slice_count(slices, mbh);
+    int rows = 0;                                                        // the tallest slice sizes every unit
+    for (int k = 0; k < ns; k++) rows = max(rows, b2_slice_row(k + 1, ns, mbh) - b2_slice_row(k, ns, mbh));
+    const int ndiag = mbw + 2 * (rows - 1);
+    const int maxdiag = rows < (mbw + 1) / 2 ? rows : (mbw + 1) / 2;    // macroblocks on the longest anti-diagonal
+    // I frames: every MB of a diagonal gets its own luma + chroma warp (cluster of up to 8 CTAs per slice).  P frames hold few,
+    // scattered intra MBs: one CTA per (frame, slice) keeps the footprint small so that other streams' kernels keep the rest.
     const int warps = all_intra ? K7_WARPS_I : K7_WARPS_P;
     int n = 1;
     if (all_intra)
@@ -574,15 +580,16 @@ void b2_intra_recon_shape(int mbw, int mbh, int all_intra, int *ncta, int *round
 }
 
 int b2_launch_intra_recon(const uint8_t *const cur[3], uint8_t *const rec[3], int pitch, int pitchc, size_t stride_y,
-                          size_t stride_c, int mbw, int mbh, int nframes, int qp, int all_intra, b2_mbinfo_t *d_info,
+                          size_t stride_c, int mbw, int mbh, int slices, int nframes, int qp, int all_intra, b2_mbinfo_t *d_info,
                           b2_mbcoef_t *d_coef, cudaStream_t st)
 {
+    const int ns = b2_slice_count(slices, mbh);
     FramePlanes fp;
     for (int i = 0; i < 3; i++) { fp.cur[i] = cur[i]; fp.ref[i] = nullptr; fp.rec[i] = rec[i]; }
     fp.pitch = pitch; fp.pitchc = pitchc; fp.stride_y = stride_y; fp.stride_c = stride_c;
     int ncta, rounds, dyn_smem;
-    b2_intra_recon_shape(mbw, mbh, all_intra, &ncta, &rounds, &dyn_smem);
-    // The diagonal tables grow with mbw + 2*mbh and sit beside the per-warp tiles; the kernel does not opt in to more than the
+    b2_intra_recon_shape(mbw, mbh, ns, all_intra, &ncta, &rounds, &dyn_smem);
+    // The diagonal tables grow with mbw + 2*mbh (of the tallest slice) and sit beside the per-warp tiles; the kernel does not opt in to more than the
     // default dynamic shared memory (48 KB in all with the static part: ndiag <= 3134).  Every size within H.264 level 6.2
     // stays below that (ndiag <= 2240, at 2112x16880); a taller picture is refused here rather than failing at launch.
     // (a property of the kernel binary, the same for both instantiations' 16 warps: read once per process)
@@ -592,12 +599,12 @@ int b2_launch_intra_recon(const uint8_t *const cur[3], uint8_t *const rec[3], in
         return cudaFuncGetAttributes(&fa, k7_intra_wavefront_kernel<K7_WARPS_I>) == cudaSuccess ? fa.maxDynamicSharedSizeBytes : -1;
     }();
     if (dyn_smem > max_dyn) {
-        fprintf(stderr, "b2enc: K7 needs %d bytes of dynamic shared memory for %d x %d macroblocks (%d diagonals), at most %d\n",
-                dyn_smem, mbw, mbh, mbw + 2 * (mbh - 1), max_dyn);
+        fprintf(stderr, "b2enc: K7 needs %d bytes of dynamic shared memory for %d x %d macroblocks in %d slices (%d diagonals), at most %d\n",
+                dyn_smem, mbw, mbh, ns, dyn_smem / (2 * (int)sizeof(int)), max_dyn);
         return -1;
     }
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(ncta, nframes, 1);
+    cfg.gridDim = dim3(ncta, nframes * ns, 1);
     cfg.blockDim = dim3((all_intra ? K7_WARPS_I : K7_WARPS_P) * 32, 1, 1);
     cfg.dynamicSmemBytes = dyn_smem;
     cfg.stream = st;
@@ -605,8 +612,8 @@ int b2_launch_intra_recon(const uint8_t *const cur[3], uint8_t *const rec[3], in
     attr[0].id = cudaLaunchAttributeClusterDimension;
     attr[0].val.clusterDim.x = ncta; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
-    if (all_intra) B2_CUDA_OK(cudaLaunchKernelEx(&cfg, k7_intra_wavefront_kernel<K7_WARPS_I>, fp, mbw, mbh, qp, d_info, d_coef));
-    else B2_CUDA_OK(cudaLaunchKernelEx(&cfg, k7_intra_wavefront_kernel<K7_WARPS_P>, fp, mbw, mbh, qp, d_info, d_coef));
+    if (all_intra) B2_CUDA_OK(cudaLaunchKernelEx(&cfg, k7_intra_wavefront_kernel<K7_WARPS_I>, fp, mbw, mbh, ns, qp, d_info, d_coef));
+    else B2_CUDA_OK(cudaLaunchKernelEx(&cfg, k7_intra_wavefront_kernel<K7_WARPS_P>, fp, mbw, mbh, ns, qp, d_info, d_coef));
     const int n = mbw * mbh * nframes;
     k7_cbp_kernel<<<(n + 255) / 256, 256, 0, st>>>(d_info, n);
     B2_CUDA_OK(cudaGetLastError());

@@ -6,7 +6,7 @@
  *
  * ITU-T H.264 9.3: context initialisation (9.3.1.1, Tables 9-12..9-23 -> b2h_cabac_ctx.h), binarisations
  * (9.3.2), context index derivation (9.3.3.1) and the arithmetic encoder (9.3.4.2: Figures 9-7..9-12).
- * One slice per picture, one reference frame, frame macroblocks only, constant QP (mb_qp_delta = 0).
+ * Row-aligned slices (contexts initialised per slice), one reference frame, frame macroblocks only, constant QP (mb_qp_delta = 0).
  * Pinned by decoding the stream with libavcodec's H.264 decoder (tests/test_cabac.py).
  */
 #include <pthread.h>
@@ -323,21 +323,22 @@ CABAC_INLINE void cabac_mb_type_intra(cabac_t *c, cabac_reg_t *r, const b2_mbinf
 }
 
 /* ---- slice ---------------------------------------------------------------------------------------------------*/
-size_t b2h_write_slice_cabac(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, int frame_num, int idr_pic_id,
+size_t b2h_write_slice_cabac(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, int frame_num, int idr_pic_id, int nrows,
                              const b2_mbinfo_t *info, b2h_levels_t *lv, uint8_t *out, size_t cap)
 {
     bs_t bs, *b = &bs;
     cabac_t cb, *c = &cb;
     cabac_reg_t rg, *r = &rg;
-    const int mbw = e->mbw, mbh = e->mbh, nmb = mbw * mbh, is_p = frame_type == B2_FRAME_P;
-    const int ys = 4 * mbw, cs = 2 * mbw;
+    const int mbw = e->mbw, row0 = e->row0, is_p = frame_type == B2_FRAME_P;
+    const int last = (row0 + nrows) * mbw - 1;                                 /* the slice's last macroblock */
+    const int ys = 4 * mbw, cs = 2 * mbw, y4top = 4 * row0, y2top = 2 * row0;
     const uint8_t *blk_x = b2h_blk_x, *blk_y = b2h_blk_y;
     bs_init(b, e->rbsp, e->rbsp_cap);
-    b2h_slice_header(b, s, is_p, frame_num, idr_pic_id);
+    b2h_slice_header(b, s, is_p, frame_num, idr_pic_id, row0 * mbw);
     if (b->nbits) bs_put(b, 8 - b->nbits, (1u << (8 - b->nbits)) - 1);    /* cabac_alignment_one_bit */
     cabac_init(c, r, b, is_p ? 1 : 0, s->qp);                                  /* cabac_init_idc 0 */
 
-    for (int mby = 0; mby < mbh; mby++)
+    for (int mby = row0; mby < row0 + nrows; mby++)
         for (int mbx = 0; mbx < mbw; mbx++) {
             const int mi = mby * mbw + mbx;
             const b2_mbinfo_t *m = &info[mi];
@@ -346,7 +347,7 @@ size_t b2h_write_slice_cabac(b2h_entropy_t *e, const b2h_seq_t *s, int frame_typ
             const int cbp_l = m->cbp & 15, cbp_c = m->cbp >> 4;
             const int intra = m->mb_type != B2_MB_P16x16;
             nb_t nb;
-            nb.availA = mbx > 0; nb.availB = mby > 0;
+            nb.availA = mbx > 0; nb.availB = mby > row0;
             nb.fA = nb.availA ? e->mbf[mi - 1] : 0; nb.fB = nb.availB ? e->mbf[mi - mbw] : 0;
             nb.cbpA = nb.availA ? e->cbp[mi - 1] : 0; nb.cbpB = nb.availB ? e->cbp[mi - mbw] : 0;
             /* reset this MB's neighbour state; filled in below as syntax elements are coded */
@@ -372,7 +373,7 @@ size_t b2h_write_slice_cabac(b2h_entropy_t *e, const b2h_seq_t *s, int frame_typ
                 cabac_encode(c, 11 + (nb.availA && !(nb.fA & B2H_MBF_SKIP)) + (nb.availB && !(nb.fB & B2H_MBF_SKIP)), skip);
                 if (skip) {
                     e->mbf[mi] = B2H_MBF_SKIP;
-                    cabac_terminate(c, mi == nmb - 1);                  /* end_of_slice_flag */
+                    cabac_terminate(c, mi == last);                     /* end_of_slice_flag */
                     continue;
                 }
                 /* mb_type (Table 9-36, P slices): 16x16 "000", 8x8 "001", 16x8 "011", 8x16 "010" */
@@ -391,8 +392,8 @@ size_t b2h_write_slice_cabac(b2h_entropy_t *e, const b2h_seq_t *s, int frame_typ
                         const b2_mv_t mvp = b2h_mv_pred(e, x4, y4, pw, dir);
                         const int d[2] = {mv.x - mvp.x, mv.y - mvp.y};
                         for (int k = 0; k < 2; k++) {
-                            /* |mvd| of the 4x4 blocks left of / above the partition (0 outside the picture, in intra and skipped MBs) */
-                            const int sum = (x4 > 0 ? e->mvd[k][y4 * ys + x4 - 1] : 0) + (y4 > 0 ? e->mvd[k][(y4 - 1) * ys + x4] : 0);
+                            /* |mvd| of the 4x4 blocks left of / above the partition (0 outside the slice, in intra and skipped MBs) */
+                            const int sum = (x4 > 0 ? e->mvd[k][y4 * ys + x4 - 1] : 0) + (y4 > y4top ? e->mvd[k][(y4 - 1) * ys + x4] : 0);
                             cabac_mvd(c, r, k ? 47 : 40, sum, d[k]);
                         }
                         const int ax = abs(d[0]) > 255 ? 255 : abs(d[0]), ay = abs(d[1]) > 255 ? 255 : abs(d[1]);
@@ -415,7 +416,7 @@ size_t b2h_write_slice_cabac(b2h_entropy_t *e, const b2h_seq_t *s, int frame_typ
                     for (int k = 0; k < 16; k += step) {
                         const int x = mbx * 4 + blk_x[k], y = mby * 4 + blk_y[k];
                         int pred = 2;
-                        if (x > 0 && y > 0) {
+                        if (x > 0 && y > y4top) {
                             const int a = e->i4[y * ys + x - 1], bb = e->i4[(y - 1) * ys + x];
                             pred = a < bb ? a : bb;
                         }
@@ -481,7 +482,7 @@ size_t b2h_write_slice_cabac(b2h_entropy_t *e, const b2h_seq_t *s, int frame_typ
                     }
                     /* neighbouring 4x4 blocks: inside the picture the map holds 0 for every block that was not coded */
                     const int ta = cbf_term(x > 0, x > 0 ? e->nnz_y[y * ys + x - 1] : 0, intra);
-                    const int tb = cbf_term(y > 0, y > 0 ? e->nnz_y[(y - 1) * ys + x] : 0, intra);
+                    const int tb = cbf_term(y > y4top, y > y4top ? e->nnz_y[(y - 1) * ys + x] : 0, intra);
                     if (m->mb_type == B2_MB_I16x16)
                         e->nnz_y[y * ys + x] = (uint8_t)cabac_residual(c, r, 1, cblk[k] + 1, 15, ta + 2 * tb);
                     else
@@ -501,12 +502,12 @@ size_t b2h_write_slice_cabac(b2h_entropy_t *e, const b2h_seq_t *s, int frame_typ
                         for (int k = 0; k < 4; k++) {
                             const int x = mbx * 2 + (k & 1), y = mby * 2 + (k >> 1);
                             const int ta = cbf_term(x > 0, x > 0 ? e->nnz_c[p][y * cs + x - 1] : 0, intra);
-                            const int tb = cbf_term(y > 0, y > 0 ? e->nnz_c[p][(y - 1) * cs + x] : 0, intra);
+                            const int tb = cbf_term(y > y2top, y > y2top ? e->nnz_c[p][(y - 1) * cs + x] : 0, intra);
                             e->nnz_c[p][y * cs + x] = (uint8_t)cabac_residual(c, r, 4, cblk[16 + 4 * p + k] + 1, 15, ta + 2 * tb);
                         }
             }
             e->mbf[mi] = (uint8_t)flags;
-            cabac_terminate(c, mi == nmb - 1);                              /* end_of_slice_flag */
+            cabac_terminate(c, mi == last);                                 /* end_of_slice_flag */
         }
     b->pos = (size_t)(c->p - b->buf);                                       /* the flush already byte-aligned the RBSP */
     if (b->overflow || c->overflow) return 0;

@@ -328,17 +328,18 @@ static int write_residual(bs_t *b, const int16_t *l, int maxn, int nC)
 }
 
 /* ---- neighbour helpers ---------------------------------------------------------------------------*/
-static inline int pred_nc(const uint8_t *map, int stride, int x, int y)
+/* y0: first block row of the slice (blocks above it are in another slice) */
+static inline int pred_nc(const uint8_t *map, int stride, int x, int y, int y0)
 {
-    int hasA = x > 0, hasB = y > 0;
+    int hasA = x > 0, hasB = y > y0;
     int nA = hasA ? map[y * stride + x - 1] : 0, nB = hasB ? map[(y - 1) * stride + x] : 0;
     if (hasA && hasB) return (nA + nB + 1) >> 1;
     return hasA ? nA : (hasB ? nB : 0);
 }
 
-void b2h_slice_header(bs_t *b, const b2h_seq_t *s, int is_p, int frame_num, int idr_pic_id)
+void b2h_slice_header(bs_t *b, const b2h_seq_t *s, int is_p, int frame_num, int idr_pic_id, int first_mb)
 {
-    bs_ue(b, 0);                                   /* first_mb_in_slice                   */
+    bs_ue(b, (uint32_t)first_mb);                  /* first_mb_in_slice                   */
     bs_ue(b, is_p ? 5 : 7);                        /* slice_type: all slices P / all I    */
     bs_ue(b, 0);                                   /* pic_parameter_set_id                */
     bs_put(b, 8, (uint32_t)frame_num & 255u);      /* frame_num, log2_max_frame_num = 8   */
@@ -374,36 +375,55 @@ void b2h_info_unpack(const b2_mbinfo_packed_t *packed, b2_mbinfo_t *info, int n)
 /* ---- slice ---------------------------------------------------------------------------------------*/
 const int16_t b2h_zero_levels[64] = {0};
 
-static size_t write_slice(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, int frame_num, int idr_pic_id,
-                          const b2_mbinfo_t *info, b2h_levels_t *lv, uint8_t *out, size_t cap);
+static size_t write_slice(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, int frame_num, int idr_pic_id, int first_row,
+                          int nrows, const b2_mbinfo_t *info, b2h_levels_t *lv, uint8_t *out, size_t cap);
+
+size_t b2h_write_slice_rows(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, int frame_num, int idr_pic_id, int first_row,
+                            int nrows, const b2_mbinfo_t *info, const b2_mbcoef_t *coef, uint8_t *out, size_t cap)
+{
+    b2h_levels_t lv = {coef, NULL, 0, 0};
+    return write_slice(e, s, frame_type, frame_num, idr_pic_id, first_row, nrows, info, &lv, out, cap);
+}
+
+size_t b2h_write_slice_rows_packed(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, int frame_num, int idr_pic_id, int first_row,
+                                   int nrows, const b2_mbinfo_t *info, const uint8_t *packed, size_t packed_bytes, uint8_t *out,
+                                   size_t cap)
+{
+    /* the stream holds the whole picture: the slice's first macroblock follows the present blocks of the ones in front of it */
+    size_t pos = 0;
+    for (int i = 0; first_row > 0 && i < first_row * e->mbw; i++) pos += 32u * (size_t)__builtin_popcount(b2_coef_present(&info[i]));
+    b2h_levels_t lv = {NULL, packed, pos, packed_bytes};
+    return write_slice(e, s, frame_type, frame_num, idr_pic_id, first_row, nrows, info, &lv, out, cap);
+}
 
 size_t b2h_write_slice(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, int frame_num, int idr_pic_id,
                        const b2_mbinfo_t *info, const b2_mbcoef_t *coef, uint8_t *out, size_t cap)
 {
-    b2h_levels_t lv = {coef, NULL, 0, 0};
-    return write_slice(e, s, frame_type, frame_num, idr_pic_id, info, &lv, out, cap);
+    return b2h_write_slice_rows(e, s, frame_type, frame_num, idr_pic_id, 0, e->mbh, info, coef, out, cap);
 }
 
 size_t b2h_write_slice_packed(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, int frame_num, int idr_pic_id,
                               const b2_mbinfo_t *info, const uint8_t *packed, size_t packed_bytes, uint8_t *out, size_t cap)
 {
-    b2h_levels_t lv = {NULL, packed, 0, packed_bytes};
-    return write_slice(e, s, frame_type, frame_num, idr_pic_id, info, &lv, out, cap);
+    return b2h_write_slice_rows_packed(e, s, frame_type, frame_num, idr_pic_id, 0, e->mbh, info, packed, packed_bytes, out, cap);
 }
 
-static size_t write_slice(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, int frame_num, int idr_pic_id,
-                          const b2_mbinfo_t *info, b2h_levels_t *lv, uint8_t *out, size_t cap)
+static size_t write_slice(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, int frame_num, int idr_pic_id, int first_row,
+                          int nrows, const b2_mbinfo_t *info, b2h_levels_t *lv, uint8_t *out, size_t cap)
 {
     bs_t bs, *b = &bs;
-    const int mbw = e->mbw, mbh = e->mbh, is_p = frame_type == B2_FRAME_P;
+    const int mbw = e->mbw, is_p = frame_type == B2_FRAME_P;
     const int ys = 4 * mbw, cs = 2 * mbw;
-    if (s->cabac) return b2h_write_slice_cabac(e, s, frame_type, frame_num, idr_pic_id, info, lv, out, cap);
+    if (first_row < 0 || nrows < 1 || first_row + nrows > e->mbh) return 0;
+    e->row0 = first_row;
+    const int y4top = 4 * first_row, y2top = 2 * first_row;
+    if (s->cabac) return b2h_write_slice_cabac(e, s, frame_type, frame_num, idr_pic_id, nrows, info, lv, out, cap);
     bs_init(b, e->rbsp, e->rbsp_cap);
-    b2h_slice_header(b, s, is_p, frame_num, idr_pic_id);
+    b2h_slice_header(b, s, is_p, frame_num, idr_pic_id, first_row * mbw);
 
     /* slice_data() */
     int skip_run = 0;
-    for (int mby = 0; mby < mbh; mby++)
+    for (int mby = first_row; mby < first_row + nrows; mby++)
         for (int mbx = 0; mbx < mbw; mbx++) {
             const int mi = mby * mbw + mbx;
             const b2_mbinfo_t *m = &info[mi];
@@ -452,7 +472,7 @@ static size_t write_slice(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, 
                     for (int k = 0; k < 16; k += i8 ? 4 : 1) {
                         int x = mbx * 4 + blk_x[k], y = mby * 4 + blk_y[k];
                         int pred = 2;
-                        if (x > 0 && y > 0) {
+                        if (x > 0 && y > y4top) {
                             int a = e->i4[y * ys + x - 1], bb = e->i4[(y - 1) * ys + x];
                             pred = a < bb ? a : bb;
                         }
@@ -473,11 +493,11 @@ static size_t write_slice(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, 
 
             /* residual() */
             if (m->mb_type == B2_MB_I16x16) {
-                write_residual(b, cblk[24], 16, pred_nc(e->nnz_y, ys, mbx * 4, mby * 4));
+                write_residual(b, cblk[24], 16, pred_nc(e->nnz_y, ys, mbx * 4, mby * 4, y4top));
                 if (cbp_l)
                     for (int k = 0; k < 16; k++) {
                         int x = mbx * 4 + blk_x[k], y = mby * 4 + blk_y[k];
-                        e->nnz_y[y * ys + x] = (uint8_t)write_residual(b, cblk[k] + 1, 15, pred_nc(e->nnz_y, ys, x, y));
+                        e->nnz_y[y * ys + x] = (uint8_t)write_residual(b, cblk[k] + 1, 15, pred_nc(e->nnz_y, ys, x, y, y4top));
                     }
             } else if (m->transform8x8 && s->transform8x8) {
                 /* 8x8 transform with CAVLC (7.3.5.3.2): the 64 levels are split into four interleaved 4x4 blocks */
@@ -487,13 +507,13 @@ static size_t write_slice(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, 
                     int16_t l4[16];
                     const int16_t *l8 = cblk[k & ~3];
                     for (int i = 0; i < 16; i++) l4[i] = l8[4 * i + (k & 3)];
-                    e->nnz_y[y * ys + x] = (uint8_t)write_residual(b, l4, 16, pred_nc(e->nnz_y, ys, x, y));
+                    e->nnz_y[y * ys + x] = (uint8_t)write_residual(b, l4, 16, pred_nc(e->nnz_y, ys, x, y, y4top));
                 }
             } else {
                 for (int k = 0; k < 16; k++) {
                     if (!(cbp_l & (1 << (k >> 2)))) continue;
                     int x = mbx * 4 + blk_x[k], y = mby * 4 + blk_y[k];
-                    e->nnz_y[y * ys + x] = (uint8_t)write_residual(b, cblk[k], 16, pred_nc(e->nnz_y, ys, x, y));
+                    e->nnz_y[y * ys + x] = (uint8_t)write_residual(b, cblk[k], 16, pred_nc(e->nnz_y, ys, x, y, y4top));
                 }
             }
             if (cbp_c) {
@@ -504,7 +524,7 @@ static size_t write_slice(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, 
                         for (int k = 0; k < 4; k++) {
                             int x = mbx * 2 + (k & 1), y = mby * 2 + (k >> 1);
                             e->nnz_c[p][y * cs + x] =
-                                (uint8_t)write_residual(b, cblk[16 + 4 * p + k] + 1, 15, pred_nc(e->nnz_c[p], cs, x, y));
+                                (uint8_t)write_residual(b, cblk[16 + 4 * p + k] + 1, 15, pred_nc(e->nnz_c[p], cs, x, y, y2top));
                         }
             }
         }

@@ -20,6 +20,10 @@
  * The x264 contract main() relies on holds: 0 = no output yet, delayed_frames() = frames in - frames out, encode(NULL)
  * returns one frame per call until the encoder is empty (av_encode.c:971-974, :1076-1083).
  * i_gop_slots = 1 (tune zerolatency) encodes every picture synchronously in the caller's thread (zero delay).
+ *
+ * Slices (i_slice_count n > 1, b2_slice_row in b2enc_types.h): a picture is SPS/PPS (IDR) + n slice NALs.  With several GOP slots
+ * an entropy job stays one frame and writes its slices one after the other (frames are already coded in parallel); in zero-delay
+ * mode the slices of the one picture are written at the same time by a pool of min(n, cores - 1) threads started at open.
  */
 #define _GNU_SOURCE                 /* syscall(SYS_gettid): per-thread nice value of the entropy workers */
 #include <pthread.h>
@@ -36,11 +40,12 @@
 #include "b2h_entropy.h"
 #include "b2h_picture.h"
 
+typedef struct { int off, size, type, ref; } nalrec_t;
 typedef struct {
     uint8_t *data;
     int size;
     int nal_count;
-    int nal_off[3], nal_size[3], nal_type[3], nal_ref[3];
+    nalrec_t *nal;              /* [slices + 2]; owned like data */
     int64_t pts;
     int key;
     int ready;
@@ -115,7 +120,24 @@ struct b2_encoder {
     double st_open, st_caller_slot_wait, st_caller_put, st_worker_busy;
     double st_dev_cpu[B2_MAX_DEVICES], st_dev_copy[B2_MAX_DEVICES], st_dev_gpu_wait[B2_MAX_DEVICES], st_dev_idle[B2_MAX_DEVICES];
     long st_dev_rounds[B2_MAX_DEVICES];
-    b2_nal_t nals[3];
+    int ns;                     /* slices per picture                                              */
+    b2_nal_t *nals;             /* [ns + 2] */
+    /* zero-delay slice pool (i_gop_slots = 1, ns > 1), guarded by sp_mu: the caller posts one picture (sp_gen++), the threads take
+     * slices k = sp_next++ and write slice k into sp_buf[k] (sp_len[k] bytes, 0 = overflow), the caller waits for sp_done == ns */
+    int sp_n;
+    pthread_t sp_thread[B2_MAX_WORKERS];
+    b2h_entropy_t *sp_ent[B2_MAX_WORKERS];
+    uint8_t **sp_buf;
+    size_t *sp_cap, *sp_len;
+    pthread_mutex_t sp_mu;
+    pthread_cond_t sp_cv_go, sp_cv_done;
+    long sp_gen;
+    int sp_next, sp_done, sp_stop;
+    const b2_mbinfo_t *sp_info;
+    const uint8_t *sp_packed;
+    size_t sp_packed_bytes;
+    int sp_t;
+    int64_t sp_gop_index;
 };
 
 /* ---- picture registry (b2h_picture.h) ------------------------------------------------------------------------------ */
@@ -262,6 +284,17 @@ int b2_param_apply_profile(b2_param_t *p, const char *profile)
 /* ---- open / close -------------------------------------------------------------------------------------------------- */
 static void *worker_main(void *arg);
 static void *dev_main(void *arg);
+static void *slice_main(void *arg);
+
+static int slice_count_wanted(const b2_param_t *p)
+{
+    int n = p->i_slice_count;
+    if (n <= 0) {                                        /* an unmodified av_encode.c cannot set the field: environment */
+        const char *e = getenv("B2ENC_SLICES");
+        n = e ? atoi(e) : 1;
+    }
+    return n < 1 ? 1 : n;
+}
 
 static int device_count_wanted(const b2_param_t *p)
 {
@@ -336,6 +369,7 @@ b2_t *b2_encoder_open(b2_param_t *p)
             }
         }
     }
+    cfg.slices = slice_count_wanted(p);
     cfg.slots = h->S; cfg.streams = h->S;             /* one stream group per slot: every GOP advances on its own */
     cfg.in_ring = h->S == 1 ? 1 : h->L;
     for (int d = 0; d < h->N; d++) {
@@ -356,9 +390,36 @@ b2_t *b2_encoder_open(b2_param_t *p)
     h->seq.deblock = p->b_deblocking_filter;
     h->seq.deblock_alpha = p->i_deblocking_filter_alphac0; h->seq.deblock_beta = p->i_deblocking_filter_beta;
     h->seq.cabac = p->b_cabac != 0; h->seq.transform8x8 = p->b_transform_8x8 != 0;
-    h->scratch_cap = (size_t)h->nmb * 3072 + 65536;
+    h->ns = b2_slice_count(cfg.slices, h->mbh);
+    h->scratch_cap = (size_t)h->nmb * 3072 + 65536 * (size_t)h->ns;
     h->scratch = (uint8_t *)malloc(h->scratch_cap);
-    if (!h->ent || !h->scratch) { b2_encoder_close(h); return NULL; }
+    h->nals = (b2_nal_t *)calloc((size_t)h->ns + 2, sizeof(b2_nal_t));
+    if (!h->ent || !h->scratch || !h->nals) { b2_encoder_close(h); return NULL; }
+    pthread_mutex_init(&h->sp_mu, NULL);
+    pthread_cond_init(&h->sp_cv_go, NULL); pthread_cond_init(&h->sp_cv_done, NULL);
+    if (h->S == 1 && h->ns > 1) {
+        long ncpu = sysconf(_SC_NPROCESSORS_ONLN);
+        int nt = ncpu > 2 ? (int)ncpu - 1 : 1;
+        if (nt > h->ns) nt = h->ns;
+        if (nt > B2_MAX_WORKERS) nt = B2_MAX_WORKERS;
+        h->sp_buf = (uint8_t **)calloc((size_t)h->ns, sizeof(uint8_t *));
+        h->sp_cap = (size_t *)calloc((size_t)h->ns, sizeof(size_t)); h->sp_len = (size_t *)calloc((size_t)h->ns, sizeof(size_t));
+        if (!h->sp_buf || !h->sp_cap || !h->sp_len) { b2_encoder_close(h); return NULL; }
+        for (int k = 0; k < h->ns; k++) {
+            const int rows = b2_slice_row(k + 1, h->ns, h->mbh) - b2_slice_row(k, h->ns, h->mbh);
+            h->sp_cap[k] = (size_t)rows * h->mbw * 3072 + 65536;
+            if (!(h->sp_buf[k] = (uint8_t *)malloc(h->sp_cap[k]))) { b2_encoder_close(h); return NULL; }
+        }
+        for (int i = 0; i < nt; i++)
+            if (!(h->sp_ent[i] = b2h_entropy_create(h->mbw, h->mbh))) { b2_encoder_close(h); return NULL; }
+        pthread_mutex_lock(&h->sp_mu);                   /* the threads look themselves up in sp_thread[] under the lock */
+        for (int i = 0; i < nt; i++) {
+            if (pthread_create(&h->sp_thread[i], NULL, slice_main, h)) break;
+            h->sp_n++;
+        }
+        pthread_mutex_unlock(&h->sp_mu);
+        if (h->sp_n == 0) { b2_encoder_close(h); return NULL; }
+    }
     if (h->S > 1) {
         long ncpu = sysconf(_SC_NPROCESSORS_ONLN);
         int nw = ncpu > 2 ? (int)ncpu - 1 : 1;          /* frames, not GOPs, are the unit of work: use the cores there are */
@@ -405,6 +466,17 @@ void b2_encoder_close(b2_t *h)
     for (int d = 0; d < h->N; d++)
         if (h->dev[d].started) pthread_join(h->dev[d].thread, NULL);
     for (int i = 0; i < h->nworkers; i++) pthread_join(h->workers[i], NULL);
+    if (h->sp_n) {
+        pthread_mutex_lock(&h->sp_mu);
+        h->sp_stop = 1;
+        pthread_cond_broadcast(&h->sp_cv_go);
+        pthread_mutex_unlock(&h->sp_mu);
+        for (int i = 0; i < h->sp_n; i++) pthread_join(h->sp_thread[i], NULL);
+    }
+    for (int i = 0; i < B2_MAX_WORKERS; i++) b2h_entropy_destroy(h->sp_ent[i]);
+    if (h->sp_buf)
+        for (int k = 0; k < h->ns; k++) free(h->sp_buf[k]);
+    free(h->sp_buf); free(h->sp_cap); free(h->sp_len);
     if (h->stats && h->S > 1) {
         const double wall = now_s() - h->st_open;
         fprintf(stderr, "b2enc stats: %lld frames, %.3f s since open | caller: %.3f s waiting for a GOP slot / the fifo, %.3f s handing pictures over | "
@@ -421,9 +493,9 @@ void b2_encoder_close(b2_t *h)
     free(h->jobs);
     for (int i = 0; i < h->pool_n; i++) free(h->pool[i]);
     if (h->fifo)
-        for (int i = 0; i < h->fifo_cap; i++) free(h->fifo[i].data);
+        for (int i = 0; i < h->fifo_cap; i++) { free(h->fifo[i].data); free(h->fifo[i].nal); }
     free(h->fifo);
-    free(h->zout.data); free(h->scratch); free(h->ret_buf);
+    free(h->zout.data); free(h->zout.nal); free(h->scratch); free(h->ret_buf); free(h->nals);
     b2h_entropy_destroy(h->ent);
     for (int d = 0; d < B2_MAX_DEVICES; d++) {
         if (h->dev[d].eng) { b2h_picture_forget_engine(h->dev[d].eng); b2_engine_destroy(h->dev[d].eng); }
@@ -431,6 +503,10 @@ void b2_encoder_close(b2_t *h)
     }
     pthread_mutex_destroy(&h->mu);
     pthread_cond_destroy(&h->cv_job); pthread_cond_destroy(&h->cv_space); pthread_cond_destroy(&h->cv_out);
+    if (h->nals) {                                       /* initialised together with the table */
+        pthread_mutex_destroy(&h->sp_mu);
+        pthread_cond_destroy(&h->sp_cv_go); pthread_cond_destroy(&h->sp_cv_done);
+    }
     free(h);
 }
 
@@ -474,34 +550,92 @@ static void put_prefix(uint8_t *d, int annexb, size_t nal_size)
     else { d[0] = (uint8_t)(nal_size >> 24); d[1] = (uint8_t)(nal_size >> 16); d[2] = (uint8_t)(nal_size >> 8); d[3] = (uint8_t)nal_size; }
 }
 
+static void add_nal(b2_t *h, outframe_t *o, uint8_t *at, size_t pos, size_t n, int type, int ref)
+{
+    put_prefix(at, h->p.b_annexb, n);
+    o->nal[o->nal_count].off = (int)pos; o->nal[o->nal_count].size = (int)n + 4;
+    o->nal[o->nal_count].type = type; o->nal[o->nal_count].ref = ref;
+    o->nal_count++;
+}
+
+/* slice k of the picture (macroblock rows b2_slice_row(k) .. b2_slice_row(k + 1)) as one NAL into out[0..cap) */
+static size_t write_slice_k(b2_t *h, b2h_entropy_t *ent, int k, const b2_mbinfo_t *info, const uint8_t *packed, size_t packed_bytes,
+                            int t, int64_t gop_index, uint8_t *out, size_t cap)
+{
+    const int r0 = b2_slice_row(k, h->ns, h->mbh), r1 = b2_slice_row(k + 1, h->ns, h->mbh);
+    return b2h_write_slice_rows_packed(ent, &h->seq, t == 0 ? B2_FRAME_I : B2_FRAME_P, t, (int)(gop_index & 0xffff), r0, r1 - r0, info,
+                                       packed, packed_bytes, out, cap);
+}
+
+/* zero-delay slice pool: one thread of it */
+static void *slice_main(void *arg)
+{
+    b2_t *h = (b2_t *)arg;
+    b2h_entropy_t *ent = NULL;
+    long seen = 0;
+    pthread_mutex_lock(&h->sp_mu);
+    for (int i = 0; i < h->sp_n; i++)
+        if (pthread_equal(h->sp_thread[i], pthread_self())) ent = h->sp_ent[i];
+    for (;;) {
+        while (!h->sp_stop && h->sp_gen == seen) pthread_cond_wait(&h->sp_cv_go, &h->sp_mu);
+        if (h->sp_stop) break;
+        seen = h->sp_gen;
+        while (h->sp_next < h->ns) {
+            const int k = h->sp_next++;
+            const b2_mbinfo_t *info = h->sp_info; const uint8_t *packed = h->sp_packed;
+            const size_t packed_bytes = h->sp_packed_bytes; const int t = h->sp_t; const int64_t gi = h->sp_gop_index;
+            pthread_mutex_unlock(&h->sp_mu);
+            const size_t n = ent ? write_slice_k(h, ent, k, info, packed, packed_bytes, t, gi, h->sp_buf[k] + 4, h->sp_cap[k] - 4) : 0;
+            pthread_mutex_lock(&h->sp_mu);
+            h->sp_len[k] = n;
+            if (++h->sp_done == h->ns) pthread_cond_signal(&h->sp_cv_done);
+        }
+    }
+    pthread_mutex_unlock(&h->sp_mu);
+    return NULL;
+}
+
 /* entropy-code one frame's results into *o (data, size, NAL table, key) */
 static int finish_frame(b2_t *h, b2h_entropy_t *ent, uint8_t *s, const b2_mbinfo_t *info, const uint8_t *packed, size_t packed_bytes,
                         int t, int64_t gop_index, outframe_t *o)
 {
     size_t pos = 0;
     o->nal_count = 0;
+    free(o->nal);
+    o->nal = (nalrec_t *)malloc(sizeof(nalrec_t) * ((size_t)h->ns + 2));
+    if (!o->nal) return -1;
     const int is_idr = t == 0;
     if (is_idr) {
         for (int k = 0; k < 2; k++) {
             size_t n = k == 0 ? b2h_write_sps(&h->seq, s + pos + 4, h->scratch_cap - pos - 4)
                               : b2h_write_pps(&h->seq, s + pos + 4, h->scratch_cap - pos - 4);
             if (!n) return -1;
-            put_prefix(s + pos, h->p.b_annexb, n);
-            o->nal_off[o->nal_count] = (int)pos; o->nal_size[o->nal_count] = (int)n + 4;
-            o->nal_type[o->nal_count] = k == 0 ? B2_NAL_SPS : B2_NAL_PPS; o->nal_ref[o->nal_count] = 3;
-            o->nal_count++;
+            add_nal(h, o, s + pos, pos, n, k == 0 ? B2_NAL_SPS : B2_NAL_PPS, 3);
             pos += n + 4;
         }
     }
     if (!info || !packed) return -1;
-    size_t n = b2h_write_slice_packed(ent, &h->seq, is_idr ? B2_FRAME_I : B2_FRAME_P, t, (int)(gop_index & 0xffff), info, packed,
-                                      packed_bytes, s + pos + 4, h->scratch_cap - pos - 4);
-    if (!n) { fprintf(stderr, "b2enc: slice buffer overflow\n"); return -1; }
-    put_prefix(s + pos, h->p.b_annexb, n);
-    o->nal_off[o->nal_count] = (int)pos; o->nal_size[o->nal_count] = (int)n + 4;
-    o->nal_type[o->nal_count] = is_idr ? B2_NAL_SLICE_IDR : B2_NAL_SLICE; o->nal_ref[o->nal_count] = is_idr ? 3 : 2;
-    o->nal_count++;
-    pos += n + 4;
+    if (h->sp_n) {                                        /* zero delay, several slices: the pool writes them at the same time */
+        pthread_mutex_lock(&h->sp_mu);
+        h->sp_info = info; h->sp_packed = packed; h->sp_packed_bytes = packed_bytes; h->sp_t = t; h->sp_gop_index = gop_index;
+        h->sp_next = 0; h->sp_done = 0; h->sp_gen++;
+        pthread_cond_broadcast(&h->sp_cv_go);
+        while (h->sp_done < h->ns) pthread_cond_wait(&h->sp_cv_done, &h->sp_mu);
+        pthread_mutex_unlock(&h->sp_mu);
+    }
+    for (int k = 0; k < h->ns; k++) {
+        size_t n;
+        if (h->sp_n) {
+            n = h->sp_len[k];
+            if (n && n + 4 <= h->scratch_cap - pos) memcpy(s + pos + 4, h->sp_buf[k] + 4, n);
+            else n = 0;
+        } else {
+            n = write_slice_k(h, ent, k, info, packed, packed_bytes, t, gop_index, s + pos + 4, h->scratch_cap - pos - 4);
+        }
+        if (!n) { fprintf(stderr, "b2enc: slice buffer overflow\n"); return -1; }
+        add_nal(h, o, s + pos, pos, n, is_idr ? B2_NAL_SLICE_IDR : B2_NAL_SLICE, is_idr ? 3 : 2);
+        pos += n + 4;
+    }
     free(o->data);
     o->data = (uint8_t *)malloc(pos);
     if (!o->data) return -1;
@@ -547,11 +681,11 @@ static void *worker_main(void *arg)
         pthread_mutex_lock(&h->mu);
         h->st_worker_busy += w1 - w0;
         res_give_locked(h, j.res, j.res_cap);
-        if (rc) { h->error = 1; free(o.data); }
+        if (rc) { h->error = 1; free(o.data); free(o.nal); }
         else {
             outframe_t *dst = &h->fifo[j.frame % h->fifo_cap];
             o.pts = dst->pts;                              /* written by the caller's thread when the picture came in */
-            free(dst->data);
+            free(dst->data); free(dst->nal);
             *dst = o;
             dst->ready = 1;
         }
@@ -701,8 +835,8 @@ static int return_frame(b2_t *h, outframe_t *o, b2_nal_t **pp_nal, int *pi_nal, 
     free(h->ret_buf);
     h->ret_buf = o->data; o->data = NULL;                           /* hand the payload over; valid until the next call */
     for (int i = 0; i < o->nal_count; i++) {
-        h->nals[i].i_ref_idc = o->nal_ref[i]; h->nals[i].i_type = o->nal_type[i];
-        h->nals[i].i_payload = o->nal_size[i]; h->nals[i].p_payload = h->ret_buf + o->nal_off[i];
+        h->nals[i].i_ref_idc = o->nal[i].ref; h->nals[i].i_type = o->nal[i].type;
+        h->nals[i].i_payload = o->nal[i].size; h->nals[i].p_payload = h->ret_buf + o->nal[i].off;
     }
     *pp_nal = h->nals; *pi_nal = o->nal_count;
     if (pic_out) {
@@ -850,8 +984,10 @@ int b2_encoder_encode(b2_t *h, b2_nal_t **pp_nal, int *pi_nal, b2_picture_t *pic
     outframe_t *head = &h->fifo[h->frames_out % h->fifo_cap];
     if (h->frames_out == h->frames_in || !head->ready) { pthread_mutex_unlock(&h->mu); return 0; }
     outframe_t o = *head;
-    head->data = NULL; head->ready = 0;
+    head->data = NULL; head->nal = NULL; head->ready = 0;
     h->frames_out++;
     pthread_mutex_unlock(&h->mu);
-    return return_frame(h, &o, pp_nal, pi_nal, pic_out);
+    const int n = return_frame(h, &o, pp_nal, pi_nal, pic_out);
+    free(o.nal);
+    return n;
 }

@@ -36,12 +36,21 @@ void b2h_entropy_destroy(b2h_entropy_t *e);
  * start code / length prefix) into out[0..cap) and returns its size, or 0 on overflow. */
 size_t b2h_write_sps(const b2h_seq_t *s, uint8_t *out, size_t cap);
 size_t b2h_write_pps(const b2h_seq_t *s, uint8_t *out, size_t cap);
+/* the whole picture as one slice; info / coef [mbh * mbw] */
 size_t b2h_write_slice(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type /* B2_FRAME_* */, int frame_num,
                        int idr_pic_id, const b2_mbinfo_t *info, const b2_mbcoef_t *coef,
                        uint8_t *out, size_t cap);
 /* same, reading the levels from the engine's packed stream (b2_engine_packed, layout in b2enc_types.h) */
 size_t b2h_write_slice_packed(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, int frame_num, int idr_pic_id,
                               const b2_mbinfo_t *info, const uint8_t *packed, size_t packed_bytes, uint8_t *out, size_t cap);
+/* the slice of macroblock rows [first_row, first_row + nrows) of a picture cut into row-aligned slices (b2_slice_row,
+ * b2enc_types.h); info / coef / packed hold the whole picture.  A writer reads nothing above first_row, so writers with their
+ * own scratch (b2h_entropy_create) may write the slices of one picture at the same time. */
+size_t b2h_write_slice_rows(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, int frame_num, int idr_pic_id, int first_row,
+                            int nrows, const b2_mbinfo_t *info, const b2_mbcoef_t *coef, uint8_t *out, size_t cap);
+size_t b2h_write_slice_rows_packed(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, int frame_num, int idr_pic_id,
+                                   int first_row, int nrows, const b2_mbinfo_t *info, const uint8_t *packed, size_t packed_bytes,
+                                   uint8_t *out, size_t cap);
 
 /* the 24-byte decision records that cross PCIe (b2_mbinfo_packed_t, include/b2enc_types.h) <-> b2_mbinfo_t, n macroblocks */
 void b2h_info_pack(const b2_mbinfo_t *info, b2_mbinfo_packed_t *packed, int n);

@@ -8,9 +8,12 @@
 #include "b2h_bits.h"
 #include "b2h_entropy.h"
 
-/* per-encoder scratch: neighbour maps of the picture being written (one slice per picture, raster order) */
+/* per-encoder scratch: neighbour maps of the picture being written (raster order).  Slices are whole macroblock rows
+ * (b2_slice_row, b2enc_types.h): a slice reads nothing above its first row, row0, so writers with their own scratch may code the
+ * slices of one picture at the same time. */
 struct b2h_entropy {
     int mbw, mbh;
+    int row0;                /* first macroblock row of the slice being written                   */
     uint8_t *nnz_y;          /* [4mbh][4mbw] total_coeff of each luma 4x4                         */
     uint8_t *nnz_c[2];       /* [2mbh][2mbw] total_coeff of each chroma AC 4x4                    */
     int8_t *i4;              /* [4mbh][4mbw] intra4x4 pred mode (2 for non-I4x4 MBs)              */
@@ -70,14 +73,15 @@ static inline b2_mv_t b2h_mv_pred(const b2h_entropy_t *e, int x4, int y4, int w4
     const int st = 4 * e->mbw;
     b2_mv_t z = {0, 0}, mvA = z, mvB = z, mvC = z;
     int refA = -1, refB = -1, refC = -1;
-    const int hasA = x4 > 0, hasB = y4 > 0;
-    /* C = block above and to the right of the partition; it must lie inside the picture and precede the partition in
+    const int top = 4 * e->row0;                          /* first 4x4 row of the slice */
+    const int hasA = x4 > 0, hasB = y4 > top;
+    /* C = block above and to the right of the partition; it must lie inside the slice and precede the partition in
      * decoding order: always true in the macroblock row above, inside the current row only left of the MB's right edge */
-    int hasC = y4 > 0 && x4 + w4 < st && ((y4 & 3) == 0 || (x4 & 3) + w4 < 4);
+    int hasC = y4 > top && x4 + w4 < st && ((y4 & 3) == 0 || (x4 & 3) + w4 < 4);
     if (hasA) { refA = e->ref4[y4 * st + x4 - 1]; mvA = e->mv4[y4 * st + x4 - 1]; }
     if (hasB) { refB = e->ref4[(y4 - 1) * st + x4]; mvB = e->mv4[(y4 - 1) * st + x4]; }
     if (hasC) { refC = e->ref4[(y4 - 1) * st + x4 + w4]; mvC = e->mv4[(y4 - 1) * st + x4 + w4]; }
-    else if (x4 > 0 && y4 > 0) { hasC = 1; refC = e->ref4[(y4 - 1) * st + x4 - 1]; mvC = e->mv4[(y4 - 1) * st + x4 - 1]; }   /* D */
+    else if (x4 > 0 && y4 > top) { hasC = 1; refC = e->ref4[(y4 - 1) * st + x4 - 1]; mvC = e->mv4[(y4 - 1) * st + x4 - 1]; }   /* D */
     if (dir == B2H_PRED_A && refA == 0) return mvA;
     if (dir == B2H_PRED_B && refB == 0) return mvB;
     if (dir == B2H_PRED_C && refC == 0) return mvC;
@@ -94,7 +98,7 @@ static inline b2_mv_t b2h_skip_mv(const b2h_entropy_t *e, int mbx, int mby)
 {
     const int st = 4 * e->mbw, x4 = 4 * mbx, y4 = 4 * mby;
     b2_mv_t z = {0, 0};
-    if (mbx == 0 || mby == 0) return z;
+    if (mbx == 0 || mby == e->row0) return z;
     const int iA = y4 * st + x4 - 1, iB = (y4 - 1) * st + x4;
     if (e->ref4[iA] == 0 && e->mv4[iA].x == 0 && e->mv4[iA].y == 0) return z;
     if (e->ref4[iB] == 0 && e->mv4[iB].x == 0 && e->mv4[iB].y == 0) return z;
@@ -131,8 +135,9 @@ static inline b2_mv_t b2h_mb_mv(const b2_mbinfo_t *m, int x, int y)
     return mv;
 }
 /* slice_header() 7.3.3 up to and including the deblocking fields */
-void b2h_slice_header(bs_t *b, const b2h_seq_t *s, int is_p, int frame_num, int idr_pic_id);
-size_t b2h_write_slice_cabac(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, int frame_num, int idr_pic_id,
+void b2h_slice_header(bs_t *b, const b2h_seq_t *s, int is_p, int frame_num, int idr_pic_id, int first_mb);
+/* rows [e->row0, e->row0 + nrows) */
+size_t b2h_write_slice_cabac(b2h_entropy_t *e, const b2h_seq_t *s, int frame_type, int frame_num, int idr_pic_id, int nrows,
                              const b2_mbinfo_t *info, b2h_levels_t *lv, uint8_t *out, size_t cap);
 extern const uint8_t b2h_blk_x[16], b2h_blk_y[16];
 
