@@ -77,6 +77,15 @@ int b2_k1_prune_rows(int merange);
 int b2k_me_fullpel_parts(const uint8_t *cur_y, const uint8_t *ref_y, int w, int h, int nframes, int merange,
                          const b2_mv_t *pmv, int lambda, b2_mv_t *mv9_out, uint32_t *cost9_out, int iters, float *kernel_ms);
 
+/* K2 alone: half- then quarter-pel SATD refinement around the full-pel vectors mv_full ([nframes][mbs], each component within
+ * +-32), as in the engine's P frames.  cur_y/ref_y, pmv and kernel_ms as for b2k_me_fullpel.  subpel 0 prices the full-pel
+ * vector only.  Outputs per MB (each may be NULL): mv_out quarter-pel vector, cost_out its cost, pred_out the 16x16
+ * motion-compensated luma prediction (256 bytes, raster).  partitions 1 with subpel 1 refines the shapes 16x8 / 8x16 / 8x8 as
+ * well: part_out = B2_PART_*, mv8_out[3] = vectors of quadrants 1..3 (mv_out is quadrant 0's); otherwise both are left 0. */
+int b2k_me_subpel(const uint8_t *cur_y, const uint8_t *ref_y, int w, int h, int nframes, const b2_mv_t *mv_full, const b2_mv_t *pmv,
+                  int lambda, int subpel, int partitions, b2_mv_t *mv_out, uint32_t *cost_out, uint8_t *pred_out, uint8_t *part_out,
+                  b2_mv_t *mv8_out, int iters, float *kernel_ms);
+
 /* sustained VABSDIFF4 lane-instructions/s of the chip (roofline denominator of K1) */
 double b2_bench_vabsdiff4_peak(int device, int outer, int reps, double *ms_best);
 

@@ -212,6 +212,32 @@ def me_fullpel_parts(cur_y, ref_y, merange, pmv=None, lam=0, iters=0):
     return mv, cost, (ms.value if iters > 0 else None)
 
 
+def me_subpel(cur_y, ref_y, mv_full, pmv=None, lam=0, subpel=1, partitions=0, iters=0):
+    """K2 alone (b2k_me_subpel): cur_y/ref_y uint8 [n,h,w] (or [h,w]), mv_full MV [n,mbs] full-pel vectors (components within
+    +-32).  Returns (mv[n,mbs] quarter-pel, cost[n,mbs], pred uint8 [n,mbs,16,16], part[n,mbs], mv8[n,mbs,3], kernel_ms|None);
+    part and mv8 stay 0 unless partitions and subpel are both set."""
+    require_gpu()
+    cur_y = np.ascontiguousarray(cur_y, np.uint8); ref_y = np.ascontiguousarray(ref_y, np.uint8)
+    if cur_y.ndim == 2:
+        cur_y = cur_y[None]; ref_y = ref_y[None]
+    n, h, w = cur_y.shape
+    nmb = (w // 16) * (h // 16)
+    mv_full = np.ascontiguousarray(mv_full, MV).reshape(n, nmb)
+    if pmv is not None:
+        pmv = np.ascontiguousarray(pmv, MV).reshape(n, nmb)
+    mv = np.zeros((n, nmb), MV); cost = np.zeros((n, nmb), np.uint32); pred = np.zeros((n, nmb, 16, 16), np.uint8)
+    part = np.zeros((n, nmb), np.uint8); mv8 = np.zeros((n, nmb, 3), MV)
+    ms = C.c_float(0)
+    L = lib()
+    L.b2k_me_subpel.argtypes = [C.c_void_p, C.c_void_p] + [C.c_int] * 3 + [C.c_void_p] * 2 + [C.c_int] * 3 + [C.c_void_p] * 5 + \
+        [C.c_int, C.c_void_p]
+    rc = L.b2k_me_subpel(_p(cur_y), _p(ref_y), w, h, n, _p(mv_full), _p(pmv), lam, subpel, partitions, _p(mv), _p(cost), _p(pred),
+                         _p(part), _p(mv8), iters, C.addressof(ms) if iters > 0 else None)
+    if rc != 0:
+        raise RuntimeError("b2k_me_subpel failed (%d)" % rc)
+    return mv, cost, pred, part, mv8, (ms.value if iters > 0 else None)
+
+
 def vabsdiff4_peak(device=0, outer=256, reps=5):
     require_gpu()
     ms = C.c_double(0)

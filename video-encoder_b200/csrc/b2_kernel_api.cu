@@ -185,6 +185,64 @@ extern "C" int b2k_me_fullpel_parts(const uint8_t *cur_y, const uint8_t *ref_y, 
     return me_fullpel_impl(cur_y, ref_y, w, h, nframes, merange, pmv, lambda, nullptr, nullptr, mv9_out, cost9_out, iters, kernel_ms);
 }
 
+extern "C" int b2k_me_subpel(const uint8_t *cur_y, const uint8_t *ref_y, int w, int h, int nframes, const b2_mv_t *mv_full,
+                             const b2_mv_t *pmv, int lambda, int subpel, int partitions, b2_mv_t *mv_out, uint32_t *cost_out,
+                             uint8_t *pred_out, uint8_t *part_out, b2_mv_t *mv8_out, int iters, float *kernel_ms)
+{
+    if ((w & 15) || (h & 15) || w <= 0 || h <= 0 || nframes <= 0 || !mv_full || lambda < 0) {
+        fprintf(stderr, "b2enc: b2k_me_subpel needs w,h multiples of 16 and the full-pel vectors\n");
+        return -1;
+    }
+    const int mbw = w / 16, mbh = h / 16;
+    const size_t nmb = (size_t)mbw * mbh * nframes;
+    for (size_t i = 0; i < nmb; i++)
+        if (abs(mv_full[i].x) > 32 || abs(mv_full[i].y) > 32) {
+            fprintf(stderr, "b2enc: b2k_me_subpel: full-pel vector (%d,%d) outside +-32\n", mv_full[i].x, mv_full[i].y);
+            return -1;
+        }
+    DevBuf d_cur, d_ref, d_mvf, d_pmv, d_mv, d_cost, d_pred, d_part, d_mv8;
+    int pitch, rows;
+    if (upload_padded(d_cur, cur_y, w, h, nframes, B2_PAD, &pitch, &rows)) return -1;
+    if (upload_padded(d_ref, ref_y, w, h, nframes, B2_PAD, &pitch, &rows)) return -1;
+    if (d_mvf.alloc(nmb * sizeof(b2_mv_t)) || d_mv.alloc(nmb * sizeof(b2_mv_t)) || d_cost.alloc(nmb * 4) || d_pred.alloc(nmb * 256) ||
+        d_part.alloc(nmb) || d_mv8.alloc(nmb * 3 * sizeof(b2_mv_t)))
+        return -1;
+    B2_CUDA_OK(cudaMemcpy(d_mvf.p, mv_full, nmb * sizeof(b2_mv_t), cudaMemcpyHostToDevice));
+    B2_CUDA_OK(cudaMemset(d_part.p, 0, nmb));
+    B2_CUDA_OK(cudaMemset(d_mv8.p, 0, nmb * 3 * sizeof(b2_mv_t)));
+    if (pmv) {
+        if (d_pmv.alloc(nmb * sizeof(b2_mv_t))) return -1;
+        B2_CUDA_OK(cudaMemcpy(d_pmv.p, pmv, nmb * sizeof(b2_mv_t), cudaMemcpyHostToDevice));
+    }
+    auto launch = [&]() {
+        return b2_launch_me_subpel((const uint8_t *)d_cur.p, (const uint8_t *)d_ref.p, pitch, (size_t)pitch * rows, mbw, mbh, nframes,
+                                   (const b2_mv_t *)d_mvf.p, (const b2_mv_t *)d_pmv.p, lambda, subpel, (b2_mv_t *)d_mv.p,
+                                   (uint32_t *)d_cost.p, (uint8_t *)d_pred.p, partitions ? (uint8_t *)d_part.p : nullptr,
+                                   partitions ? (b2_mv_t *)d_mv8.p : nullptr, nullptr, nullptr, 0);
+    };
+    if (launch()) return -1;
+    B2_CUDA_OK(cudaDeviceSynchronize());
+    if (kernel_ms) {
+        cudaEvent_t e0, e1;
+        cudaEventCreate(&e0); cudaEventCreate(&e1);
+        if (iters < 1) iters = 1;
+        cudaEventRecord(e0, 0);
+        for (int i = 0; i < iters; i++) launch();
+        cudaEventRecord(e1, 0);
+        B2_CUDA_OK(cudaEventSynchronize(e1));
+        float ms = 0;
+        cudaEventElapsedTime(&ms, e0, e1);
+        *kernel_ms = ms / iters;
+        cudaEventDestroy(e0); cudaEventDestroy(e1);
+    }
+    if (mv_out) B2_CUDA_OK(cudaMemcpy(mv_out, d_mv.p, nmb * sizeof(b2_mv_t), cudaMemcpyDeviceToHost));
+    if (cost_out) B2_CUDA_OK(cudaMemcpy(cost_out, d_cost.p, nmb * 4, cudaMemcpyDeviceToHost));
+    if (pred_out) B2_CUDA_OK(cudaMemcpy(pred_out, d_pred.p, nmb * 256, cudaMemcpyDeviceToHost));
+    if (part_out) B2_CUDA_OK(cudaMemcpy(part_out, d_part.p, nmb, cudaMemcpyDeviceToHost));
+    if (mv8_out) B2_CUDA_OK(cudaMemcpy(mv8_out, d_mv8.p, nmb * 3 * sizeof(b2_mv_t), cudaMemcpyDeviceToHost));
+    return 0;
+}
+
 static int me_fullpel_impl(const uint8_t *cur_y, const uint8_t *ref_y, int w, int h, int nframes, int merange, const b2_mv_t *pmv,
                            int lambda, b2_mv_t *mv_out, uint32_t *cost_out, b2_mv_t *mv9_out, uint32_t *cost9_out, int iters,
                            float *kernel_ms, const PruneOut *prune)

@@ -5,17 +5,23 @@
 // centre first, then the 8 quarter-pel neighbours of the winner; cost = SATD16x16 +
 // lambda*mvbits(mv - pmv); first minimum in scan order wins).
 //
-// One CTA per macroblock.  The 22x22 reference patch around the full-pel winner is staged in shared
-// memory once; the three half-sample planes b (horizontal), h (vertical) and j (centre, from the
-// UNROUNDED horizontal intermediates, as 8.4.2.2.1 requires) are built once and every one of the
-// 17 candidates is then a two-plane average -- the 6-tap filter runs ~1,300 times per MB instead
-// of ~50,000 times if each candidate were interpolated on its own.
+// One warp per macroblock, K2_MBS macroblocks per CTA.  The 22x22 reference patch around the full-pel
+// winner is staged in shared memory once; the three half-sample planes b (horizontal), h (vertical)
+// and j (centre, from the UNROUNDED horizontal intermediates, as 8.4.2.2.1 requires) are built once
+// and every one of the 17 candidates is then a two-plane average -- the 6-tap filter runs ~1,300
+// times per MB instead of ~50,000 times if each candidate were interpolated on its own.
 // Bound: integer ALU; algorithmic work = 17 candidates x 16 SATD4x4 per MB (~10x below K1).
 #include "b2_h264.cuh"
 
 namespace {
 
-constexpr int K2_THREADS = 160;
+constexpr int K2_THREADS = 160;                          // wide partition kernel: one CTA per macroblock
+// Macroblocks (one warp each) per CTA of k2_me_subpel_kernel.  K2 alone, 64 frames of 1080p on a B200: 2 -> 1.242 ms,
+// 4 -> 1.240 ms, 8 -> 1.223 ms (profiles/r3_k2_warp_per_mb.txt); 16 would exceed the 48 KB of static shared memory.
+#ifndef B2_K2_MBS
+#define B2_K2_MBS 8
+#endif
+constexpr int K2_MBS = B2_K2_MBS;
 
 // All four sample planes live in ONE shared byte array with a common row pitch, so that a candidate is
 // "average of two byte planes" with two base offsets chosen once per thread -- no per-pixel switch.
@@ -26,10 +32,10 @@ constexpr int OFF_H = OFF_B + 18 * KP;                    // h : 17 rows, origin
 constexpr int OFF_J = OFF_H + 17 * KP;                    // j : 17 rows, origin (-1,-1)
 constexpr int PLANES_BYTES = OFF_J + 17 * KP;
 
-struct K2Smem {
+struct __align__(16) K2Smem {
+    uint8_t cur[16][16];      // source macroblock (16-byte rows)
     uint8_t P[PLANES_BYTES];  // G | b | h | j
     int16_t B1[22][18];       // unrounded horizontal half samples: rows -3..18, cols -1..15
-    uint8_t cur[16][16];
     uint32_t cost[9];
     int best;
     // inter partitions (row N1): SATD per candidate and 8x8 quadrant, winners per shape part, final quadrant vectors
@@ -107,13 +113,6 @@ __device__ __forceinline__ void cur_block_rows(const K2Smem &s, int px, int py, 
     }
 }
 
-// four consecutive bytes at byte offset `off` (any alignment) + row * KP of the plane array
-struct PlaneWords {
-    const uint32_t *w; uint32_t sh;
-    __device__ __forceinline__ PlaneWords(const K2Smem &s, int off) : w((const uint32_t *)(s.P + (off & ~3))), sh((uint32_t)(off & 3) * 8u) {}
-    __device__ __forceinline__ uint32_t row(int y) const { return __funnelshift_r(w[y * (KP / 4)], w[y * (KP / 4) + 1], sh); }
-};
-
 // the two plane offsets of the candidate displaced by (cx,cy) quarter-pels, for the block at part-local pixel (bx,by)
 __device__ __forceinline__ void cand_planes(int bx, int by, int cx, int cy, int ga, int &offA, int &offB)
 {
@@ -123,19 +122,28 @@ __device__ __forceinline__ void cand_planes(int bx, int by, int cx, int cy, int 
     offB = plane_off((e >> 4) & 3, bx + ix + ((e >> 6) & 1), by + iy + ((e >> 7) & 1), ga);
 }
 
-// SATD of the 4x4 block at part-local pixel (bx,by) for the candidate displaced by (cx,cy) quarter-pels; ch = cur_block_rows
-// of the same block.  TWO = false: half-sample grid positions (one plane, stage 1); true: average of two planes (stage 2).
-template <bool TWO>
-__device__ __forceinline__ uint32_t cand_block_satd(const K2Smem &s, const int (&ch)[16], int bx, int by, int cx, int cy, int ga)
+// A plane offset (>= 0) as word index | funnel shift << 16.  Blocks and prediction words start at multiples of 4 bytes in every
+// plane (KP % 4 == 0), so a candidate's packed offsets for the block at (0,0) serve every block: add the block's word index.
+__device__ __forceinline__ uint32_t pack_off(int off) { return (uint32_t)(off >> 2) | ((uint32_t)(off & 3) << 19); }
+
+// four consecutive bytes of row y below the packed offset po, displaced by wbase words
+__device__ __forceinline__ uint32_t plane_word(const K2Smem &s, int wbase, uint32_t po, int y)
 {
-    int offA, offB;
-    cand_planes(bx, by, cx, cy, ga, offA, offB);
-    const PlaneWords A(s, offA), B(s, offB);
+    const uint32_t *w = (const uint32_t *)s.P + wbase + (po & 0xffffu) + y * (KP / 4);
+    return __funnelshift_r(w[0], w[1], po >> 16);
+}
+
+// SATD of one 4x4 block (word index wbase = (by * KP + bx) / 4) against the prediction at packed plane offsets pa / pb of the
+// block at (0,0); ch = cur_block_rows of the same block.  TWO = false: half-sample grid positions (one plane, stage 1); true:
+// average of two planes (stage 2).
+template <bool TWO>
+__device__ __forceinline__ uint32_t block_satd(const K2Smem &s, const int (&ch)[16], int wbase, uint32_t pa, uint32_t pb)
+{
     int t[16];
 #pragma unroll
     for (int y = 0; y < 4; y++) {
-        uint32_t p = A.row(y);
-        if (TWO) p = __vavgu4(p, B.row(y));
+        uint32_t p = plane_word(s, wbase, pa, y);
+        if (TWO) p = __vavgu4(p, plane_word(s, wbase, pb, y));
         t[4 * y + 0] = dp4a_us(p, H4N0, ch[4 * y + 0]); t[4 * y + 1] = dp4a_us(p, H4N1, ch[4 * y + 1]);
         t[4 * y + 2] = dp4a_us(p, H4N2, ch[4 * y + 2]); t[4 * y + 3] = dp4a_us(p, H4N3, ch[4 * y + 3]);
     }
@@ -148,114 +156,152 @@ __device__ __forceinline__ uint32_t cand_block_satd(const K2Smem &s, const int (
     return (uint32_t)sum;
 }
 
-// refinement of ONE macroblock around the full-pel vector mvf (whole CTA); PART: also the local partition refinement
+// the same for the block at part-local pixel (bx,by) and the candidate displaced by (cx,cy) quarter-pels
+template <bool TWO>
+__device__ __forceinline__ uint32_t cand_block_satd(const K2Smem &s, const int (&ch)[16], int bx, int by, int cx, int cy, int ga)
+{
+    int offA, offB;
+    cand_planes(0, 0, cx, cy, ga, offA, offB);
+    return block_satd<TWO>(s, ch, (by * KP + bx) >> 2, pack_off(offA), pack_off(offB));
+}
+
+// quarter-pel offsets of the nine candidates (c_subpel_off) as 2-bit fields (offset + 1), so that a lane can take the offset of
+// ITS candidate with a shift instead of a per-lane constant-bank load
+constexpr uint32_t SUB_DX = 0x24891u, SUB_DY = 0x2a501u;
+__device__ __forceinline__ int sub_dx(int k) { return (int)((SUB_DX >> (2 * k)) & 3u) - 1; }
+__device__ __forceinline__ int sub_dy(int k) { return (int)((SUB_DY >> (2 * k)) & 3u) - 1; }
+
+// sum over the 16 lanes of each half-warp: (half 0, half 1), both in every lane
+__device__ __forceinline__ void half_sums(uint32_t v, bool upper, uint32_t &lo, uint32_t &hi)
+{
+    lo = __reduce_add_sync(0xffffffffu, upper ? 0u : v);
+    hi = __reduce_add_sync(0xffffffffu, upper ? v : 0u);
+}
+
+// sum over the four lanes of one 8x8 quadrant (block bits 0 and 2); the lanes with blk & 5 == 0 write it
+__device__ __forceinline__ uint32_t quad_sum(uint32_t v)
+{
+    v += __shfl_xor_sync(0xffffffffu, v, 1);
+    return v + __shfl_xor_sync(0xffffffffu, v, 4);
+}
+
+// Refinement of ONE macroblock around the full-pel vector mvf by ONE warp; PART: also the local partition refinement.
+// Lane l keeps 4x4 block l & 15 for every candidate it prices; the two half-warps take different candidates (stage 1: 0..4 and
+// 5..8, stage 2: 1..4 and 5..8), so the source block's H4 rows are computed twice per macroblock and a candidate's SATD is a
+// 16-lane reduction.  Only __syncwarp orders the shared-memory phases.
 template <bool PART>
 __device__ __forceinline__ void k2_body(K2Smem &s, const uint8_t *__restrict__ cur, const uint8_t *__restrict__ ref, int pitch, size_t plane_stride,
-                                        int mbw, int mbh, const b2_mv_t mvf, const b2_mv_t pm, int lambda, int subpel,
+                                        int mbx, int mby, int frame, size_t mbi, const b2_mv_t mvf, const b2_mv_t pm, int lambda, int subpel,
                                         b2_mv_t *__restrict__ mv_out, uint32_t *__restrict__ cost_out, uint8_t *__restrict__ pred_out,
                                         uint8_t *__restrict__ part_out, b2_mv_t *__restrict__ mv8_out)
 {
-    const int tid = threadIdx.x;
-    const int mbx = blockIdx.x, mby = blockIdx.y, frame = blockIdx.z;
-    const size_t mbi = ((size_t)frame * mbh + mby) * mbw + mbx;
-
+    const int lane = threadIdx.x & 31;
     const uint8_t *cplane = cur + frame * plane_stride + (size_t)(B2_PAD + mby * 16) * pitch + B2_PAD + mbx * 16;
     const uint8_t *rplane = ref + frame * plane_stride + (size_t)(B2_PAD + mby * 16 + mvf.y - 3) * pitch + B2_PAD +
                             mbx * 16 + mvf.x - 3;
     uint8_t *PG = s.P + OFF_G, *PB = s.P + OFF_B, *PH = s.P + OFF_H, *PJ = s.P + OFF_J;
-    // 22x22 reference patch as ALIGNED words: 7 words cover a 22-byte row at any of the four alignments, 22 x 7 = 154 loads,
-    // one per thread and all in flight at once (byte-wise staging was 8 % of the instructions and 18 % of the stall samples).
-    // The row keeps its alignment in shared memory: G's column X sits at byte X + 3 + ga.  pitch, plane_stride and B2_PAD are
-    // multiples of 4 and the 64-pixel frame border covers the extra bytes.
+    // 22x22 reference patch as ALIGNED words: 7 words cover a 22-byte row at any of the four alignments, 22 x 7 = 154 loads, all
+    // in flight at once.  The row keeps its alignment in shared memory: G's column X sits at byte X + 3 + ga.  pitch, plane_stride
+    // and B2_PAD are multiples of 16 and the 64-pixel frame border covers the extra bytes.
     const int ga = (mvf.x + 1) & 3;                          // (mvf.x - 3) mod 4
-    if (tid < 154) {
-        const int r = tid / 7, wi = tid - r * 7;
-        ((uint32_t *)PG)[r * (KP / 4) + wi] = ((const uint32_t *)(rplane - ga))[(size_t)r * (pitch >> 2) + wi];
-    }
-    if (tid < 64) {
-        const int r = tid >> 2, c = tid & 3;
-        *(uint32_t *)&s.cur[r][c * 4] = *(const uint32_t *)(cplane + (size_t)r * pitch + c * 4);
-    }
-    if (tid < 9) s.cost[tid] = 0;
-    if (PART && tid < 36) s.costq[tid >> 2][tid & 3] = 0;
-    __syncthreads();
-
-    // Half-sample planes with SLIDING WINDOWS: one thread walks a whole row (b1) or column (h, j), so that every sample is
-    // loaded once and feeds six outputs -- 3 x fewer instructions than one 6-tap gather per output (K2 is issue-bound).
-    // b1: unrounded horizontal half samples, 22 rows x 17 cols (warp 0, lane = row); h: vertical half samples, 17 rows x 18
-    // cols (warp 1, lane = column).
     {
-        const int warp = tid >> 5, lane = tid & 31;
-        if (warp == 0 && lane < 22) {
-            const uint32_t *row = (const uint32_t *)(PG + lane * KP);             // 24-byte rows: word aligned
-            int g[24];
+        const uint32_t *src = (const uint32_t *)(rplane - ga);
 #pragma unroll
-            for (int i = 0; i < 6; i++) {
-                const uint32_t wv = __funnelshift_r(row[i], row[i + 1], 8 * ga);
-                g[4 * i] = wv & 255; g[4 * i + 1] = (wv >> 8) & 255; g[4 * i + 2] = (wv >> 16) & 255; g[4 * i + 3] = wv >> 24;
-            }
-#pragma unroll
-            for (int c = 0; c < 17; c++) s.B1[lane][c] = (int16_t)b2::tap6(g[c], g[c + 1], g[c + 2], g[c + 3], g[c + 4], g[c + 5]);
-        } else if (warp == 1 && lane < 18) {
-            const uint8_t *q = PG + lane + 2 + ga;                                  // column X = lane - 1
-            int g[22];
-#pragma unroll
-            for (int r = 0; r < 22; r++) g[r] = q[r * KP];
-#pragma unroll
-            for (int r = 0; r < 17; r++)
-                PH[r * KP + lane] = (uint8_t)b2_clip255((b2::tap6(g[r], g[r + 1], g[r + 2], g[r + 3], g[r + 4], g[r + 5]) + 16) >> 5);
-        }
-    }
-    __syncthreads();
-    {   // j: centre half samples from the unrounded b1 (warp 0, lane = column); b: rounded b1 (warps 1-4)
-        const int warp = tid >> 5, lane = tid & 31;
-        if (warp == 0) {
-            if (lane < 17) {
-                int g[22];
-#pragma unroll
-                for (int r = 0; r < 22; r++) g[r] = s.B1[r][lane];
-#pragma unroll
-                for (int r = 0; r < 17; r++)
-                    PJ[r * KP + lane] = (uint8_t)b2_clip255((b2::tap6(g[r], g[r + 1], g[r + 2], g[r + 3], g[r + 4], g[r + 5]) + 512) >> 10);
-            }
-        } else {
-            for (int i = tid - 32; i < 18 * 17; i += K2_THREADS - 32) {          // b: Y = r-1 -> B1 row r+2
-                const int r = i / 17, c = i - r * 17;
-                PB[r * KP + c] = (uint8_t)b2_clip255((s.B1[r + 2][c] + 16) >> 5);
+        for (int k = 0; k < 5; k++) {
+            const int i = lane + 32 * k;
+            if (i < 154) {
+                const int r = i / 7, wi = i - r * 7;
+                ((uint32_t *)PG)[r * (KP / 4) + wi] = src[(size_t)r * (pitch >> 2) + wi];
             }
         }
+        if (lane < 16) *(uint4 *)&s.cur[lane][0] = *(const uint4 *)(cplane + (size_t)lane * pitch);
     }
-    __syncthreads();
+    __syncwarp();
 
-    // every thread keeps ONE 4x4 block (tid & 15) through both stages: its H4-transformed source rows are computed once
-    const int blk = tid & 15, bx = (blk & 3) * 4, by = (blk >> 2) * 4;
+    // Half-sample planes with SLIDING WINDOWS: one lane walks a whole row (b1, and b from it) or column (h, j), so that every sample
+    // is loaded once and feeds six outputs.  b1: unrounded horizontal half samples, 22 rows x 17 cols (lane = row), rows 2..19
+    // also give b; h: vertical half samples, 17 rows x 18 cols (lane = column); j from the unrounded b1 (lane = column).
+    if (lane < 22) {
+        const uint32_t *row = (const uint32_t *)(PG + lane * KP);                 // 24-byte rows: word aligned
+        int g[24];
+#pragma unroll
+        for (int i = 0; i < 6; i++) {
+            const uint32_t wv = __funnelshift_r(row[i], row[i + 1], 8 * ga);
+            g[4 * i] = wv & 255; g[4 * i + 1] = (wv >> 8) & 255; g[4 * i + 2] = (wv >> 16) & 255; g[4 * i + 3] = wv >> 24;
+        }
+        const bool has_b = lane >= 2 && lane < 20;                                // b: Y = r-1 -> B1 row r+2
+#pragma unroll
+        for (int c = 0; c < 17; c++) {
+            const int v = b2::tap6(g[c], g[c + 1], g[c + 2], g[c + 3], g[c + 4], g[c + 5]);
+            s.B1[lane][c] = (int16_t)v;
+            if (has_b) PB[(lane - 2) * KP + c] = (uint8_t)b2_clip255((v + 16) >> 5);
+        }
+    }
+    if (lane < 18) {
+        const uint8_t *q = PG + lane + 2 + ga;                                      // column X = lane - 1
+        int g[22];
+#pragma unroll
+        for (int r = 0; r < 22; r++) g[r] = q[r * KP];
+#pragma unroll
+        for (int r = 0; r < 17; r++)
+            PH[r * KP + lane] = (uint8_t)b2_clip255((b2::tap6(g[r], g[r + 1], g[r + 2], g[r + 3], g[r + 4], g[r + 5]) + 16) >> 5);
+    }
+    __syncwarp();
+    if (lane < 17) {
+        int g[22];
+#pragma unroll
+        for (int r = 0; r < 22; r++) g[r] = s.B1[r][lane];
+#pragma unroll
+        for (int r = 0; r < 17; r++)
+            PJ[r * KP + lane] = (uint8_t)b2_clip255((b2::tap6(g[r], g[r + 1], g[r + 2], g[r + 3], g[r + 4], g[r + 5]) + 512) >> 10);
+    }
+    __syncwarp();
+
+    const int blk = lane & 15, bx = (blk & 3) * 4, by = (blk >> 2) * 4, wb = (by * KP + bx) >> 2;
+    const bool upper = lane >= 16;
     int ch[16];
     cur_block_rows(s, bx, by, ch);
+    // Plane offsets are computed once per macroblock, one candidate per lane, and fetched by shuffle: lane k < 9 holds half-pel
+    // candidate k's (a single plane)
+    uint32_t po1;
+    {
+        const int k = lane < 9 ? lane : 0;
+        int oa, ob;
+        cand_planes(0, 0, 2 * sub_dx(k), 2 * sub_dy(k), ga, oa, ob);
+        po1 = pack_off(oa);
+    }
 
+    uint32_t qm_all = 0;                                     // winner relative to the full-pel position (single-vector path)
     if (PART) {
         // ---- partitions: SATD per (candidate, quadrant); every shape part picks its half-pel winner, the cheapest shape
         // is kept and each of its parts tries the 8 quarter-pel neighbours of ITS winner (oracle: b2o_me_subpel_part) ----
-        if (tid < 9 * 16) {
-            const int cand = tid >> 4;
-            const uint32_t v = cand_block_satd<false>(s, ch, bx, by, 2 * c_subpel_off[cand][0], 2 * c_subpel_off[cand][1], ga);
-            atomicAdd(&s.costq[cand][((blk >> 1) & 1) | ((blk >> 3) << 1)], v);
+        const int q = ((blk >> 1) & 1) | ((blk >> 3) << 1);
+        const bool qlead = (blk & 5) == 0;
+#pragma unroll
+        for (int i = 0; i < 5; i++) {
+            const int cand = i + (upper ? 5 : 0);
+            const uint32_t pa = __shfl_sync(0xffffffffu, po1, cand);
+            uint32_t v = 0;
+            if (cand < 9) v = block_satd<false>(s, ch, wb, pa, 0);
+            v = quad_sum(v);
+            if (qlead && cand < 9) s.costq[cand][q] = v;
         }
-        __syncthreads();
-        if (tid < 9) {                                   // one thread per shape part
-            const int mask = c_part_mask[tid];
+        __syncwarp();
+        if (lane < 9) {                                  // one lane per shape part
+            const int mask = c_part_mask[lane];
             uint32_t best = 0xffffffffu; int bk = 0;
             for (int k = 0; k < 9; k++) {
                 const int mx = mvf.x * 4 + 2 * c_subpel_off[k][0], my = mvf.y * 4 + 2 * c_subpel_off[k][1];
                 uint32_t c = (uint32_t)(lambda * (b2_mvbits(mx - pm.x) + b2_mvbits(my - pm.y)));
 #pragma unroll
-                for (int q = 0; q < 4; q++)
-                    if (mask & (1 << q)) c += s.costq[k][q];
+                for (int qq = 0; qq < 4; qq++)
+                    if (mask & (1 << qq)) c += s.costq[k][qq];
                 if (c < best) { best = c; bk = k; }
             }
-            s.pcost[tid] = best; s.pk[tid] = bk;
+            s.pcost[lane] = best; s.pk[lane] = bk;
         }
-        __syncthreads();
-        if (tid == 0) {
+        __syncwarp();
+        if (lane == 0) {
             uint32_t bc = 0xffffffffu; int shape = 0;
             for (int sh = 0; sh < 4; sh++) {
                 uint32_t c = (uint32_t)(lambda * c_shape_bits[sh]);
@@ -265,130 +311,162 @@ __device__ __forceinline__ void k2_body(K2Smem &s, const uint8_t *__restrict__ c
             s.shape = shape;
             for (int a = 0; a < c_shape_n[shape]; a++) {
                 const int p = c_shape_first[shape] + a;
-                for (int q = 0; q < 4; q++)
-                    if (c_part_mask[p] & (1 << q)) s.qk[q] = s.pk[p];
+                for (int qq = 0; qq < 4; qq++)
+                    if (c_part_mask[p] & (1 << qq)) s.qk[qq] = s.pk[p];
             }
         }
-        if (tid < 36) s.costq[tid >> 2][tid & 3] = 0;    // reused for stage 2 (entries 1..8); stage-1 sums are folded into pcost
-        __syncthreads();
-        if (tid < 8 * 16) {
-            const int cand = 1 + (tid >> 4), q = ((blk >> 1) & 1) | ((blk >> 3) << 1);
-            const int hk = s.qk[q];
-            const uint32_t v = cand_block_satd<true>(s, ch, bx, by, 2 * c_subpel_off[hk][0] + c_subpel_off[cand][0], 2 * c_subpel_off[hk][1] + c_subpel_off[cand][1], ga);
-            atomicAdd(&s.costq[cand][q], v);
+        __syncwarp();
+        {   // stage 2: entries 1..8 of costq are overwritten; the stage-1 sums are folded into pcost.  Lane 8q + k - 1 holds the
+            // plane offsets of quarter-pel candidate k around quadrant q's half-pel winner.
+            uint32_t pa2, pb2;
+            {
+                const int hk = s.qk[lane >> 3], k = (lane & 7) + 1;
+                int oa, ob;
+                cand_planes(0, 0, 2 * sub_dx(hk) + sub_dx(k), 2 * sub_dy(hk) + sub_dy(k), ga, oa, ob);
+                pa2 = pack_off(oa); pb2 = pack_off(ob);
+            }
+#pragma unroll
+            for (int i = 0; i < 4; i++) {
+                const int cand = 1 + i + (upper ? 4 : 0), src = 8 * q + cand - 1;
+                const uint32_t pa = __shfl_sync(0xffffffffu, pa2, src), pb = __shfl_sync(0xffffffffu, pb2, src);
+                const uint32_t v = quad_sum(block_satd<true>(s, ch, wb, pa, pb));
+                if (qlead) s.costq[cand][q] = v;
+            }
         }
-        __syncthreads();
-        if (tid < c_shape_n[s.shape]) {                   // one thread per part of the chosen shape
-            const int p = c_shape_first[s.shape] + tid, mask = c_part_mask[p], hk = s.pk[p];
+        __syncwarp();
+        const int shape = s.shape;
+        if (lane < c_shape_n[shape]) {                   // one lane per part of the chosen shape
+            const int p = c_shape_first[shape] + lane, mask = c_part_mask[p], hk = s.pk[p];
             const int hx = 2 * c_subpel_off[hk][0], hy = 2 * c_subpel_off[hk][1];
-            uint32_t best = s.pcost[p]; int bx = hx, by = hy;
+            uint32_t best = s.pcost[p]; int wx = hx, wy = hy;
             for (int k = 1; k < 9; k++) {
                 const int dx = hx + c_subpel_off[k][0], dy = hy + c_subpel_off[k][1];
                 uint32_t c = (uint32_t)(lambda * (b2_mvbits(mvf.x * 4 + dx - pm.x) + b2_mvbits(mvf.y * 4 + dy - pm.y)));
 #pragma unroll
-                for (int q = 0; q < 4; q++)
-                    if (mask & (1 << q)) c += s.costq[k][q];
-                if (c < best) { best = c; bx = dx; by = dy; }
+                for (int qq = 0; qq < 4; qq++)
+                    if (mask & (1 << qq)) c += s.costq[k][qq];
+                if (c < best) { best = c; wx = dx; wy = dy; }
             }
             s.pcost[p] = best;
 #pragma unroll
-            for (int q = 0; q < 4; q++)
-                if (mask & (1 << q)) s.qmv[q] = (bx & 0xff) | ((by & 0xff) << 8);
+            for (int qq = 0; qq < 4; qq++)
+                if (mask & (1 << qq)) s.qmv[qq] = (wx & 0xff) | ((wy & 0xff) << 8);
         }
-        __syncthreads();
-        if (tid == 0) {
-            const int shape = s.shape;
+        __syncwarp();
+        if (lane == 0) {
             uint32_t total = (uint32_t)(lambda * c_shape_bits[shape]);
             for (int a = 0; a < c_shape_n[shape]; a++) total += s.pcost[c_shape_first[shape] + a];
             cost_out[mbi] = total;
             part_out[mbi] = (uint8_t)shape;
-            for (int q = 0; q < 4; q++) {
+            for (int qq = 0; qq < 4; qq++) {
                 b2_mv_t o;
-                o.x = (int16_t)(mvf.x * 4 + (int)(int8_t)(s.qmv[q] & 0xff));
-                o.y = (int16_t)(mvf.y * 4 + (int)(int8_t)((s.qmv[q] >> 8) & 0xff));
-                if (q == 0) mv_out[mbi] = o;
-                else mv8_out[mbi * 3 + q - 1] = o;
+                o.x = (int16_t)(mvf.x * 4 + (int)(int8_t)(s.qmv[qq] & 0xff));
+                o.y = (int16_t)(mvf.y * 4 + (int)(int8_t)((s.qmv[qq] >> 8) & 0xff));
+                if (qq == 0) mv_out[mbi] = o;
+                else mv8_out[mbi * 3 + qq - 1] = o;
             }
         }
     } else {
-    // stage 1: centre + 8 half-pel neighbours (offsets x2 quarter units); without sub-pel: centre only
-    const int n1 = subpel ? 9 : 1;
-    if (tid < n1 * 16) {
-        const int cand = tid >> 4;
-        const uint32_t v = cand_block_satd<false>(s, ch, bx, by, 2 * c_subpel_off[cand][0], 2 * c_subpel_off[cand][1], ga);
-        atomicAdd(&s.cost[cand], v);
-    }
-    __syncthreads();
-    if (tid < 32) {                                      // nine lanes price their candidate, a warp minimum picks the first best
+        // stage 1: centre + 8 half-pel neighbours (offsets x2 quarter units); without sub-pel: centre only.  Lane k < 9 ends up
+        // holding candidate k's SATD, prices it, and a warp minimum picks the first best.
+        const int n1 = subpel ? 9 : 1;
+        uint32_t mine = 0;
+#pragma unroll
+        for (int i = 0; i < 5; i++) {
+            if (i >= n1) break;
+            const int cand = i + (upper ? 5 : 0);
+            const uint32_t pa = __shfl_sync(0xffffffffu, po1, cand);
+            uint32_t v = 0, lo, hi;
+            if (cand < n1) v = block_satd<false>(s, ch, wb, pa, 0);
+            half_sums(v, upper, lo, hi);
+            if (lane == i) mine = lo;
+            if (lane == i + 5) mine = hi;
+        }
         uint32_t key = 0xffffffffu;
-        if (tid < n1) {
-            const int mx = mvf.x * 4 + 2 * c_subpel_off[tid][0], my = mvf.y * 4 + 2 * c_subpel_off[tid][1];
-            const uint32_t c = s.cost[tid] + (uint32_t)(lambda * (b2_mvbits(mx - pm.x) + b2_mvbits(my - pm.y)));
-            key = (c << 4) | (uint32_t)tid;              // costs stay far below 2^28; ties go to the lower candidate index
+        if (lane < n1) {
+            const int mx = mvf.x * 4 + 2 * sub_dx(lane), my = mvf.y * 4 + 2 * sub_dy(lane);
+            const uint32_t c = mine + (uint32_t)(lambda * (b2_mvbits(mx - pm.x) + b2_mvbits(my - pm.y)));
+            key = (c << 4) | (uint32_t)lane;             // costs stay far below 2^28; ties go to the lower candidate index
         }
         key = __reduce_min_sync(0xffffffffu, key);
-        __syncwarp();
-        if (tid < 9) s.cost[tid] = tid == 0 ? key >> 4 : 0u;
-        if (tid == 0) s.best = (int)(key & 15u);
-    }
-    __syncthreads();
-    const int hx = 2 * c_subpel_off[s.best][0], hy = 2 * c_subpel_off[s.best][1];
-    if (subpel) {
-        if (tid < 8 * 16) {
-            const int cand = 1 + (tid >> 4);
-            const uint32_t v = cand_block_satd<true>(s, ch, bx, by, hx + c_subpel_off[cand][0], hy + c_subpel_off[cand][1], ga);
-            atomicAdd(&s.cost[cand], v);
+        const int h1 = (int)(key & 15u);
+        const int hx = 2 * sub_dx(h1), hy = 2 * sub_dy(h1);
+        // candidate 0 = the half-pel winner itself (already priced); 1..8 its quarter-pel neighbours; first minimum wins.  Without
+        // sub-pel the centre (candidate 0 of stage 1) is final.
+        uint32_t key2 = key;
+        if (subpel) {
+            key2 = lane == 0 ? (key >> 4) << 4 : 0xffffffffu;
+            mine = 0;
+            uint32_t pa2, pb2;                           // lane k - 1 (mod 8): plane offsets of quarter-pel candidate k
+            {
+                const int k = (lane & 7) + 1;
+                int oa, ob;
+                cand_planes(0, 0, hx + sub_dx(k), hy + sub_dy(k), ga, oa, ob);
+                pa2 = pack_off(oa); pb2 = pack_off(ob);
+            }
+#pragma unroll
+            for (int i = 0; i < 4; i++) {
+                const int cand = 1 + i + (upper ? 4 : 0);
+                const uint32_t pa = __shfl_sync(0xffffffffu, pa2, cand - 1), pb = __shfl_sync(0xffffffffu, pb2, cand - 1);
+                uint32_t lo, hi;
+                half_sums(block_satd<true>(s, ch, wb, pa, pb), upper, lo, hi);
+                if (lane == 1 + i) mine = lo;
+                if (lane == 5 + i) mine = hi;
+            }
+            if (lane >= 1 && lane < 9) {
+                const int mx = mvf.x * 4 + hx + sub_dx(lane), my = mvf.y * 4 + hy + sub_dy(lane);
+                const uint32_t c = mine + (uint32_t)(lambda * (b2_mvbits(mx - pm.x) + b2_mvbits(my - pm.y)));
+                key2 = (c << 4) | (uint32_t)lane;
+            }
+            key2 = __reduce_min_sync(0xffffffffu, key2);
         }
-        __syncthreads();
-    }
-    if (tid < 32) {
-        // candidate 0 = the half-pel winner itself (already priced); 1..8 its quarter-pel neighbours; first minimum wins
-        uint32_t key = 0xffffffffu;
-        if (tid == 0) key = s.cost[0] << 4;
-        else if (tid < 9 && subpel) {
-            const int mx = mvf.x * 4 + hx + c_subpel_off[tid][0], my = mvf.y * 4 + hy + c_subpel_off[tid][1];
-            const uint32_t c = s.cost[tid] + (uint32_t)(lambda * (b2_mvbits(mx - pm.x) + b2_mvbits(my - pm.y)));
-            key = (c << 4) | (uint32_t)tid;
-        }
-        key = __reduce_min_sync(0xffffffffu, key);
-        if (tid == 0) {
-            const int k = (int)(key & 15u);
-            const int dx = hx + (k ? c_subpel_off[k][0] : 0), dy = hy + (k ? c_subpel_off[k][1] : 0);
+        const int k = (int)(key2 & 15u);
+        const int dx = hx + (k ? sub_dx(k) : 0), dy = hy + (k ? sub_dy(k) : 0);
+        if (lane == 0) {
             b2_mv_t o;
             o.x = (int16_t)(mvf.x * 4 + dx); o.y = (int16_t)(mvf.y * 4 + dy);
             mv_out[mbi] = o;
-            cost_out[mbi] = key >> 4;
-            s.best = (dx & 0xff) | ((dy & 0xff) << 8);                             // winner relative to the full-pel position
+            cost_out[mbi] = key2 >> 4;
         }
-    }
-    if (tid == 0) { s.qmv[0] = s.qmv[1] = s.qmv[2] = s.qmv[3] = s.best; }
+        qm_all = (uint32_t)((dx & 0xff) | ((dy & 0xff) << 8));
     }
     // the winner's motion-compensated luma block (K5 subtracts it from the source instead of interpolating again)
     if (pred_out != nullptr) {
-        __syncthreads();
-        if (tid < 64) {                                               // 4 pixels per thread: row r, columns 4c..4c+3
-            const int r = tid >> 2, c = (tid & 3) * 4;
-            const int qm = s.qmv[(c >> 3) | ((r >> 3) << 1)];         // displacement of the quadrant this word lies in
-            const int cx = (int)(int8_t)(qm & 0xff), cy = (int)(int8_t)((qm >> 8) & 0xff);
-            int offA, offB;
-            cand_planes(c, r, cx, cy, ga, offA, offB);
-            *(uint32_t *)(pred_out + mbi * 256 + r * 16 + c) = __vavgu4(PlaneWords(s, offA).row(0), PlaneWords(s, offB).row(0));
+        uint32_t pa, pb;                                               // lane q (mod 4): plane offsets of quadrant q's winner
+        {
+            const int qm = PART ? s.qmv[lane & 3] : (int)qm_all;
+            int oa, ob;
+            cand_planes(0, 0, (int)(int8_t)(qm & 0xff), (int)(int8_t)((qm >> 8) & 0xff), ga, oa, ob);
+            pa = pack_off(oa); pb = pack_off(ob);
+        }
+#pragma unroll
+        for (int k = 0; k < 2; k++) {                                  // 4 pixels per lane and step: row r, columns 4c..4c+3
+            const int i = lane + 32 * k, r = i >> 2, c = (i & 3) * 4;
+            const int q = (c >> 3) | ((r >> 3) << 1);                  // the quadrant the word lies in
+            const uint32_t qa = __shfl_sync(0xffffffffu, pa, q), qb = __shfl_sync(0xffffffffu, pb, q);
+            const int w = (r * KP + c) >> 2;
+            *(uint32_t *)(pred_out + mbi * 256 + r * 16 + c) = __vavgu4(plane_word(s, w, qa, 0), plane_word(s, w, qb, 0));
         }
     }
 }
 
+// one warp per macroblock, K2_MBS consecutive macroblocks of a row per CTA (the tail CTA of a row has idle warps)
 template <bool PART>
-__global__ void __launch_bounds__(K2_THREADS)
+__global__ void __launch_bounds__(32 * K2_MBS)
 k2_me_subpel_kernel(const uint8_t *__restrict__ cur, const uint8_t *__restrict__ ref, int pitch, size_t plane_stride,
                     int mbw, int mbh, const b2_mv_t *__restrict__ mv_full, const b2_mv_t *__restrict__ pmv,
                     int lambda, int subpel, b2_mv_t *__restrict__ mv_out, uint32_t *__restrict__ cost_out,
                     uint8_t *__restrict__ pred_out, uint8_t *__restrict__ part_out, b2_mv_t *__restrict__ mv8_out)
 {
-    __shared__ __align__(16) K2Smem s;
-    const size_t mbi = ((size_t)blockIdx.z * mbh + blockIdx.y) * mbw + blockIdx.x;
+    __shared__ K2Smem sm[K2_MBS];
+    const int warp = threadIdx.x >> 5;
+    const int mbx = blockIdx.x * K2_MBS + warp;
+    if (mbx >= mbw) return;                                  // whole warps only: nothing below synchronises the CTA
+    const size_t mbi = ((size_t)blockIdx.z * mbh + blockIdx.y) * mbw + mbx;
     b2_mv_t pm = {0, 0};
     if (pmv) pm = pmv[mbi];
-    k2_body<PART>(s, cur, ref, pitch, plane_stride, mbw, mbh, mv_full[mbi], pm, lambda, subpel, mv_out, cost_out, pred_out, part_out, mv8_out);
+    k2_body<PART>(sm[warp], cur, ref, pitch, plane_stride, mbx, blockIdx.y, blockIdx.z, mbi, mv_full[mbi], pm, lambda, subpel, mv_out,
+                  cost_out, pred_out, part_out, mv8_out);
 }
 
 // ---- wide partition search (row N1, partitions = 2) --------------------------------------------------------------------
@@ -432,7 +510,9 @@ k2_me_subpel_wide_kernel(const uint8_t *__restrict__ cur, const uint8_t *__restr
     if (shape == B2_PART_16x16) {                            // the common case: the tuned single-vector path around part 0's vector
         const b2_mv_t mv16 = mv9[mbi * 9];
         __syncthreads();                                     // everyone has read s.shape before the body reuses the shared struct
-        k2_body<false>(s, cur, ref, pitch, plane_stride, mbw, mbh, mv16, pm, lambda, 1, mv_out, cost_out, pred_out, nullptr, nullptr);
+        if (tid >= 32) return;                               // the single-vector body is one warp's work
+        k2_body<false>(s, cur, ref, pitch, plane_stride, mbx, mby, frame, mbi, mv16, pm, lambda, 1, mv_out, cost_out, pred_out, nullptr,
+                       nullptr);
         if (tid == 0) part_out[mbi] = B2_PART_16x16;
         return;
     }
@@ -525,8 +605,10 @@ k2_me_subpel_wide_kernel(const uint8_t *__restrict__ cur, const uint8_t *__restr
             if (tid < wq * ph) {
                 const int r = tid / wq, c = (tid - r * wq) * 4;
                 int offA, offB;
-                cand_planes(c, r, cx, cy, 0, offA, offB);
-                *(uint32_t *)(pred_out + mbi * 256 + (oy + r) * 16 + ox + c) = __vavgu4(PlaneWords(s, offA).row(0), PlaneWords(s, offB).row(0));
+                cand_planes(0, 0, cx, cy, 0, offA, offB);
+                const int w = (r * KP + c) >> 2;
+                *(uint32_t *)(pred_out + mbi * 256 + (oy + r) * 16 + ox + c) =
+                    __vavgu4(plane_word(s, w, pack_off(offA), 0), plane_word(s, w, pack_off(offB), 0));
             }
         }
         __syncthreads();                                     // planes are rebuilt for the next part
@@ -541,18 +623,19 @@ int b2_launch_me_subpel(const uint8_t *d_cur, const uint8_t *d_ref, int pitch, s
                         b2_mv_t *d_mv_out, uint32_t *d_cost_out, uint8_t *d_pred_out, uint8_t *d_part_out, b2_mv_t *d_mv8_out,
                         const b2_mv_t *d_mv9, const uint32_t *d_cost9, cudaStream_t st)
 {
-    dim3 grid(mbw, mbh, nframes);
     if (d_mv9 && d_part_out && subpel) {
+        const dim3 grid(mbw, mbh, nframes);
         k2_me_subpel_wide_kernel<<<grid, K2_THREADS, 0, st>>>(d_cur, d_ref, pitch, plane_stride, mbw, mbh, d_mv9, d_cost9, d_pmv, lambda,
                                                                d_mv_out, d_cost_out, d_pred_out, d_part_out, d_mv8_out);
         B2_CUDA_OK(cudaGetLastError());
         return 0;
     }
+    const dim3 grid((mbw + K2_MBS - 1) / K2_MBS, mbh, nframes);
     if (d_part_out && subpel)
-        k2_me_subpel_kernel<true><<<grid, K2_THREADS, 0, st>>>(d_cur, d_ref, pitch, plane_stride, mbw, mbh, d_mv_full, d_pmv,
+        k2_me_subpel_kernel<true><<<grid, 32 * K2_MBS, 0, st>>>(d_cur, d_ref, pitch, plane_stride, mbw, mbh, d_mv_full, d_pmv,
                                                                lambda, subpel, d_mv_out, d_cost_out, d_pred_out, d_part_out, d_mv8_out);
     else
-        k2_me_subpel_kernel<false><<<grid, K2_THREADS, 0, st>>>(d_cur, d_ref, pitch, plane_stride, mbw, mbh, d_mv_full, d_pmv,
+        k2_me_subpel_kernel<false><<<grid, 32 * K2_MBS, 0, st>>>(d_cur, d_ref, pitch, plane_stride, mbw, mbh, d_mv_full, d_pmv,
                                                                 lambda, subpel, d_mv_out, d_cost_out, d_pred_out, nullptr, nullptr);
     B2_CUDA_OK(cudaGetLastError());
     return 0;
